@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RCVRP n=100 POMO rollout throughput (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path (fused construction rollout: decode loop + env step + reward) over one
@@ -79,8 +79,9 @@ def profile_stamp():
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of the headline workload (the per-config block "
+                                                          "times a fixed number of steps per config: C1 5, C3 5, C4 2, C5 5)")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps before the headline's timed steps")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=1024, help="instances per GPU per step")
     ap.add_argument("--precision", type=int, default=3, choices=[1, 3], help="3 = three-term fp16-split contractions, fp32-faithful (headline); 1 = single fp16 pass")
@@ -89,7 +90,14 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block (C1, C3, C4, C5)")
     ap.add_argument("--workload", default="c2", choices=["c2", "c5"], help="headline workload: BASELINE config[1] (default) or config[4]")
     ap.add_argument("--c5-global-batch", type=int, default=4096)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the rollout outputs of the last timed headline step (rank 0) "
+                                                          "to DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def peaks():
@@ -258,6 +266,31 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+# (row-index file, outputs it selects, row budget): per-rollout vectors are whole up to 2^20 rollouts (the default 827 392
+# fit); tours ([R, T] actions, T <= 2N) are a fixed sample of 2^14 rollouts (<= 13 MB at N = 101)
+DUMP_GROUPS = (("rollout_rows", ("reward", "normalized_reward", "log_likelihood"), 1 << 20),
+               ("tour_rows", ("actions",), 1 << 14))
+
+
+def dump_outputs(out_dir, out):
+    """What `fused_rollout` handed back in the last timed step, as float32 `.npy` files (node indices are exact in
+    float32); at most ~33 MB.  Each group's rows are written beside it (`rollout_rows.npy`, `tour_rows.npy`, float64): all
+    R rollouts in order, or, above the group's budget, a sorted sample drawn with a fixed seed.  Every file of an earlier
+    dump in `out_dir` is removed first, so an output this rollout does not return is absent rather than stale."""
+    os.makedirs(out_dir, exist_ok=True)
+    for rows_name, names, _ in DUMP_GROUPS:
+        for name in (rows_name, *names):
+            if os.path.exists(os.path.join(out_dir, name + ".npy")):
+                os.remove(os.path.join(out_dir, name + ".npy"))
+    R = out["actions"].shape[0]
+    for rows_name, names, k in DUMP_GROUPS:
+        idx = torch.arange(R) if R <= k else torch.randperm(R, generator=torch.Generator().manual_seed(0))[:k].sort().values
+        np.save(os.path.join(out_dir, rows_name + ".npy"), idx.numpy().astype(np.float64))
+        for name in names:
+            if name in out:
+                np.save(os.path.join(out_dir, name + ".npy"), out[name][idx.to(out[name].device)].float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------------
 # our arm
 # --------------------------------------------------------------------------------------------------
@@ -396,14 +429,15 @@ def run_ours(args, rank, world, local_rank):
         # BASELINE config[4] as the headline: fixed GLOBAL batch sharded over the ranks (strong scaling)
         sampler = ClockSampler(local_rank) if rank == 0 else None
         launches0 = _lib.kernel_count
-        entry = measure_configs(args, rb, dev, rank, world, dist_on, timed, only=("C5",), steps=args.steps)["C5"]
-        launches = (_lib.kernel_count - launches0) // (args.steps + 3) * args.steps
+        entry = measure_configs(args, rb, dev, rank, world, dist_on, timed, only=("C5",), steps=args.steps,
+                                warmup=args.warmup, dump_dir=args.dump_outputs)["C5"]
+        launches = (_lib.kernel_count - launches0) // (args.steps + args.warmup) * args.steps
         clocks = sampler.stop() if sampler else None
         if rank == 0:
             hbm_peak, tf_peak, peak_src = peaks()
             r = entry["roofline"]
             line = {"metric": "RCVRP n100 POMO training-rollout instances/s (global batch %d)" % args.c5_global_batch,
-                    "value": entry["value"], "unit": "instances/s", "n_gpus": world, "steps": args.steps, "warmup": 3,
+                    "value": entry["value"], "unit": "instances/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
                     "ms_per_step": entry["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                     "dtype": "f32 (fp32-faithful: three-term fp16-split tcgen05 contractions, fp32 accumulate)",
                     "data": "synthetic (8 city-like asymmetric 1000-node matrices in HBM, instances sub-sampled on the device; "
@@ -427,6 +461,8 @@ def run_ours(args, rank, world, local_rank):
     ms_step, out = timed(step_resident, args.steps, args.warmup)
     launches = (_lib.kernel_count - launches0) // (args.steps + args.warmup) * args.steps
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
     T = int(out["actions"].shape[1])
     tile_steps = out["tile_steps"].clone()
     value = world * B / (ms_step * 1e-3)
@@ -875,7 +911,7 @@ def cpu_config_rate(spec, n_inst, threads, seed=777):
     return n_inst / dt, dt, int(out["actions"].shape[1])
 
 
-def measure_configs(args, rb, dev, rank, world, dist_on, timed, only=None, steps=None):
+def measure_configs(args, rb, dev, rank, world, dist_on, timed, only=None, steps=None, warmup=3, dump_dir=None):
     from rrnco_b200.sharding import gather_costs
     hbm_peak, tf_peak, _ = peaks()
     block = {}
@@ -937,7 +973,7 @@ def measure_configs(args, rb, dev, rank, world, dist_on, timed, only=None, steps
                     gather_costs(best, world * Bc)
                 state["out"] = out
                 return best.cpu()  # D2H of the costs: the step's host-visible result
-            ms_val, _ = timed(step, spec["steps"], 3)
+            ms_val, _ = timed(step, spec["steps"], warmup)
             ms_e2e, h2d, d2h = ms_val, 0, Bc * 4
             e2e_what = ("same pipeline (this config has no host inputs: instances are generated on the device from the "
                         "HBM-resident city matrices, the encoder output is a resident stand-in); D2H of the [B] best costs")
@@ -954,7 +990,7 @@ def measure_configs(args, rb, dev, rank, world, dist_on, timed, only=None, steps
                     gather_costs(best, world * Bc)
                 state["out"] = out
                 return out
-            ms_val, _ = timed(step, spec["steps"], 3)
+            ms_val, _ = timed(step, spec["steps"], warmup)
             # e2e through the public API: pinned host instance td + encoder output -> H2D -> (aug) -> reset -> policy -> D2H
             host_td = {k: v.cpu().pin_memory() for k, v in gen(Bc).items()}
             host_emb = (embeds[0][0].cpu().pin_memory(), embeds[0][1].cpu().pin_memory())
@@ -995,6 +1031,8 @@ def measure_configs(args, rb, dev, rank, world, dist_on, timed, only=None, steps
                         "GEMM, rollout, D2H of the [B] costs")
             n_units = Bc * world
         out = state["out"]
+        if dump_dir and rank == 0:  # the rollout of the last timed step
+            dump_outputs(dump_dir, out)
         if "tile_steps" in out:
             ts = (out["tile_steps"].long() - 1).clamp_min(0)
             tr = rb._lib.lib().rrnco_rollout_tile_rows(rb._lib.ENV_ID[name], N, Bc * A, S)  # POMO starts per CTA tile

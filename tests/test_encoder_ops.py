@@ -23,16 +23,28 @@ def _fixture():
     return t, params
 
 
+def _assert_same_ops_reordered(got, want):
+    """Same torch ops as the recording, so the only difference is the order in which the host's GEMM sums (its SIMD code
+    path and thread count: one thread instead of eight on the recording CPU already changes bits).  Measured across MKL's
+    AVX-512 / AVX2 / SSE4.2 paths and 1-16 threads: at most 7 fp32 ulps of the output's largest magnitude; bound: 32.
+    A 0.1 % change to 32 of the fixture's 39 parameter tensors exceeds it, and a 10 % change to the duration variant's
+    `dist_emb.2.bias`.  The other six stay within it even at 10 %, so no tolerance pins them: AFT's `to_k.bias` cancels in the
+    key softmax over the nodes, and the duration gate's `gate_temperature` of 15 (divided out as exp(15)) leaves that gate
+    near uniform, whatever its other parameters."""
+    atol = 32 * torch.finfo(torch.float32).eps * want.abs().max().item()
+    torch.testing.assert_close(got, want, rtol=0, atol=atol)
+
+
 def test_oracle_matches_reference_fixture():
     t, params = _fixture()
     for tag in ("nodur", "dur"):
         dur = t["dur"] if tag == "dur" else None
         out = oenc.dist_angle_fusion(params[tag], t["coords"], t["cost"], dur)
-        assert torch.equal(out, t[tag + ".bias"])  # same torch ops in the same order: bit-exact on the CPU
+        _assert_same_ops_reordered(out, t[tag + ".bias"])
         outT = oenc.dist_angle_fusion(params[tag], t["coords"], t["cost"].transpose(1, 2), None if dur is None else dur.transpose(1, 2))
-        assert torch.equal(outT, t[tag + ".bias_T"])
+        _assert_same_ops_reordered(outT, t[tag + ".bias_T"])
     out = oenc.aft_full(params["aft"], t["aft.x"], t["aft.y"], t["nodur.bias"] * 1.7)
-    assert torch.equal(out, t["aft.out"])
+    _assert_same_ops_reordered(out, t["aft.out"])
 
 
 def collapsed_bias(p, coords, cost):
