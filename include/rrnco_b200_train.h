@@ -17,6 +17,7 @@
  *   rrnco_train_inst_gemm / _xty  the pointer scores g . Lk^T and their gradients, one weight tile per instance (decoder.py:298-301)
  *   rrnco_train_logits_tail edge bias, log(exp(.) + 1e-6), tanh clip, mask, temperature, log-softmax and the log-prob of
  *                           the given action with its Jacobian, in one pass (decoder.py:183-198, decoding.py:311-399)
+ *   rrnco_train_nab_backward the parameter gradients of the encoder's gating neural adaptive bias (attn_freenet.py:242-289)
  *
  * Conventions as in rrnco_b200.h: plain pointers and sizes, device pointers unless noted, return 0 = RRNCO_OK or a negative
  * error, `stream` = cudaStream_t (NULL = default stream), `status` = sticky device word (RRNCO_DEV_NAN_LOGITS when an fp16
@@ -110,6 +111,24 @@ int rrnco_train_inst_gemm(int64_t n_inst, int64_t rows_per_inst, const float* x,
                           const float* row_scale, float* y, uint32_t* status, void* stream);
 int rrnco_train_inst_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* x, const float* y, const float* sx,
                          const float* sy, const float* row_scale, float* c, uint32_t* status, void* stream);
+
+/* Backward of the encoder's gating neural adaptive bias (DistAngleFusion.forward, rrnco/models/nn/attn_freenet.py:242-289,
+ * the two-way gate of ATSP / RCVRP), the forward of which is rrnco_nab_gating (rrnco_b200.h):
+ *   coords [n_inst, n_nodes, 2], cost [n_inst, n_nodes, n_nodes] (read as its transpose when transpose_cost != 0), `packed` and
+ *   `scale` exactly as the forward call got them; grad_out [n_inst, n_nodes, n_nodes] = dL/d out.
+ *   params / grads: the module's 12 tensors in nn.Linear layouts, concatenated (rrnco_train_nab_grad_floats() floats):
+ *   dist_emb.0.weight [E,1], dist_emb.0.bias [E], dist_emb.2.weight [E,E], dist_emb.2.bias [E], the same four of angle_emb,
+ *   gate.0.weight [1,2E], gate.0.bias [1], out_lin.weight [1,E], out_lin.bias [1]  (E = 128).  grads are written, not accumulated.
+ *   workspace: rrnco_train_nab_workspace_bytes(n_inst, n_nodes) bytes (depends on the current device), 8-byte aligned.
+ * One pass over the pairs (the forward's per-pair work and a per-segment histogram), nothing of size [n_inst, N, N, E];
+ * no atomics: the gradients are bitwise identical run to run on one device.  No gradients for coords / cost.
+ * rrnco_train_nab_packed_floats() = the size of `packed` this library expects (= rrnco_nab_packed_floats()). */
+int64_t rrnco_train_nab_packed_floats(void);
+int64_t rrnco_train_nab_grad_floats(void);
+int64_t rrnco_train_nab_workspace_bytes(int64_t n_inst, int32_t n_nodes);
+int rrnco_train_nab_backward(int64_t n_inst, int32_t n_nodes, const float* coords, const float* cost, int32_t transpose_cost,
+                             const float* packed, const float* params, float scale, const float* grad_out, void* workspace,
+                             float* grads, void* stream);
 
 #ifdef __cplusplus
 }

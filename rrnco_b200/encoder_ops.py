@@ -3,7 +3,9 @@
 `DistAngleFusion` mirrors `rrnco/models/nn/attn_freenet.py:201-289` (same constructor, same parameter names, so the
 reference module's state_dict loads unchanged); its forward is ONE kernel (`rrnco_nab_gating`) that never materialises the
 [B, N, N, E] embeddings upstream builds twice per block.  `patch_encoder` swaps it into an upstream `RRNetEncoder`
-(`encoder.net.layers[i].{row,col}_encoding_block.angle_distance_fusion`) for the inference path (test.py / validation).
+(`encoder.net.layers[i].{row,col}_encoding_block.angle_distance_fusion`) for the inference path (test.py / validation), and
+with `trainable=True` for training too: the backward of the two-way gate is one pass over the node pairs as well
+(`rrnco_train_nab_backward`, csrc_train/encoder_train.cu), so autograd keeps [B, N, N] tensors, not seven [B, N, N, E] ones.
 The duration-channel variant (rcvrptw: Linear(3E, E) -> SiLU -> Linear(E, 3) gate, softmax with a temperature) does not
 collapse to scalar functions (its gate is not linear in the embeddings): what remains after collapsing the linear layers is a
 [pairs x 3E] x [3E x E] contraction, which runs on tcgen05 (`rrnco_nab_dur_gating`, csrc/encoder_dur_kernel.cu).
@@ -17,15 +19,92 @@ from typing import Optional
 import torch
 from torch import nn
 
-from . import _lib
+from . import _lib, train_ops
 from ._lib import call, ptr, stream_ptr
 
 
+def _nab_params(m: "DistAngleFusion"):
+    """The 12 tensors of a two-way-gate module in the order of rrnco_train_nab_backward's `params` / `grads`."""
+    return [m.dist_emb[0].weight, m.dist_emb[0].bias, m.dist_emb[2].weight, m.dist_emb[2].bias,
+            m.angle_emb[0].weight, m.angle_emb[0].bias, m.angle_emb[2].weight, m.angle_emb[2].bias,
+            m.gate[0].weight, m.gate[0].bias, m.out_lin.weight, m.out_lin.bias]
+
+
+_train_checked = False
+
+
+def _train_lib():
+    """librrnco_b200_train.so, once checked to read `packed` in the layout the rollout library writes it."""
+    global _train_checked
+    h = train_ops.lib()
+    if not _train_checked:
+        if h.rrnco_train_nab_packed_floats() != _lib.lib().rrnco_nab_packed_floats():
+            raise RuntimeError("librrnco_b200_train.so and librrnco_b200.so disagree on the layout of the packed "
+                               "DistAngleFusion tables: rebuild both (python rrnco_b200/build.py --force)")
+        _train_checked = True
+    return h
+
+
+def nab_gating_backward(coords: torch.Tensor, cost: torch.Tensor, transposed: int, packed: torch.Tensor,
+                        flat_params: torch.Tensor, scale: float, grad_out: torch.Tensor) -> torch.Tensor:
+    """Parameter gradients of the two-way gate (rrnco_train_nab_backward) as one flat fp32 tensor in the layout of
+    `_nab_params`: `coords`, `cost` (the contiguous base, read transposed when `transposed`), `packed` and `scale` as the
+    forward call got them, `flat_params` the 12 parameters concatenated, `grad_out` [B, N, N]."""
+    h, dev = _train_lib(), cost.device
+    B, N, _ = cost.shape
+    nbytes = h.rrnco_train_nab_workspace_bytes(B, N)
+    train_ops._check(min(nbytes, 0), "rrnco_train_nab_workspace_bytes")
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    grads = torch.empty(h.rrnco_train_nab_grad_floats(), dtype=torch.float32, device=dev)
+    grad_out = grad_out.float().contiguous()
+    train_ops._check(h.rrnco_train_nab_backward(B, N, ptr(coords), ptr(cost), int(transposed), ptr(packed), ptr(flat_params),
+                                                float(scale), ptr(grad_out), ptr(ws), ptr(grads), stream_ptr(dev)),
+                     "rrnco_train_nab_backward")
+    return grads
+
+
+class _NabGating(torch.autograd.Function):
+    """out = DistAngleFusion.forward (two-way gate) through rrnco_nab_gating; backward = rrnco_train_nab_backward.  The
+    context keeps the `packed` buffer the forward used (a parameter update makes the module pack a NEW buffer) and a snapshot
+    of the parameters; no gradients flow to coords / cost."""
+
+    @staticmethod
+    def forward(ctx, coords, cost, transposed, scale, packed, *params):
+        B, N, _ = cost.shape
+        out = torch.empty((B, N, N), dtype=torch.float32, device=cost.device)
+        call("rrnco_nab_gating", B, N, ptr(coords), ptr(cost), transposed, ptr(packed), float(scale), 0, ptr(out),
+             stream_ptr(cost.device))
+        flat = torch.cat([p.detach().float().reshape(-1) for p in params])
+        ctx.save_for_backward(coords, cost, packed, flat)
+        ctx.transposed, ctx.scale = transposed, float(scale)
+        ctx.metas = [(p.shape, p.dtype) for p in params]
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out):
+        coords, cost, packed, flat = ctx.saved_tensors
+        with torch.cuda.device(cost.device):
+            grads = nab_gating_backward(coords, cost, ctx.transposed, packed, flat, ctx.scale, grad_out)
+        out, off = [], 0
+        for shape, dtype in ctx.metas:
+            n = shape.numel()
+            out.append(grads[off:off + n].view(shape).to(dtype))
+            off += n
+        return (None, None, None, None, None, *out)
+
+
 class DistAngleFusion(nn.Module):
-    def __init__(self, embed_dim: int = 128, use_duration_matrix: bool = False):
+    def __init__(self, embed_dim: int = 128, use_duration_matrix: bool = False, trainable: bool = False):
+        """`trainable=True`: under grad (with parameters that require it) the forward records an autograd node whose
+        backward is a CUDA kernel (rrnco_train_nab_backward); every other call is the inference kernel.  Two-way gate only."""
         super().__init__()
         if embed_dim != 128:
             raise NotImplementedError("the kernels are built for embed_dim = 128 (experiment/rrnet.yaml)")
+        if trainable and use_duration_matrix:
+            raise NotImplementedError("trainable=True: the backward kernel covers the two-way gate (ATSP / RCVRP) only, "
+                                      "not the rcvrptw duration gate")
+        self.trainable = bool(trainable)
         self.use_duration_matrix = bool(use_duration_matrix)
         self.embed_dim = embed_dim // 2 if use_duration_matrix else embed_dim  # (upstream's attribute, attn_freenet.py:210-214)
         self.dist_emb = nn.Sequential(nn.Linear(1, embed_dim), nn.ReLU(), nn.Linear(embed_dim, embed_dim))
@@ -61,9 +140,7 @@ class DistAngleFusion(nn.Module):
 
     def packed_parameters(self) -> torch.Tensor:
         """The module collapsed into four E-vectors + constants (rrnco_nab_pack); cached until a parameter changes."""
-        ps = [self.dist_emb[0].weight, self.dist_emb[0].bias, self.dist_emb[2].weight, self.dist_emb[2].bias,
-              self.angle_emb[0].weight, self.angle_emb[0].bias, self.angle_emb[2].weight, self.angle_emb[2].bias,
-              self.gate[0].weight, self.gate[0].bias, self.out_lin.weight, self.out_lin.bias]
+        ps = _nab_params(self)
         key = tuple((p.data_ptr(), p._version) for p in ps)
         if self._packed is None or self._packed_key != key:
             dev = ps[0].device
@@ -78,8 +155,13 @@ class DistAngleFusion(nn.Module):
         """adapt_bias [B, N, N] (times `scale`, e.g. the block's alpha).  `cost_mat` may be the transposed VIEW the
         col-encoding block passes (attn_freenet.py:480-486): it is read through its base, never copied.
         `variant` 0 = piecewise-linear segment tables (default), 1 = brute-force sum over the hidden units (cross-check)."""
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        record = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
+        if record and not self.trainable:
             raise NotImplementedError("forward-only kernel: call under torch.no_grad() / inference_mode (test.py path)")
+        if record and variant != 0:
+            raise NotImplementedError("trainable DistAngleFusion: the backward kernel follows the segment tables (variant 0)")
+        if record and (coords.requires_grad or cost_mat.requires_grad):
+            raise NotImplementedError("trainable DistAngleFusion: no gradients with respect to coords / cost_mat")
         if (duration_mat is not None) != self.use_duration_matrix:
             raise ValueError("duration_mat must be given exactly when the module was built with use_duration_matrix=True")
         B, N, _ = cost_mat.shape
@@ -88,6 +170,8 @@ class DistAngleFusion(nn.Module):
         if not cost_mat.is_contiguous() and cost_mat.transpose(1, 2).is_contiguous():
             cost_mat, transposed = cost_mat.transpose(1, 2), 1
         cost_mat = cost_mat.float().contiguous()
+        if record:  # (trainable: two-way gate only)
+            return _NabGating.apply(coords, cost_mat, transposed, float(scale), self.packed_parameters(), *_nab_params(self))
         out = torch.empty((B, N, N), dtype=torch.float32, device=cost_mat.device)
         if self.use_duration_matrix:  # three-way gate: tcgen05 kernel (encoder_dur_kernel.cu)
             dur = duration_mat
@@ -147,14 +231,19 @@ def _fused_block_forward(self, row_emb, col_emb, cost_mat, coords, duration_mat=
     return self.feed_forward(multi_head_out, row_emb)
 
 
-def patch_encoder(encoder: nn.Module, fuse_aft: bool = True) -> int:
+def patch_encoder(encoder: nn.Module, fuse_aft: bool = True, trainable: bool = False) -> int:
     """Replaces every gating `DistAngleFusion` without duration channel inside an upstream encoder (attribute
     `angle_distance_fusion` of the attention-free blocks, attn_freenet.py:386-389) by the kernel-backed module with the
     same parameters, and (fuse_aft, instances of <= 128 nodes) routes the block's bias -> AFT-full chain through the fused
-    kernel.  Inference path only.  Returns the number of blocks patched."""
+    kernel.  Inference path only, unless `trainable`: then the swapped modules are `DistAngleFusion(trainable=True)` that
+    hold upstream's own parameter tensors (an optimizer built before the patch keeps training them), the rcvrptw
+    duration-gate modules stay upstream's, and the fused block runs under torch.no_grad() only (under grad the block is
+    upstream's forward around the trainable module).  Returns the number of blocks patched."""
     import types
     n = 0
     for block in encoder.modules():
+        if trainable and hasattr(getattr(block, "neural_adaptive_bias", None), "dur_emb"):
+            continue
         # rcvrptw blocks: attribute `neural_adaptive_bias` holding a DistAngleFusion with the duration channel (:380-384)
         refd = getattr(block, "neural_adaptive_bias", None)
         if refd is not None and not isinstance(refd, DistAngleFusion) and hasattr(refd, "dur_emb") and hasattr(refd, "gate_temperature"):
@@ -175,8 +264,10 @@ def patch_encoder(encoder: nn.Module, fuse_aft: bool = True) -> int:
         ref = getattr(block, "angle_distance_fusion", None)
         if ref is None or isinstance(ref, DistAngleFusion) or hasattr(ref, "dur_emb"):
             continue
-        mine = DistAngleFusion(ref.embed_dim).to(next(ref.parameters()).device)
+        mine = DistAngleFusion(ref.embed_dim, trainable=trainable).to(next(ref.parameters()).device)
         mine.load_state_dict(ref.state_dict(), strict=True)
+        if trainable:
+            mine.dist_emb, mine.angle_emb, mine.gate, mine.out_lin = ref.dist_emb, ref.angle_emb, ref.gate, ref.out_lin
         block.angle_distance_fusion = mine
         if fuse_aft and all(hasattr(block, a) for a in ("attn_free", "norm1", "norm2", "norm3", "multi_head_combine",
                                                         "feed_forward", "alpha")):

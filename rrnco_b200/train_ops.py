@@ -37,6 +37,10 @@ _SIGNATURES = {
     "rrnco_train_inst_pack": (C.c_int, [C.c_int64, C.c_int32, _f, C.c_int32, _f, _f, _f]),
     "rrnco_train_inst_gemm": (C.c_int, [C.c_int64, C.c_int64, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_train_inst_xty": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f]),
+    "rrnco_train_nab_packed_floats": (C.c_int64, []),
+    "rrnco_train_nab_grad_floats": (C.c_int64, []),
+    "rrnco_train_nab_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
+    "rrnco_train_nab_backward": (C.c_int, [C.c_int64, C.c_int32, _f, _f, C.c_int32, _f, _f, C.c_float, _f, _f, _f, _f]),
 }
 _lib = None
 _status: dict = {}
