@@ -18,6 +18,7 @@
  *   rrnco_train_logits_tail edge bias, log(exp(.) + 1e-6), tanh clip, mask, temperature, log-softmax and the log-prob of
  *                           the given action with its Jacobian, in one pass (decoder.py:183-198, decoding.py:311-399)
  *   rrnco_train_nab_backward the parameter gradients of the encoder's gating neural adaptive bias (attn_freenet.py:242-289)
+ *   rrnco_train_nab_dur_backward  the same for the rcvrptw three-way (duration) gate
  *
  * Conventions as in rrnco_b200.h: plain pointers and sizes, device pointers unless noted, return 0 = RRNCO_OK or a negative
  * error, `stream` = cudaStream_t (NULL = default stream), `status` = sticky device word (RRNCO_DEV_NAN_LOGITS when an fp16
@@ -129,6 +130,24 @@ int64_t rrnco_train_nab_workspace_bytes(int64_t n_inst, int32_t n_nodes);
 int rrnco_train_nab_backward(int64_t n_inst, int32_t n_nodes, const float* coords, const float* cost, int32_t transpose_cost,
                              const float* packed, const float* params, float scale, const float* grad_out, void* workspace,
                              float* grads, void* stream);
+
+/* Backward of the rcvrptw three-way (duration) gate of the neural adaptive bias (DistAngleFusion.forward with
+ * use_duration_matrix), the forward of which is rrnco_nab_dur_gating (rrnco_b200.h):
+ *   coords, cost, duration, transpose, `packed` and `scale` exactly as the forward call got them; grad_out [n_inst, N, N].
+ *   params / grads: the 19 tensors in the pointer order of rrnco_nab_dur_pack (dist / angle / dur emb.0.weight, emb.0.bias,
+ *   emb.2.weight, emb.2.bias, gate.0.weight [E,3E], gate.0.bias, gate.2.weight [3,E], gate.2.bias, gate_temperature,
+ *   out_lin.weight, out_lin.bias), concatenated (rrnco_train_nab_dur_grad_floats() floats); grads are written, not accumulated.
+ *   workspace: rrnco_train_nab_dur_workspace_bytes(n_inst, n_nodes) bytes (depends on the SM count, not on n_inst), 16-byte
+ *   aligned.  status: RRNCO_DEV_NAN_LOGITS is or-ed in when an fp16 operand overflows or a value is not finite.
+ * Two tcgen05 passes over the pairs (each recomputes the forward), nothing of size [n_inst, N, N, E]; no float atomics: the
+ * gradients are bitwise identical run to run on one device.  No gradients for coords / cost / duration.
+ * rrnco_train_nab_dur_packed_bytes() = the size of `packed` this library expects (= rrnco_nab_dur_packed_bytes()). */
+int64_t rrnco_train_nab_dur_packed_bytes(void);
+int64_t rrnco_train_nab_dur_grad_floats(void);
+int64_t rrnco_train_nab_dur_workspace_bytes(int64_t n_inst, int32_t n_nodes);
+int rrnco_train_nab_dur_backward(int64_t n_inst, int32_t n_nodes, const float* coords, const float* cost, const float* duration,
+                                 int32_t transpose, const void* packed, const float* params, float scale, const float* grad_out,
+                                 void* workspace, float* grads, uint32_t* status, void* stream);
 
 #ifdef __cplusplus
 }

@@ -8,7 +8,10 @@ with `trainable=True` for training too: the backward of the two-way gate is one 
 (`rrnco_train_nab_backward`, csrc_train/encoder_train.cu), so autograd keeps [B, N, N] tensors, not seven [B, N, N, E] ones.
 The duration-channel variant (rcvrptw: Linear(3E, E) -> SiLU -> Linear(E, 3) gate, softmax with a temperature) does not
 collapse to scalar functions (its gate is not linear in the embeddings): what remains after collapsing the linear layers is a
-[pairs x 3E] x [3E x E] contraction, which runs on tcgen05 (`rrnco_nab_dur_gating`, csrc/encoder_dur_kernel.cu).
+[pairs x 3E] x [3E x E] contraction, which runs on tcgen05 (`rrnco_nab_dur_gating`, csrc/encoder_dur_kernel.cu).  With
+`train_duration_gate=True` it trains too: its backward (`rrnco_train_nab_dur_backward`, csrc_train/encoder_dur_train.cu) is
+six E x E contractions over the pairs on tcgen05 plus small sums, so autograd keeps [B, N, N] tensors, not twelve
+[B, N, N, E] ones.
 No CPU fallback: a host tensor or a missing library raises.
 """
 from __future__ import annotations
@@ -30,7 +33,16 @@ def _nab_params(m: "DistAngleFusion"):
             m.gate[0].weight, m.gate[0].bias, m.out_lin.weight, m.out_lin.bias]
 
 
+def _dur_params(m: "DistAngleFusion"):
+    """The 19 tensors of a duration-gate module in the pointer order of rrnco_nab_dur_pack (= rrnco_train_nab_dur_backward's
+    `params` / `grads`)."""
+    return [*(q for seq in (m.dist_emb, m.angle_emb, m.dur_emb) for q in (seq[0].weight, seq[0].bias, seq[2].weight, seq[2].bias)),
+            m.gate[0].weight, m.gate[0].bias, m.gate[2].weight, m.gate[2].bias, m.gate_temperature,
+            m.out_lin.weight, m.out_lin.bias]
+
+
 _train_checked = False
+_dur_train_checked = False
 
 
 def _train_lib():
@@ -43,6 +55,43 @@ def _train_lib():
                                "DistAngleFusion tables: rebuild both (python rrnco_b200/build.py --force)")
         _train_checked = True
     return h
+
+
+def _dur_train_lib():
+    """librrnco_b200_train.so, once checked to read the duration gate's `packed` in the layout the rollout library writes."""
+    global _dur_train_checked
+    h = train_ops.lib()
+    if not _dur_train_checked:
+        if h.rrnco_train_nab_dur_packed_bytes() != _lib.lib().rrnco_nab_dur_packed_bytes():
+            raise RuntimeError("librrnco_b200_train.so and librrnco_b200.so disagree on the layout of the packed "
+                               "duration-gate tables: rebuild both (python rrnco_b200/build.py --force)")
+        _dur_train_checked = True
+    return h
+
+
+def nab_dur_gating_backward(coords: torch.Tensor, cost: torch.Tensor, dur: torch.Tensor, transposed: int,
+                            packed: torch.Tensor, flat_params: torch.Tensor, scale: float,
+                            grad_out: torch.Tensor) -> torch.Tensor:
+    """Parameter gradients of the duration gate (rrnco_train_nab_dur_backward) as one flat fp32 tensor in the layout of
+    `_dur_params`: `coords`, `cost` / `dur` (the contiguous bases, read transposed when `transposed`), `packed` and `scale`
+    as the forward call got them, `flat_params` the 19 parameters concatenated, `grad_out` [B, N, N].  An fp16 operand
+    overflow or a non-finite value raises."""
+    h, dev = _dur_train_lib(), cost.device
+    B, N, _ = cost.shape
+    nbytes = h.rrnco_train_nab_dur_workspace_bytes(B, N)
+    train_ops._check(min(nbytes, 0), "rrnco_train_nab_dur_workspace_bytes")
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    grads = torch.empty(h.rrnco_train_nab_dur_grad_floats(), dtype=torch.float32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    grad_out = grad_out.float().contiguous()
+    train_ops._check(h.rrnco_train_nab_dur_backward(B, N, ptr(coords), ptr(cost), ptr(dur), int(transposed), ptr(packed),
+                                                    ptr(flat_params), float(scale), ptr(grad_out), ptr(ws), ptr(grads),
+                                                    ptr(status), stream_ptr(dev)),
+                     "rrnco_train_nab_dur_backward")
+    if int(status.item()):
+        raise AssertionError("DistAngleFusion backward: an fp16 operand overflowed (pair scalar >= 4094 or a gradient far "
+                             "outside the range of the others) or a value is not finite")
+    return grads
 
 
 def nab_gating_backward(coords: torch.Tensor, cost: torch.Tensor, transposed: int, packed: torch.Tensor,
@@ -94,16 +143,52 @@ class _NabGating(torch.autograd.Function):
         return (None, None, None, None, None, *out)
 
 
+class _NabDurGating(torch.autograd.Function):
+    """out = DistAngleFusion.forward (duration gate) through rrnco_nab_dur_gating, with its status check; backward =
+    rrnco_train_nab_dur_backward.  The context keeps the `packed` buffer the forward used and a snapshot of the parameters;
+    no gradients flow to coords / cost / duration."""
+
+    @staticmethod
+    def forward(ctx, coords, cost, dur, transposed, scale, packed, check, *params):
+        B, N, _ = cost.shape
+        out = torch.empty((B, N, N), dtype=torch.float32, device=cost.device)
+        status = torch.zeros(1, dtype=torch.int32, device=cost.device)
+        call("rrnco_nab_dur_gating", B, N, ptr(coords), ptr(cost), ptr(dur), transposed, ptr(packed), float(scale), ptr(out),
+             ptr(status), stream_ptr(cost.device))
+        if check and int(status.item()):
+            raise AssertionError("DistAngleFusion: hidden activations outside the fp16 operand range (>= 4094)")
+        flat = torch.cat([p.detach().float().reshape(-1) for p in params])
+        ctx.save_for_backward(coords, cost, dur, packed, flat)
+        ctx.transposed, ctx.scale = transposed, float(scale)
+        ctx.metas = [(p.shape, p.dtype) for p in params]
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_out):
+        coords, cost, dur, packed, flat = ctx.saved_tensors
+        with torch.cuda.device(cost.device):
+            grads = nab_dur_gating_backward(coords, cost, dur, ctx.transposed, packed, flat, ctx.scale, grad_out)
+        out, off = [], 0
+        for shape, dtype in ctx.metas:
+            n = shape.numel()
+            out.append(grads[off:off + n].view(shape).to(dtype))
+            off += n
+        return (None, None, None, None, None, None, None, *out)
+
+
 class DistAngleFusion(nn.Module):
-    def __init__(self, embed_dim: int = 128, use_duration_matrix: bool = False, trainable: bool = False):
+    def __init__(self, embed_dim: int = 128, use_duration_matrix: bool = False, trainable: bool = False,
+                 train_duration_gate: bool = False):
         """`trainable=True`: under grad (with parameters that require it) the forward records an autograd node whose
-        backward is a CUDA kernel (rrnco_train_nab_backward); every other call is the inference kernel.  Two-way gate only."""
+        backward is a CUDA kernel (rrnco_train_nab_backward); every other call is the inference kernel.  The duration gate
+        (`use_duration_matrix=True`) trains only with `train_duration_gate=True` as well (rrnco_train_nab_dur_backward)."""
         super().__init__()
         if embed_dim != 128:
             raise NotImplementedError("the kernels are built for embed_dim = 128 (experiment/rrnet.yaml)")
-        if trainable and use_duration_matrix:
-            raise NotImplementedError("trainable=True: the backward kernel covers the two-way gate (ATSP / RCVRP) only, "
-                                      "not the rcvrptw duration gate")
+        if trainable and use_duration_matrix and not train_duration_gate:
+            raise NotImplementedError("trainable=True: the backward kernel covers the two-way gate (ATSP / RCVRP); the "
+                                      "rcvrptw duration gate trains with train_duration_gate=True")
         self.trainable = bool(trainable)
         self.use_duration_matrix = bool(use_duration_matrix)
         self.embed_dim = embed_dim // 2 if use_duration_matrix else embed_dim  # (upstream's attribute, attn_freenet.py:210-214)
@@ -170,7 +255,7 @@ class DistAngleFusion(nn.Module):
         if not cost_mat.is_contiguous() and cost_mat.transpose(1, 2).is_contiguous():
             cost_mat, transposed = cost_mat.transpose(1, 2), 1
         cost_mat = cost_mat.float().contiguous()
-        if record:  # (trainable: two-way gate only)
+        if record and not self.use_duration_matrix:
             return _NabGating.apply(coords, cost_mat, transposed, float(scale), self.packed_parameters(), *_nab_params(self))
         out = torch.empty((B, N, N), dtype=torch.float32, device=cost_mat.device)
         if self.use_duration_matrix:  # three-way gate: tcgen05 kernel (encoder_dur_kernel.cu)
@@ -178,6 +263,11 @@ class DistAngleFusion(nn.Module):
             if transposed:  # the col-encoding block transposes both matrices (attn_freenet.py:476-486)
                 dur = dur.transpose(1, 2)
             dur = dur.float().contiguous()
+            if record:
+                if duration_mat.requires_grad:
+                    raise NotImplementedError("trainable DistAngleFusion: no gradients with respect to duration_mat")
+                return _NabDurGating.apply(coords, cost_mat, dur, transposed, float(scale), self._packed_duration(),
+                                           self.check_overflow, *_dur_params(self))
             status = torch.zeros(1, dtype=torch.int32, device=out.device)
             call("rrnco_nab_dur_gating", B, N, ptr(coords), ptr(cost_mat), ptr(dur), transposed, ptr(self._packed_duration()),
                  float(scale), ptr(out), ptr(status), stream_ptr(out.device))
@@ -231,24 +321,31 @@ def _fused_block_forward(self, row_emb, col_emb, cost_mat, coords, duration_mat=
     return self.feed_forward(multi_head_out, row_emb)
 
 
-def patch_encoder(encoder: nn.Module, fuse_aft: bool = True, trainable: bool = False) -> int:
+def patch_encoder(encoder: nn.Module, fuse_aft: bool = True, trainable: bool = False, train_duration_gate: bool = False) -> int:
     """Replaces every gating `DistAngleFusion` without duration channel inside an upstream encoder (attribute
     `angle_distance_fusion` of the attention-free blocks, attn_freenet.py:386-389) by the kernel-backed module with the
     same parameters, and (fuse_aft, instances of <= 128 nodes) routes the block's bias -> AFT-full chain through the fused
     kernel.  Inference path only, unless `trainable`: then the swapped modules are `DistAngleFusion(trainable=True)` that
     hold upstream's own parameter tensors (an optimizer built before the patch keeps training them), the rcvrptw
     duration-gate modules stay upstream's, and the fused block runs under torch.no_grad() only (under grad the block is
-    upstream's forward around the trainable module).  Returns the number of blocks patched."""
+    upstream's forward around the trainable module).  With `train_duration_gate` as well, the rcvrptw modules are swapped
+    too, for `DistAngleFusion(use_duration_matrix=True, trainable=True, train_duration_gate=True)` holding upstream's 19
+    parameter tensors (gate_temperature included).  Returns the number of blocks patched."""
     import types
     n = 0
     for block in encoder.modules():
-        if trainable and hasattr(getattr(block, "neural_adaptive_bias", None), "dur_emb"):
+        if trainable and not train_duration_gate and hasattr(getattr(block, "neural_adaptive_bias", None), "dur_emb"):
             continue
         # rcvrptw blocks: attribute `neural_adaptive_bias` holding a DistAngleFusion with the duration channel (:380-384)
         refd = getattr(block, "neural_adaptive_bias", None)
         if refd is not None and not isinstance(refd, DistAngleFusion) and hasattr(refd, "dur_emb") and hasattr(refd, "gate_temperature"):
-            mine = DistAngleFusion(128, use_duration_matrix=True).to(next(refd.parameters()).device)
+            mine = DistAngleFusion(128, use_duration_matrix=True, trainable=trainable,
+                                   train_duration_gate=trainable).to(next(refd.parameters()).device)
             mine.load_state_dict(refd.state_dict(), strict=True)
+            if trainable:  # upstream's own tensors: an optimizer built before the patch keeps training them
+                mine.dist_emb, mine.angle_emb, mine.dur_emb, mine.gate, mine.out_lin = (
+                    refd.dist_emb, refd.angle_emb, refd.dur_emb, refd.gate, refd.out_lin)
+                mine.gate_temperature = refd.gate_temperature
             block.neural_adaptive_bias = mine
             if fuse_aft and all(hasattr(block, a) for a in ("attn_free", "norm1", "norm2", "norm3", "multi_head_combine",
                                                             "feed_forward", "alpha")):

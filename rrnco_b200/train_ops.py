@@ -41,6 +41,11 @@ _SIGNATURES = {
     "rrnco_train_nab_grad_floats": (C.c_int64, []),
     "rrnco_train_nab_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
     "rrnco_train_nab_backward": (C.c_int, [C.c_int64, C.c_int32, _f, _f, C.c_int32, _f, _f, C.c_float, _f, _f, _f, _f]),
+    "rrnco_train_nab_dur_packed_bytes": (C.c_int64, []),
+    "rrnco_train_nab_dur_grad_floats": (C.c_int64, []),
+    "rrnco_train_nab_dur_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
+    "rrnco_train_nab_dur_backward": (C.c_int, [C.c_int64, C.c_int32, _f, _f, _f, C.c_int32, _f, _f, C.c_float, _f, _f, _f, _f,
+                                               _f]),
 }
 _lib = None
 _status: dict = {}
