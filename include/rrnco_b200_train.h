@@ -12,9 +12,10 @@
  *   rrnco_train_xty         C += X^T Y over millions of rows (weight gradients dW1 = dH^T x, dW2^T = H^T dy), with the
  *                           column sums of X and Y (bias gradients) from the same pass
  *   rrnco_train_attention   masked 8-head attention of one query row per (rollout, step) over the instance's keys
- *                           (decoder.py:281-293), forward and backward
+ *                           (decoder.py:281-293), forward and backward; _tiled: the same for up to 1024 nodes
  *   rrnco_train_context_query  the context projection as a table gather + rank-k update (context.py:18-70), forward / backward
- *   rrnco_train_inst_gemm / _xty  the pointer scores g . Lk^T and their gradients, one weight tile per instance (decoder.py:298-301)
+ *   rrnco_train_inst_gemm / _xty  the pointer scores g . Lk^T and their gradients, one weight tile per instance (decoder.py:298-301);
+ *                           rrnco_train_inst_tiled_*: the same with ceil(N / 128) key tiles per instance, up to 1024 nodes
  *   rrnco_train_logits_tail edge bias, log(exp(.) + 1e-6), tanh clip, mask, temperature, log-softmax and the log-prob of
  *                           the given action with its Jacobian, in one pass (decoder.py:183-198, decoding.py:311-399)
  *   rrnco_train_nab_backward the parameter gradients of the encoder's gating neural adaptive bias (attn_freenet.py:242-289)
@@ -74,13 +75,27 @@ int rrnco_train_attention_bwd(int64_t n_inst, int64_t rows_per_inst, int32_t n_n
                               const uint8_t* mask, const float* out, int32_t add_residual, const float* lse, const float* d_out,
                               float* dq, float* dk, float* dv, void* stream);
 
+/* The attention above (decoder.py:281-293) for n_nodes <= 1024: the same arguments, math and lse convention, with the keys streamed
+ * through shared memory in tiles of 32 (online softmax across the tiles; CUDA cores, fp32 FMAs).  The forward visits the keys in the
+ * order and with the arithmetic of rrnco_train_attention_fwd (bitwise equal outputs measured at 101 nodes).
+ * backward:  dq from row groups that loop over the key tiles; dk / dv from (instance, key tile, row split) work items whose
+ *            partials are added in a fixed order (no float atomics: bitwise reproducible run to run on one device); dk / dv are
+ *            written, not accumulated.  workspace: rrnco_train_attention_tiled_workspace_bytes(n_inst, rows_per_inst, n_nodes)
+ *            bytes (depends on the current device's SM count), 16-byte aligned: D = dO . attn [rows, 8] and the split partials. */
+int64_t rrnco_train_attention_tiled_workspace_bytes(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes);
+int rrnco_train_attention_tiled_fwd(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* q, const float* k,
+                                    const float* v, const uint8_t* mask, int32_t add_residual, float* out, float* lse, void* stream);
+int rrnco_train_attention_tiled_bwd(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* q, const float* k,
+                                    const float* v, const uint8_t* mask, const float* out, int32_t add_residual, const float* lse,
+                                    const float* d_out, void* workspace, float* dq, float* dk, float* dv, void* stream);
+
 /* Tail of the pointer for the batched replay (decoder.py:183-198 edge bias + log(exp(.) + 1e-6); decoding.py:311-361 tanh clip,
  * mask, temperature; :386-399 log-prob of the given action), one pass:
- *   z [rows, ldz] (in / out; row stride ldz >= n_nodes, <= 128): raw pointer scores g . Lk^T on entry, J = d logp / d z on return
+ *   z [rows, ldz] (in / out; row stride ldz >= n_nodes, <= 1024): raw pointer scores g . Lk^T on entry, J = d logp / d z on return
  *   (backward: dz = g_row J; padding columns are zeroed)
  *   distance / duration [n_inst, n_nodes, n_nodes] (duration NULL except rcvrptw), instance of a row = row / rows_per_inst
  *   current_node / action [rows] int64, mask [rows, n_nodes] bytes, alpha / beta device scalars (decoder.alpha / .beta)
- *   logp [rows] = log pi(action | state);  dlogp_dalpha / dlogp_dbeta [rows] (beta: NULL without duration);  n_nodes <= 128 */
+ *   logp [rows] = log pi(action | state);  dlogp_dalpha / dlogp_dbeta [rows] (beta: NULL without duration);  n_nodes <= 1024 */
 int rrnco_train_logits_tail(int64_t rows, int64_t rows_per_inst, int32_t n_nodes, int32_t ldz, float* z, const float* distance,
                             const float* duration, const int64_t* current_node, const uint8_t* mask, const int64_t* action,
                             const float* alpha, const float* beta, float inv_sqrt_e, float tanh_clipping, float temperature,
@@ -112,6 +127,24 @@ int rrnco_train_inst_gemm(int64_t n_inst, int64_t rows_per_inst, const float* x,
                           const float* row_scale, float* y, uint32_t* status, void* stream);
 int rrnco_train_inst_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* x, const float* y, const float* sx,
                          const float* sy, const float* row_scale, float* c, uint32_t* status, void* stream);
+
+/* Pointer scores (decoder.py:298-301) for n_nodes <= 1024, with n_kt = ceil(n_nodes / 128) zero-padded 128 x 128 weight tiles per
+ * instance and score rows ldz = 128 n_kt wide (padding columns are zero); operand scales, row_scale and status as above:
+ *   rrnco_train_inst_tiled_pack   w [n_inst, n_nodes, 128] -> packed (rrnco_train_inst_tiled_packed_bytes(n_inst, n_nodes) bytes),
+ *                                 transpose as for rrnco_train_inst_pack, per key tile
+ *   rrnco_train_inst_tiled_gemm   transpose == 0: y [n_inst L, ldz] = x [n_inst L, 128] B_b    (z = g Lk^T, one column block per tile)
+ *                                 transpose == 1: y [n_inst L, 128] = x [n_inst L, ldz] B_b    (dg = dz Lk, the key tiles summed in TMEM)
+ *                                 (`packed` packed with the same transpose)
+ *   rrnco_train_inst_tiled_xty    c [n_inst, n_nodes, 128] += x_b^T y_b, x [n_inst L, ldz], y [n_inst L, 128], per (instance, key
+ *                                 tile) (dLk_b = dz_b^T g_b; fp32 atomics) */
+int64_t rrnco_train_inst_tiled_packed_bytes(int64_t n_inst, int32_t n_nodes);
+int rrnco_train_inst_tiled_pack(int64_t n_inst, int32_t n_nodes, const float* w, int32_t transpose, void* packed, uint32_t* status,
+                                void* stream);
+int rrnco_train_inst_tiled_gemm(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, int32_t transpose, const float* x,
+                                const void* packed, const float* a_scale, const float* row_scale, float* y, uint32_t* status,
+                                void* stream);
+int rrnco_train_inst_tiled_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* x, const float* y, const float* sx,
+                               const float* sy, const float* row_scale, float* c, uint32_t* status, void* stream);
 
 /* Backward of the encoder's gating neural adaptive bias (DistAngleFusion.forward, rrnco/models/nn/attn_freenet.py:242-289,
  * the two-way gate of ATSP / RCVRP), the forward of which is rrnco_nab_gating (rrnco_b200.h):

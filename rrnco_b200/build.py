@@ -96,8 +96,8 @@ def build_torch_ops(force: bool = False) -> str:
 
 
 TRAIN_LIB = os.path.join(HERE, "librrnco_b200_train.so")
-TRAIN_SOURCES = ["ffn_train.cu", "attention_train.cu", "logits_train.cu", "context_train.cu", "pointer_train.cu", "encoder_train.cu",
-                 "encoder_dur_train.cu"]
+TRAIN_SOURCES = ["ffn_train.cu", "attention_train.cu", "attention_tiled_train.cu", "logits_train.cu", "context_train.cu",
+                 "pointer_train.cu", "encoder_train.cu", "encoder_dur_train.cu"]
 
 
 def build_train_library(force: bool = False) -> str:

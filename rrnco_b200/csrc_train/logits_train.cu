@@ -5,6 +5,7 @@
 //   z[row, :]  (in place) <- J = d logp / d z        (the backward pass is then  dz = g_row J, one multiply)
 //   a_out[row], b_out[row] = d logp / d alpha, d logp / d beta
 // instead of ~25 element-wise ATen passes over [rows, N] tensors (forward + autograd), none of which is saved.
+// EPL = elements per lane: 4 for rows of up to 128 scores, 32 for up to 1024 (the key-tiled pointer scores of larger instances).
 #include "../csrc/common.cuh"
 #include "../../include/rrnco_b200_train.h"
 
@@ -16,6 +17,7 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+template <int EPL>
 __global__ void __launch_bounds__(256) logits_tail_kernel(int64_t rows, int64_t L, int N, int ldz, float* __restrict__ z,
                                                          const float* __restrict__ dist, const float* __restrict__ dur,
                                                          const int64_t* __restrict__ cur, const uint8_t* __restrict__ mask,
@@ -34,10 +36,10 @@ __global__ void __launch_bounds__(256) logits_tail_kernel(int64_t rows, int64_t 
     const float* urow = dur != nullptr ? dur + (b * N + c) * N : nullptr;
     float* zrow = z + row * ldz;
     const uint8_t* mrow = mask + row * N;
-    float lj[4], dj[4], uj[4], fac[4];  // clipped logit / T, distance, duration, d l / d x
+    float lj[EPL], dj[EPL], uj[EPL], fac[EPL];  // clipped logit / T, distance, duration, d l / d x
     float mx = -INFINITY;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < EPL; ++i) {
       const int j = lane + 32 * i;
       lj[i] = -INFINITY;
       dj[i] = uj[i] = fac[i] = 0.f;
@@ -65,19 +67,21 @@ __global__ void __launch_bounds__(256) logits_tail_kernel(int64_t rows, int64_t 
       }
     }
     mx = warp_max(mx);
-    float se = 0.f, ej[4];
+    float se = 0.f, ej[EPL];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < EPL; ++i) {
       ej[i] = lj[i] > -INFINITY ? expf(lj[i] - mx) : 0.f;
       se += ej[i];
     }
     se = warp_sum(se);
     const float lse = mx + logf(se), inv_se = 1.0f / se;
-    float la = (a >> 5) == 0 ? lj[0] : (a >> 5) == 1 ? lj[1] : (a >> 5) == 2 ? lj[2] : lj[3];
+    float la = lj[0];
+#pragma unroll
+    for (int i = 1; i < EPL; ++i) la = (a >> 5) >= i ? lj[i] : la;   // a < N: lj[a >> 5]
     la = __shfl_sync(0xffffffffu, la, a & 31);
     float sa = 0.f, sb = 0.f;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < EPL; ++i) {
       const int j = lane + 32 * i;
       if (j < N) {
         float dx = 0.f;  // d logp / d x_j
@@ -86,7 +90,7 @@ __global__ void __launch_bounds__(256) logits_tail_kernel(int64_t rows, int64_t 
         sa = fmaf(-dx, dj[i], sa);
         sb = fmaf(-dx, uj[i], sb);
       } else if (j < ldz) {
-        zrow[j] = 0.f;   // padding columns of a 128-wide score row
+        zrow[j] = 0.f;   // padding columns of a 128 ceil(N / 128)-wide score row
       }
     }
     sa = warp_sum(sa);
@@ -114,13 +118,14 @@ int rrnco_train_logits_tail(int64_t rows, int64_t rows_per_inst, int32_t n_nodes
                   dlogp_dalpha && temperature > 0.f);
   RRNCO_CHECK_ARG(duration == nullptr || (beta != nullptr && dlogp_dbeta != nullptr));
   RRNCO_CHECK_ARG(ldz >= n_nodes);
-  if (n_nodes > 128 || ldz > 128) return RRNCO_ERR_UNSUPPORTED;
+  if (n_nodes > 1024 || ldz > 1024) return RRNCO_ERR_UNSUPPORTED;
   const int sms = device_sm_count();
   int64_t grid = (rows + 7) / 8;
   if (grid > 16LL * sms) grid = 16LL * sms;
-  logits_tail_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(rows, rows_per_inst, n_nodes, ldz, z, distance, duration, current_node,
-                                                                    mask, action, alpha, beta, inv_sqrt_e, tanh_clipping,
-                                                                    1.0f / temperature, logp, dlogp_dalpha, dlogp_dbeta);
+  auto kernel = ldz <= 128 ? logits_tail_kernel<4> : logits_tail_kernel<32>;
+  kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(rows, rows_per_inst, n_nodes, ldz, z, distance, duration, current_node, mask,
+                                                          action, alpha, beta, inv_sqrt_e, tanh_clipping, 1.0f / temperature, logp,
+                                                          dlogp_dalpha, dlogp_dbeta);
   return rrnco_launch_status();
 }
 

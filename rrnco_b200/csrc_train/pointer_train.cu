@@ -5,6 +5,9 @@
 //                      forward:  z  = g  Lk_b^T  (columns >= n_nodes are zero)        backward:  dg = dz Lk_b
 //   xty_inst_kernel    C_b[n_nodes, 128] = X_b^T Y_b over the rows of instance b    (dLk_b = dz_b^T g_b)
 // Scores / their gradients are kept 128 wide (row stride 128 floats): thread-per-row epilogues then store whole sectors.
+// Instances of more than 128 nodes (the rrnco_train_inst_tiled_* entry points) use ceil(N / 128) weight tiles per instance, and
+// scores rows ldz = 128 ceil(N / 128) wide: the forward writes one 128-column block per tile (grid z), dg accumulates the key tiles
+// in TMEM (the weight tile is reloaded per key tile), and dLk_b is computed per (instance, key tile) (grid z).
 #include "../csrc/common.cuh"
 #include "../csrc/tc05.cuh"
 #include "../csrc/ffn_pack.cuh"
@@ -15,27 +18,29 @@ namespace rrnco {
 constexpr int kPtThreads = 288;
 constexpr uint32_t kPtTileBytes = kFRows * kE * 2;  // one fp16 variant of a 128 x 128 tile: 32 KB
 constexpr float kPtMax = 65504.f;
+constexpr int kPtMaxNodes = 1024;   // the rrnco_train_inst_tiled_* entry points: up to 8 key tiles
 
-// [n_inst, N, 128] -> per instance [hi | lo][16-byte K chunk (16)][row n (128)][8 halves];
-// transpose == 0: B[n = node][k = e] (z = g Lk^T), transpose == 1: B[n = e][k = node] (dg = dz Lk); rows / k beyond N are zero
+// [n_inst, N, 128] -> per (instance, key tile) [hi | lo][16-byte K chunk (16)][row n (128)][8 halves], key tile = grid z;
+// transpose == 0: B[n = node][k = e] (z = g Lk^T), transpose == 1: B[n = e][k = node] (dg = dz Lk); nodes beyond N are zero
 __global__ void pack_inst_weights_kernel(const float* __restrict__ src, int N, int transpose, uint32_t* __restrict__ packed,
                                          uint32_t* __restrict__ status) {
   const int64_t b = blockIdx.y;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;  // (row n, k pair)
   if (i >= kFRows * (kE / 2)) return;
-  const int n = i >> 6, kp = i & 63, k = kp * 2;
-  const float* s = src + b * N * kE;
+  const int n = i >> 6, kp = i & 63, k = kp * 2, j0 = blockIdx.z * kFRows;
+  const float* s = src + (b * N + j0) * kE;
+  const int nj = N - j0;   // nodes of this key tile (> 128: the tile is full)
   float v0 = 0.f, v1 = 0.f;
   if (!transpose) {
-    if (n < N) { v0 = s[n * kE + k]; v1 = s[n * kE + k + 1]; }
+    if (n < nj) { v0 = s[n * kE + k]; v1 = s[n * kE + k + 1]; }
   } else {
-    if (k < N) v0 = s[k * kE + n];
-    if (k + 1 < N) v1 = s[(k + 1) * kE + n];
+    if (k < nj) v0 = s[k * kE + n];
+    if (k + 1 < nj) v1 = s[(k + 1) * kE + n];
   }
   if (!(fabsf(v0) * kLkScale < kPtMax) || !(fabsf(v1) * kLkScale < kPtMax)) atomicOr(status, RRNCO_DEV_NAN_LOGITS);
   uint32_t hi, lo;
   f16s_split2(v0, v1, kLkScale, hi, lo);
-  uint32_t* dst = packed + b * (2 * kPtTileBytes / 4) + (kp >> 2) * (kFRows * 4) + n * 4 + (kp & 3);
+  uint32_t* dst = packed + (b * gridDim.z + blockIdx.z) * (2 * kPtTileBytes / 4) + (kp >> 2) * (kFRows * 4) + n * 4 + (kp & 3);
   dst[0] = hi;
   dst[kPtTileBytes / 4] = lo;
 }
@@ -50,7 +55,10 @@ struct InstGemmSmem {
   uint32_t tmem_base;
 };
 
-__global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int rows_per_cta, const float* __restrict__ X,
+// Y[rows, grid z tiles of 128 columns] (row stride ldy) = sum over nk key tiles of X[rows, key tile] (row stride ldx) B_(b, z, kt):
+// nk == 1, one column block: the 128-node form; weight tile (b, z, kt) at packed index (b gridDim.z + z) nk + kt
+__global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int rows_per_cta, int ldx, int nk, int ldy,
+                                                                 const float* __restrict__ X,
                                                                  const unsigned char* __restrict__ packed,
                                                                  const float* __restrict__ a_scale_ptr,
                                                                  const float* __restrict__ row_scale, float* __restrict__ Y,
@@ -77,27 +85,37 @@ __global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int
   const int uwarp = __shfl_sync(0xffffffffu, warp, 0);
   if (uwarp == 8) {
     if (tc05::elect_one()) {
-      // the instance's weight tile, once per CTA
-      tc05::mbar_arrive_expect_tx(&sm.bar_b, 2 * kPtTileBytes);
-      tc05::bulk_g2s(sm.b_hi, packed + b * (2 * (size_t)kPtTileBytes), kPtTileBytes, &sm.bar_b);
-      tc05::bulk_g2s(sm.b_lo, packed + b * (2 * (size_t)kPtTileBytes) + kPtTileBytes, kPtTileBytes, &sm.bar_b);
-      tc05::mbar_wait(&sm.bar_b, 0u);
+      const unsigned char* pb = packed + (b * gridDim.z + blockIdx.z) * (size_t)nk * (2 * (size_t)kPtTileBytes);
+      auto load_b = [&](int kt, uint32_t parity) {
+        tc05::mbar_arrive_expect_tx(&sm.bar_b, 2 * kPtTileBytes);
+        tc05::bulk_g2s(sm.b_hi, pb + kt * (2 * (size_t)kPtTileBytes), kPtTileBytes, &sm.bar_b);
+        tc05::bulk_g2s(sm.b_lo, pb + kt * (2 * (size_t)kPtTileBytes) + kPtTileBytes, kPtTileBytes, &sm.bar_b);
+        tc05::mbar_wait(&sm.bar_b, parity);
+      };
+      if (nk == 1) load_b(0, 0u);   // the instance's weight tile, once per CTA
       const uint32_t idesc = tc05::make_idesc_f16(128, 128);
       const uint32_t a_hi = tc05::smem_u32(sm.a_hi), a_lo = tc05::smem_u32(sm.a_lo);
       const uint32_t b_hi = tc05::smem_u32(sm.b_hi), b_lo = tc05::smem_u32(sm.b_lo);
       for (int i = 0; i < n_tiles; ++i) {
-        tc05::mbar_wait(&sm.bar_a, i & 1);
-        tc05::fence_after_sync();
+        for (int kt = 0; kt < nk; ++kt) {
+          const int c = i * nk + kt;   // MMA step: bar_a / bar_mma phase c
+          if (nk > 1) {                // key tile kt replaces the previous one once the MMAs that read it have completed
+            if (c > 0) tc05::mbar_wait(&sm.bar_mma, (c - 1) & 1);
+            load_b(kt, c & 1);
+          }
+          tc05::mbar_wait(&sm.bar_a, c & 1);
+          tc05::fence_after_sync();
 #pragma unroll
-        for (int ks = 0; ks < 8; ++ks) {
-          const uint32_t o = ks * 2 * kLboTile;
-          const uint64_t dah = tc05::make_desc(a_hi + o, kLboTile, kSbo), dal = tc05::make_desc(a_lo + o, kLboTile, kSbo);
-          const uint64_t dbh = tc05::make_desc(b_hi + o, kLboTile, kSbo), dbl = tc05::make_desc(b_lo + o, kLboTile, kSbo);
-          tc05::mma_ss_f16(tb, dah, dbh, idesc, ks > 0 ? 1u : 0u);
-          tc05::mma_ss_f16(tb, dal, dbh, idesc, 1u);
-          tc05::mma_ss_f16(tb, dah, dbl, idesc, 1u);
+          for (int ks = 0; ks < 8; ++ks) {
+            const uint32_t o = ks * 2 * kLboTile;
+            const uint64_t dah = tc05::make_desc(a_hi + o, kLboTile, kSbo), dal = tc05::make_desc(a_lo + o, kLboTile, kSbo);
+            const uint64_t dbh = tc05::make_desc(b_hi + o, kLboTile, kSbo), dbl = tc05::make_desc(b_lo + o, kLboTile, kSbo);
+            tc05::mma_ss_f16(tb, dah, dbh, idesc, (kt > 0 || ks > 0) ? 1u : 0u);
+            tc05::mma_ss_f16(tb, dal, dbh, idesc, 1u);
+            tc05::mma_ss_f16(tb, dah, dbl, idesc, 1u);
+          }
+          tc05::commit(&sm.bar_mma);
         }
-        tc05::commit(&sm.bar_mma);
       }
     }
     return;
@@ -110,13 +128,13 @@ __global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int
   const float unscale = 1.0f / (a_scale * kLkScale);
   float amax = 0.f;
   float4 buf[16];   // this thread's 8 (row, 8-column chunk) items of a tile, raw: the next tile is in flight while the current one is consumed
-  auto load_tile = [&](int64_t m0) {
+  auto load_tile = [&](int64_t m0, int kt) {
 #pragma unroll
     for (int it = 0; it < 8; ++it) {
       const int idx = tid + it * 256, r = idx & 127, c8 = idx >> 7;
       float4 v0 = make_float4(0.f, 0.f, 0.f, 0.f), v1 = v0;
       if (m0 + r < row_hi) {
-        const float4* src = reinterpret_cast<const float4*>(X + (m0 + r) * kE) + c8 * 2;
+        const float4* src = reinterpret_cast<const float4*>(X + (m0 + r) * ldx + kt * kFRows) + c8 * 2;
         v0 = __ldg(src);
         v1 = __ldg(src + 1);
         if (row_scale != nullptr) {  // x = diag(row_scale) X: the upstream gradient of a row times its saved Jacobian
@@ -129,8 +147,9 @@ __global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int
       buf[2 * it + 1] = v1;
     }
   };
-  if (n_tiles > 0) load_tile(row_lo);
-  for (int i = 0; i < n_tiles; ++i) {
+  if (n_tiles > 0) load_tile(row_lo, 0);
+  for (int c = 0; c < n_tiles * nk; ++c) {
+    const int i = c / nk, kt = c - i * nk;
     const int64_t m0 = row_lo + (int64_t)i * kFRows;
     // x tile -> fp16 hi | lo core-matrix tiles (the previous tile's MMAs have completed: its epilogue waited for them)
 #pragma unroll
@@ -148,11 +167,13 @@ __global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int
       *reinterpret_cast<uint4*>(&sm.a_hi[dst]) = make_uint4(h[0], h[1], h[2], h[3]);
       *reinterpret_cast<uint4*>(&sm.a_lo[dst]) = make_uint4(l[0], l[1], l[2], l[3]);
     }
-    if (i + 1 < n_tiles) load_tile(m0 + kFRows);
+    if (kt + 1 < nk) load_tile(m0, kt + 1);
+    else if (i + 1 < n_tiles) load_tile(m0 + kFRows, 0);
     tc05::fence_proxy_async();
     tc05::mbar_arrive(&sm.bar_a);
-    tc05::mbar_wait(&sm.bar_mma, i & 1);
+    tc05::mbar_wait(&sm.bar_mma, c & 1);
     tc05::fence_after_sync();
+    if (kt + 1 < nk) continue;   // the accumulator sums the remaining key tiles first
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
       const int col0 = colhalf * 64 + q * 16;
@@ -173,7 +194,7 @@ __global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int
     for (int k = tid; k < kFRows * (kE / 4); k += 256) {
       const int r = k >> 5, c4 = k & 31;
       if (m0 + r < row_hi)
-        reinterpret_cast<float4*>(Y + (m0 + r) * kE)[c4] = *reinterpret_cast<const float4*>(&sm.stage[r * 132 + c4 * 4]);
+        reinterpret_cast<float4*>(Y + (m0 + r) * ldy + blockIdx.z * kFRows)[c4] = *reinterpret_cast<const float4*>(&sm.stage[r * 132 + c4 * 4]);
     }
     // (the next tile's epilogue writes `stage` only after bar_mma, i.e. after every thread has arrived on bar_a behind this loop)
   }
@@ -183,8 +204,9 @@ __global__ void __launch_bounds__(kPtThreads, 1) inst_gemm_kernel(int64_t L, int
   if (warp == 0) tc05::tmem_dealloc(tb, 128);
 }
 
-// C_b[n_nodes, 128] += X_b^T Y_b over a slab of the rows of instance b (X, Y: [rows, 128]); as xty_kernel of ffn_train.cu with one
-// 128-feature block: 32-row tiles, two-stage operand buffer, 8 conversion warps (thread = one column of X or of Y) + issuer.
+// C_b[n_nodes, 128] += X_b^T Y_b over a slab of the rows of instance b (X: [rows, ldx], Y: [rows, 128]); as xty_kernel of ffn_train.cu
+// with one 128-feature block: 32-row tiles, two-stage operand buffer, 8 conversion warps (thread = one column of X or of Y) + issuer.
+// Grid z = key tile: columns [128 z, 128 z + 128) of X give rows [128 z, ..) of C_b.
 constexpr int kXiRows = 32;
 struct XtyInstSmem {
   uint16_t x_hi[2][kE * kXiRows];   // [8-row K chunk (4)][feature (128)][8 halves]
@@ -195,7 +217,7 @@ struct XtyInstSmem {
   uint32_t tmem_base;
 };
 
-__global__ void __launch_bounds__(kPtThreads, 2) xty_inst_kernel(int64_t L, int rows_per_cta, int N, const float* __restrict__ X,
+__global__ void __launch_bounds__(kPtThreads, 2) xty_inst_kernel(int64_t L, int rows_per_cta, int N, int ldx, const float* __restrict__ X,
                                                                 const float* __restrict__ Y, const float* __restrict__ sx_ptr,
                                                                 const float* __restrict__ sy_ptr,
                                                                 const float* __restrict__ row_scale, float* __restrict__ C,
@@ -250,7 +272,9 @@ __global__ void __launch_bounds__(kPtThreads, 2) xty_inst_kernel(int64_t L, int 
   const float sx = sx_ptr ? __ldg(sx_ptr) : kAScale, sy = sy_ptr ? __ldg(sy_ptr) : kAScale;
   const bool is_x = tid < 128;
   const int f = tid & 127;
-  const float* src = (is_x ? X : Y) + f;
+  const int n0 = blockIdx.z * kFRows;
+  const float* src = is_x ? X + n0 + f : Y + f;
+  const int64_t lds = is_x ? ldx : kE;
   const float sc = is_x ? sx : sy;
   float amax = 0.f;
   for (int it = 0; it < n_tiles; ++it) {
@@ -258,7 +282,7 @@ __global__ void __launch_bounds__(kPtThreads, 2) xty_inst_kernel(int64_t L, int 
     const int64_t r0 = row_lo + (int64_t)it * kXiRows;
     float xv[kXiRows];
 #pragma unroll
-    for (int r = 0; r < kXiRows; ++r) xv[r] = (r0 + r < row_hi) ? __ldg(src + (r0 + r) * kE) : 0.f;
+    for (int r = 0; r < kXiRows; ++r) xv[r] = (r0 + r < row_hi) ? __ldg(src + (r0 + r) * lds) : 0.f;
     if (is_x && row_scale != nullptr) {
 #pragma unroll
       for (int r = 0; r < kXiRows; ++r) xv[r] *= (r0 + r < row_hi) ? __ldg(row_scale + r0 + r) : 0.f;
@@ -293,8 +317,8 @@ __global__ void __launch_bounds__(kPtThreads, 2) xty_inst_kernel(int64_t L, int 
       uint32_t v[16];
       tc05::tmem_ld16(tb + lane_b + colhalf * 64 + q * 16, v);
       tc05::tmem_wait_ld();
-      if (m < N) {
-        float* crow = C + (b * N + m) * kE + colhalf * 64 + q * 16;
+      if (n0 + m < N) {
+        float* crow = C + (b * N + n0 + m) * kE + colhalf * 64 + q * 16;
 #pragma unroll
         for (int i = 0; i < 16; ++i) atomicAdd(crow + i, __uint_as_float(v[i]) * unscale);
       }
@@ -316,6 +340,47 @@ static int pt_rows_per_cta(int64_t L, int64_t n_inst, int* ctas_per_inst) {
   return (int)rows;
 }
 
+static int pt_pack(int64_t n_inst, int32_t n_nodes, const float* w, int32_t transpose, void* packed, uint32_t* status, void* stream) {
+  pack_inst_weights_kernel<<<dim3(kFRows * (kE / 2) / 256, (unsigned)n_inst, (unsigned)((n_nodes + kFRows - 1) / kFRows)), 256, 0,
+                             (cudaStream_t)stream>>>(w, n_nodes, transpose, reinterpret_cast<uint32_t*>(packed), status);
+  return rrnco_launch_status();
+}
+
+// n_out column blocks of 128 (grid z), nk key tiles summed per block
+static int pt_gemm(int64_t n_inst, int64_t rows_per_inst, int ldx, int nk, int ldy, int n_out, const float* x, const void* packed,
+                   const float* a_scale, const float* row_scale, float* y, uint32_t* status, void* stream) {
+  static PerDeviceOnce once;
+  if (once.first()) {
+    if (cudaFuncSetAttribute(inst_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(InstGemmSmem)) != cudaSuccess) {
+      once.undo();
+      return RRNCO_ERR_CUDA;
+    }
+  }
+  int per = 1;
+  const int rows = pt_rows_per_cta(rows_per_inst, n_inst * n_out, &per);
+  inst_gemm_kernel<<<dim3((unsigned)per, (unsigned)n_inst, (unsigned)n_out), kPtThreads, sizeof(InstGemmSmem), (cudaStream_t)stream>>>(
+      rows_per_inst, rows, ldx, nk, ldy, x, reinterpret_cast<const unsigned char*>(packed), a_scale, row_scale, y, status);
+  return rrnco_launch_status();
+}
+
+static int pt_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, int ldx, const float* x, const float* y, const float* sx,
+                  const float* sy, const float* row_scale, float* c, uint32_t* status, void* stream) {
+  static PerDeviceOnce once;
+  if (once.first()) {
+    if (cudaFuncSetAttribute(xty_inst_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(XtyInstSmem)) != cudaSuccess ||
+        cudaFuncSetAttribute(xty_inst_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) != cudaSuccess) {
+      once.undo();
+      return RRNCO_ERR_CUDA;
+    }
+  }
+  const int n_kt = (n_nodes + kFRows - 1) / kFRows;
+  int per = 1;
+  const int rows = pt_rows_per_cta(rows_per_inst, n_inst * n_kt, &per);
+  xty_inst_kernel<<<dim3((unsigned)per, (unsigned)n_inst, (unsigned)n_kt), kPtThreads, sizeof(XtyInstSmem), (cudaStream_t)stream>>>(
+      rows_per_inst, rows, n_nodes, ldx, x, y, sx, sy, row_scale, c, status);
+  return rrnco_launch_status();
+}
+
 }  // namespace rrnco
 
 using namespace rrnco;
@@ -329,9 +394,7 @@ int rrnco_train_inst_pack(int64_t n_inst, int32_t n_nodes, const float* w, int32
   if (n_inst == 0) return RRNCO_OK;
   RRNCO_CHECK_ARG(n_inst > 0 && n_nodes > 0 && w && packed && status && (reinterpret_cast<uintptr_t>(packed) & 15u) == 0);
   if (n_nodes > 128 || n_inst > 65535) return RRNCO_ERR_UNSUPPORTED;
-  pack_inst_weights_kernel<<<dim3(kFRows * (kE / 2) / 256, (unsigned)n_inst), 256, 0, (cudaStream_t)stream>>>(
-      w, n_nodes, transpose, reinterpret_cast<uint32_t*>(packed), status);
-  return rrnco_launch_status();
+  return pt_pack(n_inst, n_nodes, w, transpose, packed, status, stream);
 }
 
 int rrnco_train_inst_gemm(int64_t n_inst, int64_t rows_per_inst, const float* x, const void* packed, const float* a_scale,
@@ -340,18 +403,7 @@ int rrnco_train_inst_gemm(int64_t n_inst, int64_t rows_per_inst, const float* x,
   RRNCO_CHECK_ARG(n_inst > 0 && rows_per_inst > 0 && x && packed && y && status);
   RRNCO_CHECK_ARG(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(packed) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0);
   if (n_inst > 65535) return RRNCO_ERR_UNSUPPORTED;
-  static PerDeviceOnce once;
-  if (once.first()) {
-    if (cudaFuncSetAttribute(inst_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(InstGemmSmem)) != cudaSuccess) {
-      once.undo();
-      return RRNCO_ERR_CUDA;
-    }
-  }
-  int per = 1;
-  const int rows = pt_rows_per_cta(rows_per_inst, n_inst, &per);
-  inst_gemm_kernel<<<dim3((unsigned)per, (unsigned)n_inst), kPtThreads, sizeof(InstGemmSmem), (cudaStream_t)stream>>>(
-      rows_per_inst, rows, x, reinterpret_cast<const unsigned char*>(packed), a_scale, row_scale, y, status);
-  return rrnco_launch_status();
+  return pt_gemm(n_inst, rows_per_inst, kE, 1, kE, 1, x, packed, a_scale, row_scale, y, status, stream);
 }
 
 int rrnco_train_inst_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* x, const float* y, const float* sx,
@@ -359,19 +411,40 @@ int rrnco_train_inst_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes,
   if (n_inst == 0 || rows_per_inst == 0) return RRNCO_OK;
   RRNCO_CHECK_ARG(n_inst > 0 && rows_per_inst > 0 && n_nodes > 0 && x && y && c && status);
   if (n_nodes > 128 || n_inst > 65535) return RRNCO_ERR_UNSUPPORTED;
-  static PerDeviceOnce once;
-  if (once.first()) {
-    if (cudaFuncSetAttribute(xty_inst_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(XtyInstSmem)) != cudaSuccess ||
-        cudaFuncSetAttribute(xty_inst_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) != cudaSuccess) {
-      once.undo();
-      return RRNCO_ERR_CUDA;
-    }
-  }
-  int per = 1;
-  const int rows = pt_rows_per_cta(rows_per_inst, n_inst, &per);
-  xty_inst_kernel<<<dim3((unsigned)per, (unsigned)n_inst), kPtThreads, sizeof(XtyInstSmem), (cudaStream_t)stream>>>(
-      rows_per_inst, rows, n_nodes, x, y, sx, sy, row_scale, c, status);
-  return rrnco_launch_status();
+  return pt_xty(n_inst, rows_per_inst, n_nodes, kE, x, y, sx, sy, row_scale, c, status, stream);
+}
+
+int64_t rrnco_train_inst_tiled_packed_bytes(int64_t n_inst, int32_t n_nodes) {
+  if (n_inst <= 0 || n_nodes <= 0 || n_nodes > kPtMaxNodes) return 0;
+  return n_inst * ((n_nodes + kFRows - 1) / kFRows) * 2 * (int64_t)kPtTileBytes;
+}
+
+int rrnco_train_inst_tiled_pack(int64_t n_inst, int32_t n_nodes, const float* w, int32_t transpose, void* packed, uint32_t* status,
+                                void* stream) {
+  if (n_inst == 0) return RRNCO_OK;
+  RRNCO_CHECK_ARG(n_inst > 0 && n_nodes > 0 && w && packed && status && (reinterpret_cast<uintptr_t>(packed) & 15u) == 0);
+  if (n_nodes > kPtMaxNodes || n_inst > 65535) return RRNCO_ERR_UNSUPPORTED;
+  return pt_pack(n_inst, n_nodes, w, transpose, packed, status, stream);
+}
+
+int rrnco_train_inst_tiled_gemm(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, int32_t transpose, const float* x,
+                                const void* packed, const float* a_scale, const float* row_scale, float* y, uint32_t* status,
+                                void* stream) {
+  if (n_inst == 0 || rows_per_inst == 0) return RRNCO_OK;
+  RRNCO_CHECK_ARG(n_inst > 0 && rows_per_inst > 0 && n_nodes > 0 && x && packed && y && status);
+  RRNCO_CHECK_ARG(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(packed) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0);
+  if (n_nodes > kPtMaxNodes || n_inst > 65535) return RRNCO_ERR_UNSUPPORTED;
+  const int n_kt = (n_nodes + kFRows - 1) / kFRows, ldz = n_kt * kFRows;
+  return transpose ? pt_gemm(n_inst, rows_per_inst, ldz, n_kt, kE, 1, x, packed, a_scale, row_scale, y, status, stream)
+                   : pt_gemm(n_inst, rows_per_inst, kE, 1, ldz, n_kt, x, packed, a_scale, row_scale, y, status, stream);
+}
+
+int rrnco_train_inst_tiled_xty(int64_t n_inst, int64_t rows_per_inst, int32_t n_nodes, const float* x, const float* y, const float* sx,
+                               const float* sy, const float* row_scale, float* c, uint32_t* status, void* stream) {
+  if (n_inst == 0 || rows_per_inst == 0) return RRNCO_OK;
+  RRNCO_CHECK_ARG(n_inst > 0 && rows_per_inst > 0 && n_nodes > 0 && x && y && c && status);
+  if (n_nodes > kPtMaxNodes || n_inst > 65535) return RRNCO_ERR_UNSUPPORTED;
+  return pt_xty(n_inst, rows_per_inst, n_nodes, (n_nodes + kFRows - 1) / kFRows * kFRows, x, y, sx, sy, row_scale, c, status, stream);
 }
 
 }  // extern "C"

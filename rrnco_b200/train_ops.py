@@ -2,7 +2,8 @@
 parts of the training hand-off (`training.batched_logprobs`) as hand-written sm_100a kernels, forward AND backward.
 
     fused_ffn(x, w1, b1, w2, b2)             residual FFN of the pointer (decoder.py:272-277, 296) on tcgen05, fp32-faithful
-    fused_attention(q, k, v, mask)           masked 8-head attention + residual (decoder.py:281-293)
+    fused_attention(q, k, v, mask)           masked 8-head attention + residual (decoder.py:281-293), N <= 1024
+    pointer_scores(g, lk) / pointer_logprob  pointer scores g . Lk^T on tcgen05 (decoder.py:298-301), N <= 1024
     fused_logits_tail(z, decoder, ...)       edge bias / log(exp + 1e-6) / tanh clip / mask / log-softmax / gather
                                              (decoder.py:183-198, decoding.py:311-399)
 
@@ -18,7 +19,9 @@ import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "librrnco_b200_train.so")
-MAX_NODES_ATTENTION = 102   # K, V, dK, dV tiles of one instance in shared memory (rrnco_train_attention_bwd)
+MAX_NODES_ATTENTION = 102   # K, V, dK, dV tiles of one instance in shared memory (rrnco_train_attention_bwd); above: key-tiled kernels
+MAX_NODES_POINTER = 128     # one 128 x 128 weight tile per instance (rrnco_train_inst_*); above: ceil(N / 128) key tiles
+MAX_NODES_REPLAY = 1024     # largest instance of the key-tiled kernels (rrnco_train_attention_tiled_*, rrnco_train_inst_tiled_*)
 DEV_NAN_LOGITS = 1
 
 _f = C.c_void_p
@@ -29,6 +32,10 @@ _SIGNATURES = {
     "rrnco_train_xty": (C.c_int, [C.c_int64, _f, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_train_attention_fwd": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, C.c_int32, _f, _f, _f]),
     "rrnco_train_attention_bwd": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, _f, C.c_int32, _f, _f, _f, _f, _f, _f]),
+    "rrnco_train_attention_tiled_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int64, C.c_int32]),
+    "rrnco_train_attention_tiled_fwd": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, C.c_int32, _f, _f, _f]),
+    "rrnco_train_attention_tiled_bwd": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, _f, C.c_int32, _f, _f, _f, _f, _f,
+                                                  _f, _f]),
     "rrnco_train_context_query_fwd": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, _f, C.c_int32, _f, _f, _f]),
     "rrnco_train_context_query_bwd": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, C.c_int32, _f, _f, _f, _f]),
     "rrnco_train_logits_tail": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f, C.c_float, C.c_float,
@@ -37,6 +44,10 @@ _SIGNATURES = {
     "rrnco_train_inst_pack": (C.c_int, [C.c_int64, C.c_int32, _f, C.c_int32, _f, _f, _f]),
     "rrnco_train_inst_gemm": (C.c_int, [C.c_int64, C.c_int64, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_train_inst_xty": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f]),
+    "rrnco_train_inst_tiled_packed_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
+    "rrnco_train_inst_tiled_pack": (C.c_int, [C.c_int64, C.c_int32, _f, C.c_int32, _f, _f, _f]),
+    "rrnco_train_inst_tiled_gemm": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, C.c_int32, _f, _f, _f, _f, _f, _f, _f]),
+    "rrnco_train_inst_tiled_xty": (C.c_int, [C.c_int64, C.c_int64, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_train_nab_packed_floats": (C.c_int64, []),
     "rrnco_train_nab_grad_floats": (C.c_int64, []),
     "rrnco_train_nab_workspace_bytes": (C.c_int64, [C.c_int64, C.c_int32]),
@@ -209,8 +220,9 @@ class _FusedAttention(torch.autograd.Function):
         N = k.shape[1]
         out = torch.empty_like(q)
         lse = torch.empty(n_inst, L, 8, dtype=torch.float32, device=dev)
-        _check(h.rrnco_train_attention_fwd(n_inst, L, N, _p(q), _p(k), _p(v), _p(m8), int(add_residual), _p(out), _p(lse),
-                                           _stream(dev)), "rrnco_train_attention_fwd")
+        fwd = h.rrnco_train_attention_fwd if N <= MAX_NODES_ATTENTION else h.rrnco_train_attention_tiled_fwd
+        _check(fwd(n_inst, L, N, _p(q), _p(k), _p(v), _p(m8), int(add_residual), _p(out), _p(lse), _stream(dev)),
+               "rrnco_train_attention_fwd" if N <= MAX_NODES_ATTENTION else "rrnco_train_attention_tiled_fwd")
         ctx.save_for_backward(q, k, v, m8, out, lse)
         ctx.add_residual = int(add_residual)
         return out
@@ -224,13 +236,20 @@ class _FusedAttention(torch.autograd.Function):
         N = k.shape[1]
         d_out = d_out.contiguous().float()
         dq, dk, dv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
-        _check(h.rrnco_train_attention_bwd(n_inst, L, N, _p(q), _p(k), _p(v), _p(m8), _p(out), ctx.add_residual, _p(lse),
-                                           _p(d_out), _p(dq), _p(dk), _p(dv), _stream(dev)), "rrnco_train_attention_bwd")
+        if N <= MAX_NODES_ATTENTION:
+            _check(h.rrnco_train_attention_bwd(n_inst, L, N, _p(q), _p(k), _p(v), _p(m8), _p(out), ctx.add_residual, _p(lse),
+                                               _p(d_out), _p(dq), _p(dk), _p(dv), _stream(dev)), "rrnco_train_attention_bwd")
+        else:
+            ws = torch.empty(h.rrnco_train_attention_tiled_workspace_bytes(n_inst, L, N), dtype=torch.uint8, device=dev)
+            _check(h.rrnco_train_attention_tiled_bwd(n_inst, L, N, _p(q), _p(k), _p(v), _p(m8), _p(out), ctx.add_residual, _p(lse),
+                                                     _p(d_out), _p(ws), _p(dq), _p(dk), _p(dv), _stream(dev)),
+                   "rrnco_train_attention_tiled_bwd")
         return dq, dk, dv, None, None
 
 
 def fused_attention(q, k, v, mask, add_residual: bool = True):
-    """softmax(q_h k_h^T / 4 + mask) v_h (+ q): q [n_inst, L, 128], k / v [n_inst, N, 128], mask [n_inst, L, N] bool."""
+    """softmax(q_h k_h^T / 4 + mask) v_h (+ q): q [n_inst, L, 128], k / v [n_inst, N, 128], mask [n_inst, L, N] bool.
+    N <= 102: K, V, dK and dV of an instance resident in shared memory; 102 < N <= 1024: the key-tiled kernels."""
     return _FusedAttention.apply(q, k, v, mask, add_residual)
 
 
@@ -276,18 +295,56 @@ def context_query(table_a, index_a, table_b=None, index_b=None, state=None, stat
     return _ContextQuery.apply(table_a, index_a, table_b, index_b, state, state_w)
 
 
+def score_width(N: int) -> int:
+    """Row width ldz of the pointer scores of an N-node instance: 128 ceil(N / 128) (one 128-column block per weight tile)."""
+    return 128 * ((N + 127) // 128)
+
+
+def _inst_pack(lk, transpose, dev):
+    h, st = lib(), status_word(dev)
+    n_inst, N, _ = lk.shape
+    if N <= MAX_NODES_POINTER:
+        packed = torch.empty(h.rrnco_train_inst_packed_bytes(n_inst), dtype=torch.uint8, device=dev)
+        _check(h.rrnco_train_inst_pack(n_inst, N, _p(lk), transpose, _p(packed), _p(st), _stream(dev)), "rrnco_train_inst_pack")
+    else:
+        packed = torch.empty(h.rrnco_train_inst_tiled_packed_bytes(n_inst, N), dtype=torch.uint8, device=dev)
+        _check(h.rrnco_train_inst_tiled_pack(n_inst, N, _p(lk), transpose, _p(packed), _p(st), _stream(dev)),
+               "rrnco_train_inst_tiled_pack")
+    return packed
+
+
+def _inst_gemm(x, packed, N, transpose, a_scale, row_scale, y):
+    """y = x B_b per instance: the 128-node kernel, or the key-tiled one (transpose: which operand holds the key tiles)."""
+    h, dev = lib(), x.device
+    n_inst, L, _ = x.shape
+    st = status_word(dev)
+    if N <= MAX_NODES_POINTER:
+        _check(h.rrnco_train_inst_gemm(n_inst, L, _p(x), _p(packed), _p(a_scale), _p(row_scale), _p(y), _p(st), _stream(dev)),
+               "rrnco_train_inst_gemm")
+    else:
+        _check(h.rrnco_train_inst_tiled_gemm(n_inst, L, N, transpose, _p(x), _p(packed), _p(a_scale), _p(row_scale), _p(y), _p(st),
+                                             _stream(dev)), "rrnco_train_inst_tiled_gemm")
+
+
+def _inst_xty(x, g, N, s_x, row_scale, dlk):
+    h, dev = lib(), g.device
+    n_inst, L, _ = g.shape
+    st = status_word(dev)
+    xty = h.rrnco_train_inst_xty if N <= MAX_NODES_POINTER else h.rrnco_train_inst_tiled_xty
+    _check(xty(n_inst, L, N, _p(x), _p(g), _p(s_x), None, _p(row_scale), _p(dlk), _p(st), _stream(dev)), "rrnco_train_inst_xty")
+
+
 class _PointerScores(torch.autograd.Function):
     @staticmethod
     @_on_device
     def forward(ctx, g, lk):
-        h, dev, st = lib(), g.device, status_word(g.device)
+        dev = g.device
         g, lk = g.detach().contiguous().float(), lk.detach().contiguous().float()
         n_inst, L, _ = g.shape
         N = lk.shape[1]
-        packed = torch.empty(h.rrnco_train_inst_packed_bytes(n_inst), dtype=torch.uint8, device=dev)
-        _check(h.rrnco_train_inst_pack(n_inst, N, _p(lk), 0, _p(packed), _p(st), _stream(dev)), "rrnco_train_inst_pack")
-        z = torch.empty(n_inst, L, 128, dtype=torch.float32, device=dev)
-        _check(h.rrnco_train_inst_gemm(n_inst, L, _p(g), _p(packed), None, None, _p(z), _p(st), _stream(dev)), "rrnco_train_inst_gemm")
+        packed = _inst_pack(lk, 0, dev)
+        z = torch.empty(n_inst, L, score_width(N), dtype=torch.float32, device=dev)
+        _inst_gemm(g, packed, N, 0, None, None, z)
         ctx.save_for_backward(g, lk)
         return z
 
@@ -295,23 +352,22 @@ class _PointerScores(torch.autograd.Function):
     @_on_device
     def backward(ctx, dz):
         g, lk = ctx.saved_tensors
-        h, dev, st = lib(), g.device, status_word(g.device)
-        n_inst, L, _ = g.shape
+        dev = g.device
         N = lk.shape[1]
         dz = dz.contiguous().float()
         s_dz = pow2_scale(dz)
-        packed = torch.empty(h.rrnco_train_inst_packed_bytes(n_inst), dtype=torch.uint8, device=dev)
-        _check(h.rrnco_train_inst_pack(n_inst, N, _p(lk), 1, _p(packed), _p(st), _stream(dev)), "rrnco_train_inst_pack")
+        packed = _inst_pack(lk, 1, dev)
         dg = torch.empty_like(g)
-        _check(h.rrnco_train_inst_gemm(n_inst, L, _p(dz), _p(packed), _p(s_dz), None, _p(dg), _p(st), _stream(dev)), "rrnco_train_inst_gemm (dg)")
+        _inst_gemm(dz, packed, N, 1, s_dz, None, dg)
         dlk = torch.zeros_like(lk)
-        _check(h.rrnco_train_inst_xty(n_inst, L, N, _p(dz), _p(g), _p(s_dz), None, None, _p(dlk), _p(st), _stream(dev)), "rrnco_train_inst_xty")
+        _inst_xty(dz, g, N, s_dz, None, dlk)
         return dg, dlk
 
 
 def pointer_scores(g, lk):
-    """z [n_inst, L, 128] = g lk^T (columns >= N are zero): g [n_inst, L, 128], lk [n_inst, N <= 128, 128]; forward, dg and dlk on
-    tcgen05 in the fp32-faithful fp16 hi|lo split (decoder.py:298-301 without the 1 / sqrt(E), which the tail applies)."""
+    """z [n_inst, L, ldz] = g lk^T (columns >= N are zero; ldz = score_width(N) = 128 ceil(N / 128)): g [n_inst, L, 128],
+    lk [n_inst, N <= 1024, 128]; forward, dg and dlk on tcgen05 in the fp32-faithful fp16 hi|lo split (decoder.py:298-301 without the
+    1 / sqrt(E), which the tail applies).  N <= 128: one weight tile per instance; above: ceil(N / 128) key tiles."""
     return _PointerScores.apply(g, lk)
 
 
@@ -320,7 +376,7 @@ class _LogitsTail(torch.autograd.Function):
     @_on_device
     def forward(ctx, z, alpha, beta, distance, duration, cur, mask, act, tanh_clipping, temperature):
         h, dev = lib(), z.device
-        n_inst, L, ldz = z.shape      # ldz >= N: the 128-wide rows of pointer_scores, or exactly N
+        n_inst, L, ldz = z.shape      # N <= ldz <= 1024: the score_width(N)-wide rows of pointer_scores, or exactly N
         N = distance.shape[-1]
         jac = z.detach()
         if not jac.is_contiguous() or jac.dtype != torch.float32:
@@ -354,8 +410,8 @@ class _LogitsTail(torch.autograd.Function):
 
 
 def fused_logits_tail(z, alpha, beta, distance, duration, cur, mask, act, tanh_clipping, temperature):
-    """log pi(act | state) [n_inst, L] from the raw pointer scores z = g . Lk^T [n_inst, L, N] (consumed: overwritten in place by
-    the Jacobian); distance / duration [n_inst, N, N], cur / act [n_inst, L] int64, mask [n_inst, L, N] bool."""
+    """log pi(act | state) [n_inst, L] from the raw pointer scores z = g . Lk^T [n_inst, L, ldz], N <= ldz <= 1024 (consumed:
+    overwritten in place by the Jacobian); distance / duration [n_inst, N, N], cur / act [n_inst, L] int64, mask [n_inst, L, N] bool."""
     return _LogitsTail.apply(z, alpha, beta, distance, duration, cur, mask, act, tanh_clipping, temperature)
 
 
@@ -366,14 +422,14 @@ class _PointerLogProb(torch.autograd.Function):
     @staticmethod
     @_on_device
     def forward(ctx, g, lk, alpha, beta, distance, duration, cur, mask, act, tanh_clipping, temperature):
-        h, dev, st = lib(), g.device, status_word(g.device)
+        h, dev = lib(), g.device
         g, lk = g.detach().contiguous().float(), lk.detach().contiguous().float()
         n_inst, L, _ = g.shape
         N = lk.shape[1]
-        packed = torch.empty(h.rrnco_train_inst_packed_bytes(n_inst), dtype=torch.uint8, device=dev)
-        _check(h.rrnco_train_inst_pack(n_inst, N, _p(lk), 0, _p(packed), _p(st), _stream(dev)), "rrnco_train_inst_pack")
-        jac = torch.empty(n_inst, L, 128, dtype=torch.float32, device=dev)
-        _check(h.rrnco_train_inst_gemm(n_inst, L, _p(g), _p(packed), None, None, _p(jac), _p(st), _stream(dev)), "rrnco_train_inst_gemm")
+        ldz = score_width(N)
+        packed = _inst_pack(lk, 0, dev)
+        jac = torch.empty(n_inst, L, ldz, dtype=torch.float32, device=dev)
+        _inst_gemm(g, packed, N, 0, None, None, jac)
         logp = torch.empty(n_inst, L, dtype=torch.float32, device=dev)
         da = torch.empty(n_inst, L, dtype=torch.float32, device=dev)
         db = torch.empty(n_inst, L, dtype=torch.float32, device=dev) if duration is not None else None
@@ -382,7 +438,7 @@ class _PointerLogProb(torch.autograd.Function):
         distance, cur, act = distance.contiguous(), cur.contiguous(), act.contiguous()
         duration = duration.contiguous() if duration is not None else None
         m8 = mask.contiguous().view(torch.uint8)
-        _check(h.rrnco_train_logits_tail(n_inst * L, L, N, 128, _p(jac), _p(distance), _p(duration), _p(cur), _p(m8), _p(act),
+        _check(h.rrnco_train_logits_tail(n_inst * L, L, N, ldz, _p(jac), _p(distance), _p(duration), _p(cur), _p(m8), _p(act),
                                          _p(alpha_d), _p(beta_d), 1.0 / math.sqrt(128.0), float(tanh_clipping), float(temperature),
                                          _p(logp), _p(da), _p(db), _stream(dev)), "rrnco_train_logits_tail")
         ctx.save_for_backward(g, lk, jac, da, db)
@@ -395,25 +451,22 @@ class _PointerLogProb(torch.autograd.Function):
     @_on_device
     def backward(ctx, gl):
         g, lk, jac, da, db = ctx.saved_tensors
-        h, dev, st = lib(), g.device, status_word(g.device)
-        n_inst, L, _ = g.shape
+        dev = g.device
         N = lk.shape[1]
         gl = gl.contiguous().float()
         s_dz = pow2_scale(gl, bound_factor=ctx.jmax)
-        packed = torch.empty(h.rrnco_train_inst_packed_bytes(n_inst), dtype=torch.uint8, device=dev)
-        _check(h.rrnco_train_inst_pack(n_inst, N, _p(lk), 1, _p(packed), _p(st), _stream(dev)), "rrnco_train_inst_pack")
+        packed = _inst_pack(lk, 1, dev)
         dg = torch.empty_like(g)
-        _check(h.rrnco_train_inst_gemm(n_inst, L, _p(jac), _p(packed), _p(s_dz), _p(gl), _p(dg), _p(st), _stream(dev)),
-               "rrnco_train_inst_gemm (dg)")
+        _inst_gemm(jac, packed, N, 1, s_dz, gl, dg)
         dlk = torch.zeros_like(lk)
-        _check(h.rrnco_train_inst_xty(n_inst, L, N, _p(jac), _p(g), _p(s_dz), None, _p(gl), _p(dlk), _p(st), _stream(dev)),
-               "rrnco_train_inst_xty")
+        _inst_xty(jac, g, N, s_dz, gl, dlk)
         dalpha = (gl * da).sum().reshape(ctx.shapes[0])
         dbeta = (gl * db).sum().reshape(ctx.shapes[1]) if db is not None else None
         return dg, dlk, dalpha, dbeta, None, None, None, None, None, None, None
 
 
 def pointer_logprob(g, lk, alpha, beta, distance, duration, cur, mask, act, tanh_clipping, temperature):
-    """log pi(act | state) [n_inst, L] from the pointer input g [n_inst, L, 128] and the logit keys lk [n_inst, N, 128]
-    (decoder.py:183-198, 298-301; decoding.py:311-399): pointer_scores and fused_logits_tail as one autograd node."""
+    """log pi(act | state) [n_inst, L] from the pointer input g [n_inst, L, 128] and the logit keys lk [n_inst, N <= 1024, 128]
+    (decoder.py:183-198, 298-301; decoding.py:311-399): pointer_scores and fused_logits_tail as one autograd node.  The saved
+    Jacobian is [n_inst, L, score_width(N)]."""
     return _PointerLogProb.apply(g, lk, alpha, beta, distance, duration, cur, mask, act, tanh_clipping, temperature)

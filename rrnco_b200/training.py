@@ -13,9 +13,9 @@ The fused rollout kernel is forward-only.  Upstream's training step (`rrnco/mode
         sequential small-kernel steps.  On CUDA tensors those rows go through the hand-written kernels of
         librrnco_b200_train.so, forward AND backward (`train_ops.py`: context query as a table gather, attention on the CUDA
         cores with mma.sync row sums, tcgen05 FFN with a relu bit mask and an X^T Y weight-gradient kernel, tcgen05 pointer
-        scores + a one-pass tail that leaves the Jacobian); torch keeps the autograd graph and the two tiny per-instance
-        projections.  `REPLAY_IMPL = "aten"` (and any CPU tensor, bf16 autocast, N > 102) selects the same math as plain
-        torch ops.
+        scores + a one-pass tail that leaves the Jacobian; instances of more than 102 / 128 nodes, up to 1024, on the key-tiled
+        attention and pointer kernels); torch keeps the autograd graph and the two tiny per-instance projections.
+        `REPLAY_IMPL = "aten"` (and any CPU tensor, bf16 autocast, N > 1024) selects the same math as plain torch ops.
   3. `pomo_shared_baseline_loss` = rl4co REINFORCE with the shared (POMO) baseline [rl4co-recalled], rl.py:119-128.
 
 The plain-torch form is checked against the oracle's per-step decoder on the CPU (tests/test_training_handoff.py); the kernels
@@ -85,6 +85,16 @@ def collect_decode_inputs(decoder, env, td, actions: torch.Tensor, num_starts: i
     return {k: torch.cat([c[k] for c in chunks]) for k in chunks[0]}
 
 
+def uses_replay_kernels(col_emb: torch.Tensor, N: int) -> bool:
+    """Which form `batched_logprobs` takes: the kernels of train_ops for CUDA fp32 replays of up to 1024 nodes
+    (train_ops.MAX_NODES_REPLAY), the plain-torch form for REPLAY_IMPL = "aten", bf16 autocast, CPU or non-fp32 tensors and larger
+    instances."""
+    if not (col_emb.is_cuda and col_emb.dtype == torch.float32 and REPLAY_IMPL == "fused" and not torch.is_autocast_enabled()):
+        return False
+    from . import train_ops
+    return N <= train_ops.MAX_NODES_REPLAY
+
+
 def batched_logprobs(decoder, row_emb, col_emb, distance, duration, inputs: dict, actions: torch.Tensor,
                      num_starts: int, temperature: float = 1.0, tanh_clipping: float = 10.0,
                      step_chunk: int = 32, autocast_dtype=None) -> torch.Tensor:
@@ -110,10 +120,7 @@ def batched_logprobs(decoder, row_emb, col_emb, distance, duration, inputs: dict
         else:
             yield from inputs
 
-    fused = col_emb.is_cuda and REPLAY_IMPL == "fused" and not torch.is_autocast_enabled()
-    if fused:
-        from . import train_ops
-        fused = N <= train_ops.MAX_NODES_ATTENTION and E == 128 and H == 8  # larger instances: the ATen form below
+    fused = uses_replay_kernels(col_emb, N) and E == 128 and H == 8
     k, v, lk = F.linear(col_emb, decoder.project_node_embeddings.weight).chunk(3, dim=-1)  # decoder.py:214-232
     W = decoder.context_embedding.project_context.weight
 
