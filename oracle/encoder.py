@@ -19,16 +19,21 @@ def _mlp2(p, prefix, x):
     return F.linear(h, p[f"{prefix}.2.weight"], p[f"{prefix}.2.bias"])
 
 
-def pairwise_angles(coords):
-    """attn_freenet.py:254-262: angle of x_i - x_j for every ordered pair, [B, N, N]."""
-    diff = coords.unsqueeze(2) - coords.unsqueeze(1)
+def pairwise_angles(coords, rows=None):
+    """attn_freenet.py:254-262: angle of x_i - x_j for every ordered pair, [B, N, N] (rows i in range(*rows) only: [B, R, N])."""
+    ci = coords if rows is None else coords[:, rows[0]:rows[1]]
+    diff = ci.unsqueeze(2) - coords.unsqueeze(1)
     return torch.atan2(diff[..., 1], diff[..., 0])
 
 
-def dist_angle_fusion(p, coords, cost_mat, duration_mat=None):
+def dist_angle_fusion(p, coords, cost_mat, duration_mat=None, rows=None):
     """DistAngleFusion.forward (attn_freenet.py:242-289): adapt_bias [B, N, N].
-    Materialises [B, N, N, E] embeddings exactly like the reference: small sizes only."""
-    angles = pairwise_angles(coords)
+    Materialises [B, N, N, E] embeddings exactly like the reference: small sizes only.  `rows` = (i0, i1) evaluates the
+    rows i0 <= i < i1 alone ([B, i1 - i0, N]): every pair is computed by the same ops, so large N can be done in chunks."""
+    angles = pairwise_angles(coords, rows)
+    if rows is not None:
+        cost_mat = cost_mat[:, rows[0]:rows[1]]
+        duration_mat = None if duration_mat is None else duration_mat[:, rows[0]:rows[1]]
     dist_emb = _mlp2(p, "dist_emb", cost_mat.unsqueeze(-1))
     angle_emb = _mlp2(p, "angle_emb", angles.unsqueeze(-1))
     if duration_mat is not None:

@@ -223,9 +223,9 @@ __global__ void __launch_bounds__(kDThreads, 2) nab_dur_kernel(int N, int64_t n_
           float h[8];
 #pragma unroll
           for (int e = 0; e < 8; ++e) {
-            h[e] = fmaxf(fmaf(w1[x * kE + k0 + e], s, b1[x * kE + k0 + e]), 0.f);
+            h[e] = fmax_nan(fmaf(w1[x * kE + k0 + e], s, b1[x * kE + k0 + e]), 0.f);  // a NaN scalar: NaN (upstream's relu)
             od = fmaf(uo[x * kE + k0 + e], h[e], od);
-            hmax = fmaxf(hmax, h[e]);
+            hmax = fmax_nan(hmax, h[e]);
           }
           uint32_t hh[4], ll[4];
 #pragma unroll
@@ -234,7 +234,7 @@ __global__ void __launch_bounds__(kDThreads, 2) nab_dur_kernel(int N, int64_t n_
           *reinterpret_cast<uint4*>(&a_hi[dst]) = make_uint4(hh[0], hh[1], hh[2], hh[3]);
           *reinterpret_cast<uint4*>(&a_lo[dst]) = make_uint4(ll[0], ll[1], ll[2], ll[3]);
         }
-        if (!(hmax * kAScale < 65504.f)) atomicOr(status, RRNCO_DEV_NAN_LOGITS);  // fp16 operand overflow (or NaN input): loud
+        if (!(hmax * kAScale < 65504.f)) atomicOr(status, RRNCO_DEV_NAN_LOGITS);  // fp16 operand overflow or non-finite input: loud
         od += __shfl_xor_sync(0xffffffffu, od, 16);
         if (dh == 0) sm.od[x][grow] = od;
         tc05::fence_proxy_async();

@@ -133,10 +133,10 @@ __global__ void __launch_bounds__(kNabThreads) nab_gating_kernel(int N, const fl
     const float4 pa = *reinterpret_cast<const float4*>(&sp[k * 8 + 4]);  // w1a, b1a, ug_a, uo_a
 #pragma unroll
     for (int m = 0; m < kNabPairs; ++m) {
-      const float hd = fmaxf(fmaf(pd.x, c[m], pd.y), 0.f);
+      const float hd = fmax_nan(fmaf(pd.x, c[m], pd.y), 0.f);  // a NaN scalar stays NaN, as in the table variant
       gd[m] = fmaf(pd.z, hd, gd[m]);
       od[m] = fmaf(pd.w, hd, od[m]);
-      const float ha = fmaxf(fmaf(pa.x, th[m], pa.y), 0.f);
+      const float ha = fmax_nan(fmaf(pa.x, th[m], pa.y), 0.f);
       ga[m] = fmaf(pa.z, ha, ga[m]);
       oa[m] = fmaf(pa.w, ha, oa[m]);
     }

@@ -114,9 +114,9 @@ __global__ void __launch_bounds__(256) nab_dur_bound_kernel(int N, int64_t n_pai
 #pragma unroll
     for (int x = 0; x < 3; ++x) {
       float o = co[x];
-      for (int k = 0; k < kE; ++k) o = fmaf(v[6 * kE + x * kE + k], fmaxf(fmaf(v[x * kE + k], sx[x], v[3 * kE + x * kE + k]), 0.f), o);
-      omax = fmaxf(omax, o);
-      omin = fminf(omin, o);
+      for (int k = 0; k < kE; ++k) o = fmaf(v[6 * kE + x * kE + k], fmax_nan(fmaf(v[x * kE + k], sx[x], v[3 * kE + x * kE + k]), 0.f), o);
+      omax = fmax_nan(omax, o);  // a NaN scalar makes the bound NaN, which counts as infinite
+      omin = fmin_nan(omin, o);
     }
     const float a = fabsf(scale * __ldg(grad_out + p)) * (omax - omin);
     m = max(m, a == a ? __float_as_uint(a) : 0x7f800000u);

@@ -156,7 +156,8 @@ class _NabDurGating(torch.autograd.Function):
         call("rrnco_nab_dur_gating", B, N, ptr(coords), ptr(cost), ptr(dur), transposed, ptr(packed), float(scale), ptr(out),
              ptr(status), stream_ptr(cost.device))
         if check and int(status.item()):
-            raise AssertionError("DistAngleFusion: hidden activations outside the fp16 operand range (>= 4094)")
+            raise AssertionError("DistAngleFusion: hidden activations outside the fp16 operand range (>= 4094) "
+                                 "or a cost / duration / coordinate that is not finite")
         flat = torch.cat([p.detach().float().reshape(-1) for p in params])
         ctx.save_for_backward(coords, cost, dur, packed, flat)
         ctx.transposed, ctx.scale = transposed, float(scale)
@@ -272,7 +273,8 @@ class DistAngleFusion(nn.Module):
             call("rrnco_nab_dur_gating", B, N, ptr(coords), ptr(cost_mat), ptr(dur), transposed, ptr(self._packed_duration()),
                  float(scale), ptr(out), ptr(status), stream_ptr(out.device))
             if self.check_overflow and int(status.item()):
-                raise AssertionError("DistAngleFusion: hidden activations outside the fp16 operand range (>= 4094)")
+                raise AssertionError("DistAngleFusion: hidden activations outside the fp16 operand range (>= 4094) "
+                                     "or a cost / duration / coordinate that is not finite")
             return out
         call("rrnco_nab_gating", B, N, ptr(coords), ptr(cost_mat), transposed, ptr(self.packed_parameters()), float(scale),
              int(variant), ptr(out), stream_ptr(cost_mat.device))
