@@ -261,15 +261,30 @@ int rrnco_decoder_logits_large(int32_t env, int32_t n_nodes, int64_t n_inst, int
                                float* logits_out, uint32_t* status, void* workspace, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
- * DecodingStrategy.step  rrnco/models/decoding.py:219-298 with process_logits :311-361 (top-k / top-p off)
+ * DecodingStrategy.step  rrnco/models/decoding.py:219-298 with process_logits :311-361
  *   logits fp32 [R,N] (decoder output), mask bool [R,N]  ->  action int64 [R], log-prob of the action fp32 [R]
  *   greedy: argmax of the log-softmax, lowest index on ties; sampling: Gumbel-max with noise
  *   Philox(seed; (r, step, n >> 2))[n & 3]; evaluate: forced_action [R].
+ *   rrnco_select_action = rrnco_select_action_filtered with top_k = 0, top_p = 0 (no filter).
+ *
+ * Logit filters (rrnco_select_action_filtered, rrnco_rollout_filtered), applied after tanh clipping, the mask and the
+ * temperature, before the log-softmax, for every decode mode:
+ *   top_k > 0      keep the entries >= the k-th largest value (ties kept; masked entries take part, so a row with fewer
+ *                  than k feasible nodes is unchanged).  top_k = 0: off.
+ *   0 < top_p < 1  then keep entry j iff the softmax mass of the entries strictly greater than it is < top_p (a tie group
+ *                  is kept or dropped whole; the top entry is always kept).  top_p = 0 or 1: off.
+ *   The log-probs are renormalised over the kept entries; a forced (evaluate) action that is feasible but filtered out
+ *   gets log-prob -inf and is not reported as infeasible.  Sampling draws the same Gumbel noise as without a filter and
+ *   skips the dropped entries.  top_k < 0 or top_p outside [0, 1] (or NaN): RRNCO_ERR_BAD_ARG, nothing launched.
  * ---------------------------------------------------------------------------------------------- */
 int rrnco_select_action(int64_t n_rollouts, int32_t n_nodes, const float* logits, const uint8_t* mask,
                         int32_t decode_mode, float tanh_clipping, float temperature, uint64_t seed, int32_t step,
                         const int64_t* forced_action, int64_t* action_out, float* logprob_out, uint32_t* status,
                         void* stream);
+int rrnco_select_action_filtered(int64_t n_rollouts, int32_t n_nodes, const float* logits, const uint8_t* mask,
+                                 int32_t decode_mode, float tanh_clipping, float temperature, uint64_t seed, int32_t step,
+                                 const int64_t* forced_action, int64_t* action_out, float* logprob_out, uint32_t* status,
+                                 int32_t top_k, float top_p, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Fused construction rollout = RRNetPolicy.forward decode loop  rrnco/models/policy.py:203-243
@@ -311,6 +326,17 @@ int rrnco_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts
                   const int64_t* forced_actions, int32_t forced_T, int32_t t_cap, int64_t* actions_out,
                   float* logprob_out, float* loglik_out, float* norm_reward_out, float* real_reward_out,
                   int32_t* max_steps_out, uint32_t* status, void* workspace, void* stream);
+/* rrnco_rollout with the logit filters described at rrnco_select_action_filtered (rrnco_rollout = top_k 0, top_p 0).  A
+ * filter runs on the single-tile tcgen05 engines (n_nodes <= RRNCO_MAX_NODES_TILE, engines 1 and 2); the key-tiled
+ * kernel (n_nodes > RRNCO_MAX_NODES_TILE) and the mma.sync engine 0 return RRNCO_ERR_UNSUPPORTED for an active filter:
+ * decode such calls with the per-step entry points (rrnco_decoder_logits_large + rrnco_select_action_filtered). */
+int rrnco_rollout_filtered(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts, int32_t multistart,
+                           int32_t decode_mode, uint64_t seed, const rrnco_decoder_weights_t* w,
+                           const rrnco_decoder_cache_t* cache, const rrnco_instance_data_t* data,
+                           const int64_t* forced_actions, int32_t forced_T, int32_t t_cap, int64_t* actions_out,
+                           float* logprob_out, float* loglik_out, float* norm_reward_out, float* real_reward_out,
+                           int32_t* max_steps_out, uint32_t* status, void* workspace, int32_t top_k, float top_p,
+                           void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Encoder hot spot (SURVEY.md 8(f) rank 4): gating neural adaptive bias of an attention-free block, variant without the

@@ -84,18 +84,23 @@ _SIGNATURES = {
                                              C.c_int32, _f, _f, _f, _f]),
     "rrnco_select_action": (C.c_int, [C.c_int64, C.c_int32, _f, _f, C.c_int32, C.c_float, C.c_float, C.c_uint64,
                                       C.c_int32, _f, _f, _f, _f, _f]),
+    "rrnco_select_action_filtered": (C.c_int, [C.c_int64, C.c_int32, _f, _f, C.c_int32, C.c_float, C.c_float, C.c_uint64,
+                                               C.c_int32, _f, _f, _f, _f, C.c_int32, C.c_float, _f]),
     "rrnco_pointer_ffn_workspace_bytes": (C.c_int64, []),
     "rrnco_pointer_ffn": (C.c_int, [C.c_int64, _f, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_rollout_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int64, C.c_int32]),
     "rrnco_rollout": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_uint64,
                                 C.POINTER(DecoderWeights), C.POINTER(DecoderCache), C.POINTER(InstanceData), _f,
                                 C.c_int32, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f, _f]),
+    "rrnco_rollout_filtered": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_uint64,
+                                         C.POINTER(DecoderWeights), C.POINTER(DecoderCache), C.POINTER(InstanceData), _f,
+                                         C.c_int32, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f, C.c_int32, C.c_float, _f]),
 }
 
 _lib = None
 launch_count = 0  # library calls that enqueued work
 kernel_count = 0  # CUDA kernels those calls launched (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {"rrnco_rollout": 3, "rrnco_pointer_ffn": 2, "rrnco_decoder_logits_large": 4}  # rollout: weight pack + rollout + finalize  # rollout_kernel + finalize_kernel; every other entry point launches one
+_KERNELS_PER_CALL = {"rrnco_rollout": 3, "rrnco_rollout_filtered": 3, "rrnco_pointer_ffn": 2, "rrnco_decoder_logits_large": 4}  # rollout: weight pack + rollout + finalize  # rollout_kernel + finalize_kernel; every other entry point launches one
 
 
 def lib():

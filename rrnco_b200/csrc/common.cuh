@@ -10,6 +10,9 @@
     if (!(cond)) return RRNCO_ERR_BAD_ARG; \
   } while (0)
 
+// a top-k / top-p pair that can drop an entry (top_k > 0, or 0 < top_p < 1): those calls run the filtered kernels
+static inline bool rrnco_filter_active(int32_t top_k, float top_p) { return top_k > 0 || (top_p > 0.f && top_p < 1.f); }
+
 static inline int rrnco_launch_status() {
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? RRNCO_OK : RRNCO_ERR_CUDA;
@@ -110,6 +113,63 @@ __device__ __forceinline__ uint4 philox4x32(uint4 ctr, uint2 key) {
 // so the largest value is 1 - 2^-24 < 1 and -log(-log(u)) stays finite.  (A 24-bit k would round 16777215.5 up to
 // 2^24 and return exactly 1.0 -> +inf Gumbel noise once per 2^24 draws.)
 __host__ __device__ __forceinline__ float u01(uint32_t x) { return ((float)(x >> 9) + 0.5f) * (1.0f / 8388608.0f); }
+
+// ---- decode-time logit filters: top-k / top-p (rl4co process_logits, decoding.py:311-361) --------------------------
+// A filter keeps the set {j : v_j >= cut} of a row's processed values v (after tanh clipping, the mask as -inf and the
+// temperature), so a decoder only needs the cut value and then treats v < cut like a masked entry.
+//   top-k (k > 0, at most the row length): cut = the k-th largest v; ties with it are kept, -inf entries take part.
+//   top-p (0 < p < 1), applied to the top-k survivors: keep j iff the softmax mass of the entries strictly greater than
+//   v_j is < p.  That keeps or drops a tie group as a whole; the top entry is always kept.
+// Both cuts are the largest key K with W(K) >= target, W(K) = sum over the entries with key >= K of a weight (1 for
+// top-k, exp(v - shift) for top-p), found bit by bit on the order-preserving uint32 key of the float.
+__device__ __forceinline__ uint32_t filter_key(float x) {
+  const uint32_t u = __float_as_uint(x + 0.f);  // -0 -> +0: key order = float order for every non-NaN value
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+// Row is how the threads that decode one row hold it: row.for_each(f) calls f(v) on each value this thread owns,
+// row.sum(x) / row.count(c) reduce over the threads that share the row.  Every one of them returns the same cut.
+template <class Row>
+__device__ __forceinline__ float filter_cut(const Row& row, int top_k, float top_p, float shift) {
+  uint32_t kcut = 0u;  // 0: keep everything
+  if (top_k > 0) {
+#pragma unroll 1
+    for (int bit = 31; bit >= 0; --bit) {
+      const uint32_t cand = kcut | (1u << bit);
+      int c = 0;
+      row.for_each([&](float v) { c += filter_key(v) >= cand ? 1 : 0; });
+      if (row.count(c) >= top_k) kcut = cand;
+    }
+  }
+  if (top_p > 0.f && top_p < 1.f) {
+    if (shift == -INFINITY) shift = 0.f;  // no feasible entry (reported by the caller): keep the sums free of NaN
+    float tot = 0.f;
+    row.for_each([&](float v) { tot += filter_key(v) >= kcut ? __expf(v - shift) : 0.f; });
+    const float target = top_p * row.sum(tot);
+    uint32_t pcut = 0u;
+#pragma unroll 1
+    for (int bit = 31; bit >= 0; --bit) {
+      const uint32_t cand = pcut | (1u << bit);
+      const uint32_t lo = cand > kcut ? cand : kcut;
+      float s = 0.f;
+      row.for_each([&](float v) { s += filter_key(v) >= lo ? __expf(v - shift) : 0.f; });
+      if (row.sum(s) >= target) pcut = cand;
+    }
+    kcut = pcut > kcut ? pcut : kcut;
+  }
+  if (kcut <= filter_key(-INFINITY)) return -INFINITY;
+  return __uint_as_float((kcut & 0x80000000u) ? (kcut & 0x7fffffffu) : ~kcut);
+}
+// the whole row in this thread's own memory (no reduction)
+struct FilterRowLocal {
+  const float* v;
+  int n;
+  template <class F>
+  __device__ __forceinline__ void for_each(F&& f) const {
+    for (int i = 0; i < n; ++i) f(v[i]);
+  }
+  __device__ __forceinline__ float sum(float x) const { return x; }
+  __device__ __forceinline__ int count(int c) const { return c; }
+};
 
 // ---- per-device launch configuration ----------------------------------------------------------
 // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) and the SM count belong to a DEVICE, not to the process: launchers

@@ -33,6 +33,8 @@ struct RolloutParams {
   const unsigned char* ffn_packed;  // tcgen05 variant: W1 / W2 packed fp16 hi | lo slices (ffn_pack.cuh)
   const float* ffn_bias_scaled;     // lean engine: kAScale * b1 [512] | kAScale * b2 [128] (written by its weight-pack kernel)
   unsigned char* kv_pack;           // tcgen05 variant: kKvSlots per-SM slots of packed fp16 K | V tiles (kKvSlotBytes each)
+  int32_t top_k;                    // logit filters (filter_cut, common.cuh): read by the filtered instantiations only
+  float top_p;
 };
 
 // Transcendentals of the softmax / bias / clip chain on the SFU (ex2 / lg2 / rcp .approx): absolute error

@@ -199,8 +199,9 @@ __device__ __forceinline__ int cta_sync_and(int pred) {
   return (int)r;
 }
 
-template <int kEnv, int kNTMax, int kPasses, bool kTc>
+template <int kEnv, int kNTMax, int kPasses, bool kTc, bool kFilter>
 __global__ void __launch_bounds__(kTc ? kThreadsTc : kThreads, 1) rollout_kernel(const RolloutParams p) {
+  static_assert(kTc || !kFilter, "the top-k / top-p filters are built for the tcgen05 engine");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
 
@@ -1277,6 +1278,11 @@ __global__ void __launch_bounds__(kTc ? kThreadsTc : kThreads, 1) rollout_kernel
 #pragma unroll
           for (int i = 0; i < 16; ++i) mxl = fmaxf(mxl, __uint_as_float(v[i]));
           tc05::tmem_st16(t_l + 32 * q, v);
+          if (kFilter) {  // the values also overwrite this thread's own columns of the bias tile (read by filter_cut below)
+#pragma unroll
+            for (int i = 0; i < 16; i += 4)
+              *reinterpret_cast<uint4*>(const_cast<float*>(brow) + 32 * q + i) = make_uint4(v[i], v[i + 1], v[i + 2], v[i + 3]);
+          }
         }
         {  // the O tile of the next step's attention accumulates: zero it
           uint32_t z[16];
@@ -1290,6 +1296,12 @@ __global__ void __launch_bounds__(kTc ? kThreadsTc : kThreads, 1) rollout_kernel
         if (nan_seen) atomicOr(p.status, RRNCO_DEV_NAN_LOGITS);
         sm.xf[0][colhalf][row] = mxl;
         cta_sync<kTc>();
+        float cut = -INFINITY;  // top-k / top-p: both threads of the row find the same cut over the row's values
+        if (kFilter) {
+          cut = filter_cut(FilterRowLocal{sm.Bs + row * kLdA, R16}, p.top_k, p.top_p,
+                           fmaxf(sm.xf[0][0][row], sm.xf[0][1][row]));
+          cta_sync<kTc>();
+        }
         // bias tile and logit-key tiles are dead: the producer may load the packed K / V tiles of the next decode step
         if (tid == 0) tc05::mbar_arrive(&sm.bar_kvgo);
         const float mx = fmaxf(sm.xf[0][0][row], sm.xf[0][1][row]);
@@ -1300,6 +1312,10 @@ __global__ void __launch_bounds__(kTc ? kThreadsTc : kThreads, 1) rollout_kernel
           uint32_t v[16];
           tc05::tmem_ld16(t_l + 32 * q, v);
           tc05::tmem_wait_ld();
+          if (kFilter) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(v[i]) < cut ? __float_as_uint(-INFINITY) : v[i];
+          }
 #pragma unroll
           for (int i = 0; i < 16; ++i) sel += fexp(__uint_as_float(v[i]) - mx);
         }
@@ -1322,6 +1338,10 @@ __global__ void __launch_bounds__(kTc ? kThreadsTc : kThreads, 1) rollout_kernel
           uint32_t v[16];
           tc05::tmem_ld16(t_l + 32 * q, v);
           tc05::tmem_wait_ld();
+          if (kFilter) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(v[i]) < cut ? __float_as_uint(-INFINITY) : v[i];
+          }
           const int cbase = 32 * q + hsh;
           if (p.mode == RRNCO_DECODE_SAMPLING) {
 #pragma unroll 1
@@ -1751,9 +1771,9 @@ __global__ void __launch_bounds__(256) finalize_kernel(RolloutParams p, float* l
 
 // The kernel template is instantiated in two translation units so that they compile in parallel:
 // this file (mma.sync FFN, also the logits-only mode) and rollout_kernel_tc.cu (RRNCO_BUILD_TC: tcgen05 FFN).
-template <int kEnv, int kNTMax, int kPasses, bool kTc>
+template <int kEnv, int kNTMax, int kPasses, bool kTc, bool kFilter = false>
 int launch_rollout(const RolloutParams& p, cudaStream_t st) {
-  auto kern = rollout_kernel<kEnv, kNTMax, kPasses, kTc>;
+  auto kern = rollout_kernel<kEnv, kNTMax, kPasses, kTc, kFilter>;
   static PerDeviceOnce once;  // per device ordinal; idempotent attribute, benign if raced
   if (once.first()) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem)) != cudaSuccess) {
@@ -1769,6 +1789,10 @@ int launch_rollout(const RolloutParams& p, cudaStream_t st) {
 
 template <int kEnv, bool kTc>
 int dispatch_rollout(const RolloutParams& p, int passes, cudaStream_t st) {
+  if constexpr (kTc) {
+    if (rrnco_filter_active(p.top_k, p.top_p))  // filtered: the NT <= 16 form only (it serves every N <= 128)
+      return passes == 1 ? launch_rollout<kEnv, 16, 1, true, true>(p, st) : launch_rollout<kEnv, 16, 3, true, true>(p, st);
+  }
   if (p.NT <= 13)
     return passes == 1 ? launch_rollout<kEnv, 13, 1, kTc>(p, st) : launch_rollout<kEnv, 13, 3, kTc>(p, st);
   return passes == 1 ? launch_rollout<kEnv, 16, 1, kTc>(p, st) : launch_rollout<kEnv, 16, 3, kTc>(p, st);
@@ -1959,14 +1983,19 @@ int rrnco_decoder_logits(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n
   return dispatch_env(p, env, g_passes, (cudaStream_t)stream);
 }
 
-int rrnco_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts, int32_t multistart,
-                  int32_t decode_mode, uint64_t seed, const rrnco_decoder_weights_t* w,
-                  const rrnco_decoder_cache_t* cache, const rrnco_instance_data_t* data,
-                  const int64_t* forced_actions, int32_t forced_T, int32_t t_cap, int64_t* actions_out,
-                  float* logprob_out, float* loglik_out, float* norm_reward_out, float* real_reward_out,
-                  int32_t* max_steps_out, uint32_t* status, void* workspace, void* stream) {
+int rrnco_rollout_filtered(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts, int32_t multistart,
+                           int32_t decode_mode, uint64_t seed, const rrnco_decoder_weights_t* w,
+                           const rrnco_decoder_cache_t* cache, const rrnco_instance_data_t* data,
+                           const int64_t* forced_actions, int32_t forced_T, int32_t t_cap, int64_t* actions_out,
+                           float* logprob_out, float* loglik_out, float* norm_reward_out, float* real_reward_out,
+                           int32_t* max_steps_out, uint32_t* status, void* workspace, int32_t top_k, float top_p,
+                           void* stream) {
+  RRNCO_CHECK_ARG(top_k >= 0 && top_p >= 0.f && top_p <= 1.f);  // (a NaN top_p fails both comparisons)
   int rc = check_common(env, n_nodes, n_inst, n_starts, w, cache, data);
   if (rc != RRNCO_OK) return rc;
+  const bool filtered = rrnco_filter_active(top_k, top_p);
+  // a filter needs a row's values at once: the key-tiled kernel never holds them; the mma.sync engine is not built for it
+  if (filtered && (n_nodes > RRNCO_MAX_NODES_TILE || g_engine == 0)) return RRNCO_ERR_UNSUPPORTED;
   RRNCO_CHECK_ARG(actions_out && max_steps_out && status && workspace && aligned16(workspace) && t_cap > 0);
   RRNCO_CHECK_ARG(decode_mode >= 0 && decode_mode <= 2);
   RRNCO_CHECK_ARG(multistart || n_starts == 1);
@@ -1996,6 +2025,7 @@ int rrnco_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts
   p.ffn_bias_scaled = reinterpret_cast<const float*>(packed + kFfnPackedBytes);
   p.kv_pack = packed + kFfnPackedBytes + kLeanBiasBytes;  // 16-byte aligned: every part above is a multiple of 16 bytes
   p.max_steps_out = max_steps_out; p.status = status;
+  p.top_k = filtered ? top_k : 0; p.top_p = filtered ? top_p : 0.f;
   if (cudaMemsetAsync(max_steps_out, 0, sizeof(int32_t), st) != cudaSuccess) return RRNCO_ERR_CUDA;
   g_last_tiled = n_nodes > RRNCO_MAX_NODES_TILE;
   if (n_nodes > RRNCO_MAX_NODES_TILE) {  // key-tiled tcgen05 kernel (the only fused engine for more than one key tile)
@@ -2023,6 +2053,17 @@ int rrnco_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts
     default: finalize_kernel<RRNCO_ENV_RCVRPTW><<<fgrid, 256, 0, st>>>(p, loglik_out, norm_reward_out, real_reward_out); break;
   }
   return rrnco_launch_status();
+}
+
+int rrnco_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts, int32_t multistart,
+                  int32_t decode_mode, uint64_t seed, const rrnco_decoder_weights_t* w,
+                  const rrnco_decoder_cache_t* cache, const rrnco_instance_data_t* data,
+                  const int64_t* forced_actions, int32_t forced_T, int32_t t_cap, int64_t* actions_out,
+                  float* logprob_out, float* loglik_out, float* norm_reward_out, float* real_reward_out,
+                  int32_t* max_steps_out, uint32_t* status, void* workspace, void* stream) {
+  return rrnco_rollout_filtered(env, n_nodes, n_inst, n_starts, multistart, decode_mode, seed, w, cache, data, forced_actions,
+                                forced_T, t_cap, actions_out, logprob_out, loglik_out, norm_reward_out, real_reward_out,
+                                max_steps_out, status, workspace, 0, 0.f, stream);
 }
 
 }  // extern "C"

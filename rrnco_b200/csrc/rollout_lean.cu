@@ -178,7 +178,8 @@ __device__ __forceinline__ float lean_transition(LeanSmem<kEnv>& sm, int N, int 
   return leg;
 }
 
-template <int kEnv, int kPasses>
+// kFilter: decode with the top-k / top-p filters of p (single-pass select only)
+template <int kEnv, int kPasses, bool kFilter>
 __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const RolloutParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   using SmemT = LeanSmem<kEnv>;
@@ -1013,6 +1014,43 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
       float m = clip > 0.f ? __fdiv_rn(clip, temperature) : -INFINITY;
       float ssum = 0.f, best = -INFINITY, bestv = -INFINITY, chk = 0.f;
       int besti = 255;
+      float cut = -INFINITY;
+      if constexpr (kFilter) {
+        // top-k / top-p: the processed values (as computed below) go to TMEM in place and over this thread's own columns
+        // of the bias tile; after the barrier both threads of the row find the same cut over the whole row, and the pass
+        // below reads the values back and drops those under the cut like masked ones
+        float* vrow = reinterpret_cast<float*>(sm.A) + row * kLBiasLd;
+#pragma unroll 1
+        for (int q = 0; q < nq; ++q) {
+          uint32_t v[16];
+          tc05::tmem_ld16(t_l + 32 * q, v);
+          float bv[16];
+#pragma unroll
+          for (int i = 0; i < 16; i += 4) *reinterpret_cast<float4*>(&bv[i]) = *reinterpret_cast<const float4*>(brow + 32 * q + i);
+          const uint32_t mq = mrow[q] >> hsh;
+          tc05::tmem_wait_ld();
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            chk = fmaf(__uint_as_float(v[i]), 0.f, chk);
+            const float u = __fadd_rn(ex2a(fmaf(__uint_as_float(v[i]), k1, -bv[i])), 1e-6f);
+            float x;
+            if (clip > 0.f) x = __fmul_rn(fmaf(-2.0f, rcpa(fmaf(u, u, 1.0f)), 1.0f), clip);
+            else x = flog(u);
+            x = ((mq >> i) & 1u) ? x : -INFINITY;
+            if (temperature != 1.0f) x = __fdiv_rn(x, temperature);
+            v[i] = __float_as_uint(x);
+          }
+          tc05::tmem_st16(t_l + 32 * q, v);
+#pragma unroll
+          for (int i = 0; i < 16; i += 4)
+            *reinterpret_cast<uint4*>(vrow + hsh + 32 * q + i) = make_uint4(v[i], v[i + 1], v[i + 2], v[i + 3]);
+        }
+        tc05::tmem_wait_st();
+        lean_sync();
+        float vmax = -INFINITY;
+        for (int c = 0; c < R16; ++c) vmax = fmaxf(vmax, vrow[c]);
+        cut = filter_cut(FilterRowLocal{vrow, R16}, p.top_k, p.top_p, vmax);
+      }
 #pragma unroll 1
       for (int q = 0; q < nq; ++q) {
         uint32_t v[16];
@@ -1024,6 +1062,10 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
         const int cbase = 32 * q + hsh;
         tc05::tmem_wait_ld();
         float val[16];
+        if constexpr (kFilter) {
+#pragma unroll
+          for (int i = 0; i < 16; ++i) val[i] = __uint_as_float(v[i]) < cut ? -INFINITY : __uint_as_float(v[i]);
+        } else {
         if (clip > 0.f) {
 #pragma unroll
           for (int i = 0; i < 16; ++i) {
@@ -1043,6 +1085,7 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
         if (temperature != 1.0f) {
 #pragma unroll
           for (int i = 0; i < 16; ++i) val[i] = __fdiv_rn(val[i], temperature);
+        }
         }
         float bm = fmaxf(fmaxf(fmaxf(val[0], val[1]), fmaxf(val[2], val[3])), fmaxf(fmaxf(val[4], val[5]), fmaxf(val[6], val[7])));
         bm = fmaxf(bm, fmaxf(fmaxf(fmaxf(val[8], val[9]), fmaxf(val[10], val[11])), fmaxf(fmaxf(val[12], val[13]), fmaxf(val[14], val[15]))));
@@ -1302,9 +1345,9 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
   if (warp == 0) tc05::tmem_dealloc(sm.tmem_base, 256);
 }
 
-template <int kEnv, int kPasses>
+template <int kEnv, int kPasses, bool kFilter>
 static int launch_lean(const RolloutParams& p, cudaStream_t st) {
-  auto kern = rollout_lean_kernel<kEnv, kPasses>;
+  auto kern = rollout_lean_kernel<kEnv, kPasses, kFilter>;
   static PerDeviceOnce once;
   if (once.first()) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LeanSmem<kEnv>)) != cudaSuccess ||
@@ -1342,10 +1385,24 @@ int dispatch_env_lean(const RolloutParams& p, int env, int passes, cudaStream_t 
   static_assert(sizeof(LeanSmem<RRNCO_ENV_RCVRPTW>) <= 115712 && sizeof(LeanSmem<RRNCO_ENV_RCVRP>) <= 115712 &&
                     sizeof(LeanSmem<RRNCO_ENV_ATSP>) <= 115712, "two CTAs per SM need <= 113 KB of shared memory each");
   static_assert(kLBiasBytes + 4 * 2 * kRows * 4 + 2 * kRows <= kRows * kE * 4, "bias tile + exchange arrays fit the A region");
+  if (rrnco_filter_active(p.top_k, p.top_p)) {
+#ifdef RRNCO_LEAN_SELECT3
+    return RRNCO_ERR_UNSUPPORTED;  // the filtered select is built on the single-pass form
+#else
+    switch (env) {
+      case RRNCO_ENV_ATSP: return passes == 1 ? launch_lean<RRNCO_ENV_ATSP, 1, true>(p, st) : launch_lean<RRNCO_ENV_ATSP, 3, true>(p, st);
+      case RRNCO_ENV_RCVRP: return passes == 1 ? launch_lean<RRNCO_ENV_RCVRP, 1, true>(p, st) : launch_lean<RRNCO_ENV_RCVRP, 3, true>(p, st);
+      case RRNCO_ENV_RCVRPTW:
+        return passes == 1 ? launch_lean<RRNCO_ENV_RCVRPTW, 1, true>(p, st) : launch_lean<RRNCO_ENV_RCVRPTW, 3, true>(p, st);
+      default: return RRNCO_ERR_BAD_ARG;
+    }
+#endif
+  }
   switch (env) {
-    case RRNCO_ENV_ATSP: return passes == 1 ? launch_lean<RRNCO_ENV_ATSP, 1>(p, st) : launch_lean<RRNCO_ENV_ATSP, 3>(p, st);
-    case RRNCO_ENV_RCVRP: return passes == 1 ? launch_lean<RRNCO_ENV_RCVRP, 1>(p, st) : launch_lean<RRNCO_ENV_RCVRP, 3>(p, st);
-    case RRNCO_ENV_RCVRPTW: return passes == 1 ? launch_lean<RRNCO_ENV_RCVRPTW, 1>(p, st) : launch_lean<RRNCO_ENV_RCVRPTW, 3>(p, st);
+    case RRNCO_ENV_ATSP: return passes == 1 ? launch_lean<RRNCO_ENV_ATSP, 1, false>(p, st) : launch_lean<RRNCO_ENV_ATSP, 3, false>(p, st);
+    case RRNCO_ENV_RCVRP: return passes == 1 ? launch_lean<RRNCO_ENV_RCVRP, 1, false>(p, st) : launch_lean<RRNCO_ENV_RCVRP, 3, false>(p, st);
+    case RRNCO_ENV_RCVRPTW:
+      return passes == 1 ? launch_lean<RRNCO_ENV_RCVRPTW, 1, false>(p, st) : launch_lean<RRNCO_ENV_RCVRPTW, 3, false>(p, st);
     default: return RRNCO_ERR_BAD_ARG;
   }
 }

@@ -388,13 +388,34 @@ __global__ void __launch_bounds__(256) logits_mma_kernel(const StepArgs a, int n
   if (__any_sync(0xffffffffu, nan_seen) && lane == 0) atomicOr(a.status, RRNCO_DEV_NAN_LOGITS);
 }
 
-// DecodingStrategy.step: process_logits (tanh clip, mask, temperature, log-softmax) + greedy / Gumbel-max / forced
+// a row of select_action_kernel for filter_cut: one warp, lane l owns the columns l, l + 32, ...
+template <class Clipped>
+struct FilterRowWarp {
+  const Clipped& clipped;
+  int N, lane;
+  template <class F>
+  __device__ __forceinline__ void for_each(F&& f) const {
+    for (int n = lane; n < N; n += 32) f(clipped(n));
+  }
+  __device__ __forceinline__ float sum(float x) const {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+    return x;
+  }
+  __device__ __forceinline__ int count(int c) const { return __reduce_add_sync(0xffffffffu, c); }
+};
+
+// DecodingStrategy.step: process_logits (tanh clip, mask, temperature, [top-k, top-p,] log-softmax) + greedy / Gumbel-max /
+// forced.  kFilter: entries below the cut of filter_cut are dropped like masked ones (a forced action among them gets
+// log p = -inf and is not reported as infeasible); every column draws the same Gumbel noise as without a filter.
+template <bool kFilter>
 __global__ void __launch_bounds__(kStepWarps * 32) select_action_kernel(int64_t R, int N, const float* __restrict__ logits,
                                                                        const uint8_t* __restrict__ mask, int mode,
                                                                        float tanh_clip, float temperature, uint64_t seed,
                                                                        int step, const int64_t* __restrict__ forced,
                                                                        int64_t* __restrict__ action_out,
-                                                                       float* __restrict__ logp_out, uint32_t* status) {
+                                                                       float* __restrict__ logp_out, uint32_t* status,
+                                                                       int top_k, float top_p) {
   const int64_t r = (int64_t)blockIdx.x * kStepWarps + (threadIdx.x >> 5);
   if (r >= R) return;
   const int lane = threadIdx.x & 31;
@@ -408,8 +429,15 @@ __global__ void __launch_bounds__(kStepWarps * 32) select_action_kernel(int64_t 
   float mx = -INFINITY;
   for (int n = lane; n < N; n += 32) mx = fmaxf(mx, clipped(n));
   mx = warp_max(mx);
+  float cut = -INFINITY;
+  if constexpr (kFilter) cut = filter_cut(FilterRowWarp<decltype(clipped)>{clipped, N, lane}, top_k, top_p, mx);
+  auto kept = [&](int n) -> float {  // clipped(n), or -inf when the filter drops it
+    const float v = clipped(n);
+    if constexpr (kFilter) return v < cut ? -INFINITY : v;
+    return v;
+  };
   float se = 0.f;
-  for (int n = lane; n < N; n += 32) se += sfexp(clipped(n) - mx);
+  for (int n = lane; n < N; n += 32) se += sfexp((kFilter ? kept(n) : clipped(n)) - mx);
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
   se = __logf(se);
@@ -417,7 +445,7 @@ __global__ void __launch_bounds__(kStepWarps * 32) select_action_kernel(int64_t 
   int besti = 0x7fffffff;
   const uint2 key2 = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
   for (int n = lane; n < N; n += 32) {
-    const float lp = __fsub_rn(__fsub_rn(clipped(n), mx), se);
+    const float lp = __fsub_rn(__fsub_rn(kFilter ? kept(n) : clipped(n), mx), se);
     float key = lp;
     if (mode == RRNCO_DECODE_SAMPLING) {  // same stream as the fused kernel: Philox(seed; (r, step, n >> 2))[n & 3]
       const uint4 rnd = philox4x32(make_uint4((uint32_t)r, (uint32_t)(r >> 32), (uint32_t)step, (uint32_t)(n >> 2)), key2);
@@ -438,7 +466,7 @@ __global__ void __launch_bounds__(kStepWarps * 32) select_action_kernel(int64_t 
   if (lane == 0) {
     if (!mrow[act]) atomicOr(status, besti == 0x7fffffff ? RRNCO_DEV_NO_FEASIBLE : RRNCO_DEV_INFEASIBLE);
     action_out[r] = act;
-    logp_out[r] = __fsub_rn(__fsub_rn(clipped(act), mx), se);
+    logp_out[r] = __fsub_rn(__fsub_rn(kFilter ? kept(act) : clipped(act), mx), se);
   }
 }
 
@@ -548,17 +576,28 @@ int rrnco_decoder_logits_large(int32_t env, int32_t n_nodes, int64_t n_inst, int
   return rrnco_launch_status();
 }
 
-int rrnco_select_action(int64_t n_rollouts, int32_t n_nodes, const float* logits, const uint8_t* mask, int32_t decode_mode,
-                        float tanh_clipping, float temperature, uint64_t seed, int32_t step, const int64_t* forced_action,
-                        int64_t* action_out, float* logprob_out, uint32_t* status, void* stream) {
+int rrnco_select_action_filtered(int64_t n_rollouts, int32_t n_nodes, const float* logits, const uint8_t* mask,
+                                 int32_t decode_mode, float tanh_clipping, float temperature, uint64_t seed, int32_t step,
+                                 const int64_t* forced_action, int64_t* action_out, float* logprob_out, uint32_t* status,
+                                 int32_t top_k, float top_p, void* stream) {
+  RRNCO_CHECK_ARG(top_k >= 0 && top_p >= 0.f && top_p <= 1.f);  // (a NaN top_p fails both comparisons)
   if (n_rollouts == 0) return RRNCO_OK;
   RRNCO_CHECK_ARG(n_rollouts > 0 && n_nodes > 0 && logits && mask && action_out && logprob_out && status);
   RRNCO_CHECK_ARG(decode_mode >= 0 && decode_mode <= 2 && temperature > 0.f);
   RRNCO_CHECK_ARG(decode_mode != RRNCO_DECODE_EVALUATE || forced_action);
-  select_action_kernel<<<(unsigned)((n_rollouts + kStepWarps - 1) / kStepWarps), kStepWarps * 32, 0, (cudaStream_t)stream>>>(
-      n_rollouts, n_nodes, logits, mask, decode_mode, tanh_clipping, temperature, seed, step, forced_action, action_out,
-      logprob_out, status);
+  const unsigned grid = (unsigned)((n_rollouts + kStepWarps - 1) / kStepWarps);
+  auto kern = rrnco_filter_active(top_k, top_p) ? select_action_kernel<true> : select_action_kernel<false>;
+  kern<<<grid, kStepWarps * 32, 0, (cudaStream_t)stream>>>(n_rollouts, n_nodes, logits, mask, decode_mode, tanh_clipping,
+                                                           temperature, seed, step, forced_action, action_out, logprob_out,
+                                                           status, top_k, top_p);
   return rrnco_launch_status();
+}
+
+int rrnco_select_action(int64_t n_rollouts, int32_t n_nodes, const float* logits, const uint8_t* mask, int32_t decode_mode,
+                        float tanh_clipping, float temperature, uint64_t seed, int32_t step, const int64_t* forced_action,
+                        int64_t* action_out, float* logprob_out, uint32_t* status, void* stream) {
+  return rrnco_select_action_filtered(n_rollouts, n_nodes, logits, mask, decode_mode, tanh_clipping, temperature, seed, step,
+                                      forced_action, action_out, logprob_out, status, 0, 0.f, stream);
 }
 
 }  // extern "C"

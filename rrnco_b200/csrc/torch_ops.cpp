@@ -33,6 +33,8 @@ Tensor u8c(const Tensor& t) {
   Tensor c = t.contiguous();
   return c.scalar_type() == at::kBool ? c.view(at::kByte) : c.to(at::kByte);
 }
+// top_k above the row length keeps every entry; a negative one reaches the C ABI, which rejects it
+int32_t clamp_k(int64_t k) { return k > INT32_MAX ? INT32_MAX : k < 0 ? -1 : (int32_t)k; }
 template <typename T>
 const T* cptr(const OptTensor& t) { return t.has_value() && t->defined() ? t->data_ptr<T>() : nullptr; }
 
@@ -135,7 +137,8 @@ std::tuple<Tensor, Tensor> tour_reward(const Tensor& actions, const Tensor& dist
 
 // -> (action, log-prob); `status` (int32 [1]) is OR-ed in place
 std::tuple<Tensor, Tensor> select_action(const Tensor& logits, const Tensor& mask, int64_t decode_mode, double tanh_clipping,
-                                         double temperature, int64_t seed, int64_t step, const OptTensor& forced, Tensor status) {
+                                         double temperature, int64_t seed, int64_t step, const OptTensor& forced, Tensor status,
+                                         int64_t top_k, double top_p) {
   TORCH_CHECK(logits.is_cuda() && logits.dim() == 2, "logits [R,N] on CUDA expected");
   c10::cuda::CUDAGuard guard(logits.device());
   Tensor lg = f32c(logits), m = u8c(mask);
@@ -143,10 +146,11 @@ std::tuple<Tensor, Tensor> select_action(const Tensor& logits, const Tensor& mas
   Tensor action = at::empty({R}, lg.options().dtype(at::kLong)), logp = at::empty({R}, lg.options());
   Tensor f;
   if (forced.has_value() && forced->defined()) f = forced->contiguous();
-  check_rc(rrnco_select_action(R, (int32_t)N, lg.data_ptr<float>(), m.data_ptr<uint8_t>(), (int32_t)decode_mode,
-                               (float)tanh_clipping, (float)temperature, (uint64_t)seed, (int32_t)step,
-                               f.defined() ? f.data_ptr<int64_t>() : nullptr, action.data_ptr<int64_t>(), logp.data_ptr<float>(),
-                               reinterpret_cast<uint32_t*>(status.data_ptr<int32_t>()), stream_of(lg)), "select_action");
+  check_rc(rrnco_select_action_filtered(R, (int32_t)N, lg.data_ptr<float>(), m.data_ptr<uint8_t>(), (int32_t)decode_mode,
+                                        (float)tanh_clipping, (float)temperature, (uint64_t)seed, (int32_t)step,
+                                        f.defined() ? f.data_ptr<int64_t>() : nullptr, action.data_ptr<int64_t>(),
+                                        logp.data_ptr<float>(), reinterpret_cast<uint32_t*>(status.data_ptr<int32_t>()),
+                                        clamp_k(top_k), (float)top_p, stream_of(lg)), "select_action");
   return {action, logp};
 }
 
@@ -159,7 +163,8 @@ std::tuple<Tensor, Tensor> select_action(const Tensor& logits, const Tensor& mas
 std::tuple<Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor> rollout(
     int64_t env, int64_t n_starts, bool multistart, int64_t decode_mode, int64_t seed, const c10::List<OptTensor>& weights,
     double alpha, double beta, double tanh_clipping, double temperature, const c10::List<OptTensor>& cache,
-    const c10::List<OptTensor>& data, const OptTensor& forced_actions, int64_t t_cap, bool per_step_logprobs, Tensor workspace) {
+    const c10::List<OptTensor>& data, const OptTensor& forced_actions, int64_t t_cap, bool per_step_logprobs, Tensor workspace,
+    int64_t top_k, double top_p) {
   TORCH_CHECK(weights.size() == 6 && cache.size() == 5 && data.size() == 12, "rollout: weights[6], cache[5], data[12] expected");
   auto W = [&](size_t i) -> OptTensor { return weights.get(i); };
   auto C = [&](size_t i) -> OptTensor { return cache.get(i); };
@@ -197,12 +202,13 @@ std::tuple<Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor> rollout(
   const int64_t need = rrnco_rollout_workspace_bytes((int32_t)env, (int32_t)N, n_inst, (int32_t)n_starts);
   TORCH_CHECK(workspace.is_cuda() && workspace.scalar_type() == at::kByte && workspace.numel() >= need,
               "rollout: workspace of >= ", need, " bytes (uint8, CUDA) expected");
-  check_rc(rrnco_rollout((int32_t)env, (int32_t)N, n_inst, (int32_t)n_starts, multistart ? 1 : 0, (int32_t)decode_mode,
-                         (uint64_t)seed, &w, &c, &d, forced.defined() ? forced.data_ptr<int64_t>() : nullptr, (int32_t)forced_T,
-                         (int32_t)t_cap, actions.data_ptr<int64_t>(), per_step_logprobs ? logprob.data_ptr<float>() : nullptr,
-                         ll.data_ptr<float>(), norm.data_ptr<float>(), has_mm ? real.data_ptr<float>() : nullptr,
-                         info.data_ptr<int32_t>(), reinterpret_cast<uint32_t*>(info.data_ptr<int32_t>() + 1),
-                         workspace.data_ptr<uint8_t>(), stream_of(key)), "rollout");
+  check_rc(rrnco_rollout_filtered((int32_t)env, (int32_t)N, n_inst, (int32_t)n_starts, multistart ? 1 : 0, (int32_t)decode_mode,
+                                  (uint64_t)seed, &w, &c, &d, forced.defined() ? forced.data_ptr<int64_t>() : nullptr,
+                                  (int32_t)forced_T, (int32_t)t_cap, actions.data_ptr<int64_t>(),
+                                  per_step_logprobs ? logprob.data_ptr<float>() : nullptr, ll.data_ptr<float>(),
+                                  norm.data_ptr<float>(), has_mm ? real.data_ptr<float>() : nullptr, info.data_ptr<int32_t>(),
+                                  reinterpret_cast<uint32_t*>(info.data_ptr<int32_t>() + 1), workspace.data_ptr<uint8_t>(),
+                                  clamp_k(top_k), (float)top_p, stream_of(key)), "rollout");
   const int64_t tile_rows = rrnco_rollout_tile_rows((int32_t)env, (int32_t)N, n_inst, (int32_t)n_starts);
   const int64_t n_tiles = n_inst * ((n_starts + tile_rows - 1) / tile_rows);
   Tensor tile_steps = workspace.narrow(0, 2 * R * 8, 4 * n_tiles).view(at::kInt);
@@ -224,10 +230,11 @@ TORCH_LIBRARY(rrnco_b200, m) {
   m.def("tour_reward(Tensor actions, Tensor distance, bool prepend_depot, Tensor? open_route, Tensor? min_d, Tensor? max_d) -> "
         "(Tensor, Tensor)");
   m.def("select_action(Tensor logits, Tensor mask, int decode_mode, float tanh_clipping, float temperature, int seed, int step, "
-        "Tensor? forced, Tensor(a!) status) -> (Tensor, Tensor)");
+        "Tensor? forced, Tensor(a!) status, int top_k=0, float top_p=0.0) -> (Tensor, Tensor)");
   m.def("rollout(int env, int n_starts, bool multistart, int decode_mode, int seed, Tensor?[] weights, float alpha, float beta, "
         "float tanh_clipping, float temperature, Tensor?[] cache, Tensor?[] data, Tensor? forced_actions, int t_cap, "
-        "bool per_step_logprobs, Tensor(a!) workspace) -> (Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)");
+        "bool per_step_logprobs, Tensor(a!) workspace, int top_k=0, float top_p=0.0) -> "
+        "(Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)");
   m.def("rollout_workspace_bytes(int env, int n_nodes, int n_inst, int n_starts) -> int", &rollout_workspace_bytes);
 }
 

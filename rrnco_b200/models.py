@@ -6,8 +6,10 @@ decoder and the whole decode loop running as fused sm_100a kernels (librrnco_b20
   RRNetPolicy   <- rrnco/models/policy.py:19-255; `forward` returns the same out-dict.  The encoder stays the
                    reference's PyTorch module (pass it as `encoder=`), as BASELINE.json's north star states.
 
-Unsupported reference options raise NotImplementedError (beam search, top-k / top-p, select_best,
-store_all_logp / return_entropy, mask_logits=False, dynamic embeddings): they are not on any BASELINE config.
+The logit filters `top_k` / `top_p` of rl4co's `process_logits` run inside the decode kernels (any decode type), except
+under grad in phase "train" without forced actions: the differentiable replay does not filter, so that call raises.
+Unsupported reference options raise NotImplementedError (beam search, select_best, store_all_logp / return_entropy,
+mask_logits=False, dynamic embeddings): they are not on any BASELINE config.
 """
 from __future__ import annotations
 
@@ -291,9 +293,11 @@ class RRNetPolicy(nn.Module):
             raise ValueError("pass an instantiated rrnco_b200 env")
         if return_entropy or decoding_kwargs.get("store_all_logp"):
             raise NotImplementedError("store_all_logp / return_entropy")
-        for k in ("top_k", "top_p"):
-            if decoding_kwargs.get(k):
-                raise NotImplementedError(k)
+        top_k, top_p = filter_args(decoding_kwargs.pop("top_k", None), decoding_kwargs.pop("top_p", None))
+        filtered = filter_active(top_k, top_p)
+        if filtered and phase == "train" and torch.is_grad_enabled() and actions is None:
+            raise NotImplementedError("top_k / top_p under grad in phase 'train': the differentiable replay of the sampled "
+                                      "actions (training.batched_logprobs) does not filter")
         if decoding_kwargs.get("select_best"):
             raise NotImplementedError("select_best")
         if td.device.type != "cuda":
@@ -322,12 +326,15 @@ class RRNetPolicy(nn.Module):
         self._calls += 1
         n_nodes = cache.glimpse_key.shape[1]
         # N <= 128: single-tile fused kernels; N <= 1024: key-tiled fused kernel; beyond (or large_n_path = "stepwise"): the
-        # per-step kernel pipeline
-        use_fused = n_nodes <= _lib.MAX_NODES_TILE or (n_nodes <= _lib.MAX_NODES_FUSED and self.large_n_path == "fused")
+        # per-step kernel pipeline.  top-k / top-p above 128 nodes: the per-step pipeline (the key-tiled kernel never holds
+        # a whole row of scores, which the filters need)
+        use_fused = n_nodes <= _lib.MAX_NODES_TILE or (n_nodes <= _lib.MAX_NODES_FUSED and self.large_n_path == "fused"
+                                                       and not filtered)
         rollout_fn = fused_rollout if use_fused else stepwise_rollout
         rollout_args = dict(forced_actions=actions, seed=decoding_kwargs.pop("seed", self._seed_base() + self._calls),
                             temperature=temperature, tanh_clipping=tanh_clipping, calc_reward=calc_reward,
-                            per_step_logprobs=not return_sum_log_likelihood, check=self.decoder.check_nan)
+                            per_step_logprobs=not return_sum_log_likelihood, check=self.decoder.check_nan,
+                            top_k=top_k, top_p=top_p)
         try:
             out = rollout_fn(self.decoder, cache, env, td, S, multistart, decode_type.replace("multistart_", ""), **rollout_args)
         except SoftmaxRangeError:
@@ -363,6 +370,24 @@ class RRNetPolicy(nn.Module):
 FALLBACKS = {"softmax_range": 0}  # rollouts re-run through the per-step pipeline (diagnostics)
 
 
+def filter_args(top_k=None, top_p=None) -> Tuple[int, float]:
+    """rl4co's `top_k` / `top_p` decoding arguments as (int, float), None meaning off; raises ValueError for values the
+    kernels reject (top_k < 0, top_p outside [0, 1] or NaN), before anything is launched."""
+    k = 0 if top_k is None else top_k
+    p = 0.0 if top_p is None else top_p
+    if isinstance(k, bool) or int(k) != k or k < 0:
+        raise ValueError(f"top_k must be a non-negative integer (got {top_k!r})")
+    p = float(p)
+    if not 0.0 <= p <= 1.0:  # (NaN fails too)
+        raise ValueError(f"top_p must be in [0, 1] (got {top_p!r})")
+    return int(k), p
+
+
+def filter_active(top_k: int, top_p: float) -> bool:
+    """True when the filters can drop an entry (top_k > 0, or 0 < top_p < 1)."""
+    return top_k > 0 or 0.0 < top_p < 1.0
+
+
 class SoftmaxRangeError(RuntimeError):
     """RRNCO_DEV_SOFTMAX_RANGE: the key-tiled fused kernel cannot represent this model's attention scores; its outputs
     were discarded (use stepwise_rollout)."""
@@ -385,8 +410,10 @@ def _workspace(dev, nbytes: int):
 def fused_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, num_starts: int, multistart: bool,
                   kind: str, forced_actions=None, seed: int = 0, temperature: float = 1.0, tanh_clipping: float = 10.0,
                   calc_reward: bool = True, per_step_logprobs: bool = False, check: bool = True,
-                  t_cap: Optional[int] = None) -> dict:
-    """policy.py:203-243 as ONE kernel launch (+ a finalize kernel).  `td` is the reset td ([n_inst] batch)."""
+                  t_cap: Optional[int] = None, top_k: int = 0, top_p: float = 0.0) -> dict:
+    """policy.py:203-243 as ONE kernel launch (+ a finalize kernel).  `td` is the reset td ([n_inst] batch).
+    top_k / top_p: rl4co's logit filters (N <= 128 only; larger N: stepwise_rollout)."""
+    top_k, top_p = filter_args(top_k, top_p)
     name = decoder.env_name
     dev = cache.glimpse_key.device
     n_inst, N, _ = cache.glimpse_key.shape
@@ -394,6 +421,9 @@ def fused_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, num_s
     R = n_inst * S
     if N > _lib.MAX_NODES_FUSED:
         raise NotImplementedError(f"fused rollout supports N <= {_lib.MAX_NODES_FUSED} nodes (got {N})")
+    if filter_active(top_k, top_p) and N > _lib.MAX_NODES_TILE:
+        raise NotImplementedError(f"top_k / top_p in the fused rollout need N <= {_lib.MAX_NODES_TILE} (got {N}): use "
+                                  "stepwise_rollout")
     num_loc = getattr(getattr(env, "generator", None), "num_loc", None)
     if multistart and num_loc is not None and num_loc != (N if name == "atsp" else N - 1):
         # select_start_nodes is `arange(S) % generator.num_loc` upstream; the kernel derives it from the instance size
@@ -417,7 +447,7 @@ def fused_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, num_s
         acts, logp, ll, norm, real, info, _ = torch_ops.ops().rollout(
             ENV_ID[name], S, bool(multistart), DECODE_ID[kind], seed, wt, alpha, beta, float(tanh_clipping), float(temperature),
             [cache.glimpse_key, cache.glimpse_val, cache.logit_key, cache.ctx_node_proj, cache.ctx_node_proj2],
-            instance_tensors_from_td(name, td), forced, t_cap, bool(per_step_logprobs), ws)
+            instance_tensors_from_td(name, td), forced, t_cap, bool(per_step_logprobs), ws, top_k, top_p)
         _lib.count_call("rrnco_rollout")
         real = real if has_minmax else None
     else:
@@ -431,9 +461,9 @@ def fused_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, num_s
         real = torch.empty(R, dtype=torch.float32, device=dev) if has_minmax else None
         info = torch.zeros(2, dtype=torch.int32, device=dev)  # [max_steps, status]
         cs = cache.struct()
-        call("rrnco_rollout", ENV_ID[name], N, n_inst, S, int(multistart), DECODE_ID[kind], seed,
+        call("rrnco_rollout_filtered", ENV_ID[name], N, n_inst, S, int(multistart), DECODE_ID[kind], seed,
              C.byref(w), C.byref(cs), C.byref(data), ptr(forced), forced_T, t_cap, ptr(acts), ptr(logp), ptr(ll),
-             ptr(norm), ptr(real), ptr(info[0:1]), ptr(info[1:2]), ptr(ws), stream_ptr(dev))
+             ptr(norm), ptr(real), ptr(info[0:1]), ptr(info[1:2]), ptr(ws), min(top_k, 2**31 - 1), top_p, stream_ptr(dev))
     T, status = info.tolist()  # the ONE host sync of the rollout (upstream: 3-5 per decode step)
     if status & _lib.DEV_SOFTMAX_RANGE:  # never silently inaccurate, whatever `check` says
         raise SoftmaxRangeError("attention scores outside the range of the key-tiled kernel's fixed softmax shift")
@@ -458,15 +488,18 @@ def fused_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, num_s
 
 
 def select_action(logits, mask, kind: str = "greedy", tanh_clipping: float = 10.0, temperature: float = 1.0,
-                  seed: int = 0, step: int = 0, forced_action=None, status=None):
-    """DecodingStrategy.step (decoding.py:219-298): (action int64 [R], log-prob fp32 [R]) in one kernel."""
+                  seed: int = 0, step: int = 0, forced_action=None, status=None, top_k: int = 0, top_p: float = 0.0):
+    """DecodingStrategy.step (decoding.py:219-298): (action int64 [R], log-prob fp32 [R]) in one kernel, with rl4co's
+    top_k / top_p logit filters (decoding.py:311-361; include/rrnco_b200.h describes the tie rule)."""
+    top_k, top_p = filter_args(top_k, top_p)
     if status is None:
         status = torch.zeros(1, dtype=torch.int32, device=logits.device)
     from . import torch_ops
     if torch_ops.enabled():
         _lib.count_call("rrnco_select_action")
         action, logp = torch_ops.ops().select_action(logits, mask, DECODE_ID[kind], float(tanh_clipping), float(temperature),
-                                                     int(seed) & (2**63 - 1), int(step), forced_action, status)
+                                                     int(seed) & (2**63 - 1), int(step), forced_action, status, top_k,
+                                                     top_p)
         return action, logp, status
     logits, mask = logits.contiguous(), mask.contiguous()
     R, N = logits.shape
@@ -475,9 +508,9 @@ def select_action(logits, mask, kind: str = "greedy", tanh_clipping: float = 10.
     if status is None:
         status = torch.zeros(1, dtype=torch.int32, device=logits.device)
     forced = None if forced_action is None else forced_action.contiguous()
-    call("rrnco_select_action", R, N, ptr(logits), ptr(_u8(mask)), DECODE_ID[kind], float(tanh_clipping),
+    call("rrnco_select_action_filtered", R, N, ptr(logits), ptr(_u8(mask)), DECODE_ID[kind], float(tanh_clipping),
          float(temperature), int(seed) & (2**63 - 1), int(step), ptr(forced), ptr(action), ptr(logp), ptr(status),
-         stream_ptr(logits.device))
+         min(top_k, 2**31 - 1), top_p, stream_ptr(logits.device))
     return action, logp, status
 
 
@@ -492,11 +525,14 @@ _ROLLOUT_STATE_KEYS = {
 
 def stepwise_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, num_starts: int, multistart: bool,
                      kind: str, forced_actions=None, seed: int = 0, temperature: float = 1.0, tanh_clipping: float = 10.0,
-                     calc_reward: bool = True, per_step_logprobs: bool = False, check: bool = True, t_cap=None) -> dict:
+                     calc_reward: bool = True, per_step_logprobs: bool = False, check: bool = True, t_cap=None,
+                     top_k: int = 0, top_p: float = 0.0) -> dict:
     """policy.py:203-243 as a per-step kernel pipeline for ANY number of nodes (decoder_logits_large ->
     select_action -> env step), used when N exceeds the fused kernel's 128-key tile.  Only the rollout STATE is
     replicated over the POMO starts; matrices / demands / time windows stay one copy per instance (the kernels
-    index row r % data_rows), so the n=1000 configs never materialise upstream's S-fold `batchify` of [N,N] data."""
+    index row r % data_rows), so the n=1000 configs never materialise upstream's S-fold `batchify` of [N,N] data.
+    top_k / top_p: rl4co's logit filters, for any N."""
+    top_k, top_p = filter_args(top_k, top_p)
     from .tdlite import TensorDictLite, batchify
     from .envs import tour_reward
     name = decoder.env_name
@@ -527,7 +563,7 @@ def stepwise_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, nu
             break
         logits, mask = decoder(roll, cache, S)
         forced = forced_actions[:, step].to(dev) if kind == "evaluate" else None
-        a, lp, status = select_action(logits, mask, kind, tanh_clipping, temperature, seed, step, forced, status)
+        a, lp, status = select_action(logits, mask, kind, tanh_clipping, temperature, seed, step, forced, status, top_k, top_p)
         roll.set("action", a)
         roll = env.step(roll)["next"]
         done = roll["done"]
