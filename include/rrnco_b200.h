@@ -50,6 +50,7 @@ extern "C" {
 #define RRNCO_DEV_SOFTMAX_RANGE 16u   /* key-tiled fused kernel (N > RRNCO_MAX_NODES_TILE) only: an attention head's scores
                                          exceed the range its fixed softmax shift covers (|q_h| max|k_h| / 4 > 4.85); the
                                          rollout's outputs must be discarded and the per-step entry points used instead */
+#define RRNCO_DEV_BAD_PARENT 32u      /* rrnco_beam_backtrack: a parent row outside [0, n_rows) (corrupted beam records) */
 
 #define RRNCO_ENV_ATSP 0
 #define RRNCO_ENV_RCVRP 1
@@ -285,6 +286,31 @@ int rrnco_select_action_filtered(int64_t n_rollouts, int32_t n_nodes, const floa
                                  int32_t decode_mode, float tanh_clipping, float temperature, uint64_t seed, int32_t step,
                                  const int64_t* forced_action, int64_t* action_out, float* logprob_out, uint32_t* status,
                                  int32_t top_k, float top_p, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
+ * Beam search (rl4co BeamSearch._make_beam_step / _backtrack, decoding.py:402-542), one decode step per call.
+ *   Rows r = w * n_inst + b (beam w of instance b, the (w b) order of batchify).  Beam w's log-probs lp[r, n] are the
+ *   per-row math of rrnco_select_action (tanh clipping, mask, temperature, log-softmax); the candidates of instance b are
+ *   score_in[r] + lp[r, n] with flat index w * n_nodes + n.  The beam_width largest, ranked by (value descending, flat
+ *   index ascending: lower index first among equal values), become the new beams: rank w' writes row w' * n_inst + b with
+ *   action_out = n, parent_out = the parent's ROW (w * n_inst + b), logprob_out = lp[parent, n], score_out = the candidate
+ *   value (fp32, score + lp).  When fewer than beam_width candidates are finite, ranks from #finite upward copy rank 0
+ *   (no finite candidate at all sets RRNCO_DEV_NO_FEASIBLE).  score_out may alias score_in.
+ *   beam_width < 2: RRNCO_ERR_BAD_ARG; > RRNCO_MAX_BEAM_WIDTH: RRNCO_ERR_UNSUPPORTED; both before any CUDA call.
+ *
+ * rrnco_beam_backtrack: actions / parents int64 and logprobs fp32, step-major [n_steps, n_rows] (row t = what step t
+ *   wrote; parents of step 0 are never read) -> actions_out int64 [n_rows, n_steps], logprob_out fp32 [n_rows, n_steps]
+ *   (may be NULL) aligned along the path of final beam r, loglik_out fp32 [n_rows] = their fp64 sum.  A parent row
+ *   outside [0, n_rows) sets RRNCO_DEV_BAD_PARENT in `status`; that row's earlier steps come out as action 0 with
+ *   log-prob NaN and its log-likelihood is NaN.
+ * ---------------------------------------------------------------------------------------------- */
+#define RRNCO_MAX_BEAM_WIDTH 1024
+int rrnco_beam_select(int64_t n_inst, int32_t beam_width, int32_t n_nodes, const float* logits, const uint8_t* mask,
+                      const float* score_in, float tanh_clipping, float temperature, int64_t* action_out, int64_t* parent_out,
+                      float* logprob_out, float* score_out, uint32_t* status, void* stream);
+int rrnco_beam_backtrack(int64_t n_rows, int32_t n_steps, const int64_t* actions, const int64_t* parents,
+                         const float* logprobs, int64_t* actions_out, float* logprob_out, float* loglik_out,
+                         uint32_t* status, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Fused construction rollout = RRNetPolicy.forward decode loop  rrnco/models/policy.py:203-243

@@ -11,8 +11,8 @@ No CPU fallback, no Triton / torch.compile: if the CUDA library is missing, call
 """
 from ._lib import RRNCOError, set_ffn_engine, set_precision, set_step_tiling  # noqa: F401
 from .envs import ATSPEnv, RCVRPEnv, RMTVRPEnv, get_env  # noqa: F401
-from .models import (PrecomputedCache, RRNetDecoder, RRNetPolicy, fused_rollout, select_action,  # noqa: F401
-                     stepwise_rollout)
+from .models import (PrecomputedCache, RRNetDecoder, RRNetPolicy, beam_backtrack, beam_search_rollout,  # noqa: F401
+                     beam_select, fused_rollout, select_action, stepwise_rollout)
 from .dataio import iter_batches, load_city_npz, load_npz_to_tensordict, prepare_test_td  # noqa: F401
 from .hostio import HostPrefetcher  # noqa: F401
 from .sampler import CityOnDevice, Real_World_Sampler, remove_outlier_points  # noqa: F401
@@ -25,7 +25,7 @@ from .training import (batched_logprobs, collect_decode_inputs, iter_decode_inpu
                        replay_log_likelihood)
 
 __all__ = ["ATSPEnv", "RCVRPEnv", "RMTVRPEnv", "get_env", "RRNetDecoder", "RRNetPolicy", "PrecomputedCache",
-           "fused_rollout", "stepwise_rollout", "select_action", "Real_World_Sampler", "TensorDictLite", "batchify", "unbatchify", "set_precision", "set_ffn_engine", "set_step_tiling",
+           "fused_rollout", "stepwise_rollout", "select_action", "beam_search_rollout", "beam_select", "beam_backtrack", "Real_World_Sampler", "TensorDictLite", "batchify", "unbatchify", "set_precision", "set_ffn_engine", "set_step_tiling",
            "RRNCOError", "HostPrefetcher", "load_city_npz", "load_npz_to_tensordict", "prepare_test_td", "iter_batches", "replay_log_likelihood", "batched_logprobs", "collect_decode_inputs", "iter_decode_inputs",
            "pomo_shared_baseline_loss", "CityOnDevice", "remove_outlier_points", "LazyATSPGenerator", "LazyRCVRPGenerator",
            "LazyRMTVRPGenerator", "StateAugmentation", "dihedral_8_augmentation"]

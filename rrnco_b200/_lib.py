@@ -16,8 +16,10 @@ LIB_PATH = os.path.join(_HERE, "librrnco_b200.so")
 ENV_ID = {"atsp": 0, "rcvrp": 1, "rcvrptw": 2}
 DECODE_ID = {"greedy": 0, "sampling": 1, "evaluate": 2}
 DEV_NAN_LOGITS, DEV_INFEASIBLE, DEV_NO_FEASIBLE, DEV_TRUNCATED, DEV_SOFTMAX_RANGE = 1, 2, 4, 8, 16
+DEV_BAD_PARENT = 32
 MAX_NODES_TILE = 128     # one key tile: rrnco_decoder_logits, single-tile fused kernels
 MAX_NODES_FUSED = 1024   # rrnco_rollout (key-tiled kernel above MAX_NODES_TILE)
+MAX_BEAM_WIDTH = 1024   # rrnco_beam_select
 MIN_STARTS_TILED = 8   # RRNetDecoder.forward: starts per instance from which the any-N tile kernels serve every N
 
 _f = C.c_void_p  # every device pointer travels as void*
@@ -86,6 +88,9 @@ _SIGNATURES = {
                                       C.c_int32, _f, _f, _f, _f, _f]),
     "rrnco_select_action_filtered": (C.c_int, [C.c_int64, C.c_int32, _f, _f, C.c_int32, C.c_float, C.c_float, C.c_uint64,
                                                C.c_int32, _f, _f, _f, _f, C.c_int32, C.c_float, _f]),
+    "rrnco_beam_select": (C.c_int, [C.c_int64, C.c_int32, C.c_int32, _f, _f, _f, C.c_float, C.c_float, _f, _f, _f, _f, _f,
+                                    _f]),
+    "rrnco_beam_backtrack": (C.c_int, [C.c_int64, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_pointer_ffn_workspace_bytes": (C.c_int64, []),
     "rrnco_pointer_ffn": (C.c_int, [C.c_int64, _f, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_rollout_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int64, C.c_int32]),
@@ -188,3 +193,5 @@ def raise_device_status(word: int):
         raise AssertionError("infeasible action selected")  # rrnco/models/decoding.py:278-280
     if word & DEV_NO_FEASIBLE:
         raise AssertionError("no feasible action (fully masked row)")
+    if word & DEV_BAD_PARENT:
+        raise AssertionError("beam backtrack: a parent row outside the beam rows (corrupted beam records)")

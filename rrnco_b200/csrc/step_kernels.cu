@@ -470,6 +470,188 @@ __global__ void __launch_bounds__(kStepWarps * 32) select_action_kernel(int64_t 
   }
 }
 
+// rl4co BeamSearch._make_beam_step for one instance b per CTA: the W beam rows r = w * n_inst + b, candidate (w, n) of value
+// score[r] + lp[r, n] and flat index w * N + n.  The W largest candidates are found with a 4-pass 8-bit radix select on the
+// order-preserving key of filter_key (every pass recomputes the candidates from the L1/L2-resident logits: nothing of size
+// W x N is stored), ranked by (value desc, flat index asc), and ranks from #finite upward copy rank 0 (_fill_up_beams).
+// lp is select_action_kernel's per-row math (same operations, same order), so both give the same log-probs bit for bit.
+constexpr int kBeamThreads = 512;
+__global__ void __launch_bounds__(kBeamThreads) beam_select_kernel(int64_t n_inst, int W, int N, const float* __restrict__ logits,
+                                                                   const uint8_t* __restrict__ mask, const float* score_in,
+                                                                   float tanh_clip, float temperature,
+                                                                   int64_t* __restrict__ action_out,
+                                                                   int64_t* __restrict__ parent_out,
+                                                                   float* __restrict__ logp_out, float* score_out,
+                                                                   uint32_t* status) {
+  extern __shared__ float bsm[];
+  float* rmx = bsm;                                          // [W] row max of the processed logits
+  float* rse = rmx + W;                                      // [W] row log-sum-exp
+  float* rsc = rse + W;                                      // [W] beam scores (read before any is written: may alias)
+  uint32_t* ckey = reinterpret_cast<uint32_t*>(rsc + W);     // [W] selected keys, unordered
+  int* cidx = reinterpret_cast<int*>(ckey + W);              // [W] their flat indices
+  int* sidx = cidx + W;                                      // [W] flat index of rank w
+  float* sval = reinterpret_cast<float*>(sidx + W);          // [W] value of rank w
+  __shared__ int hist[256];
+  __shared__ int wsum[kBeamThreads / 32];
+  __shared__ int s_digit, s_need, s_gt, s_eq;
+  const int64_t b = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+  const int M = W * N;
+  auto clipped = [&](const float* lrow, int n) -> float {
+    float l = lrow[n];
+    if (tanh_clip > 0.f) l = __fmul_rn(1.0f - __fdividef(2.0f, __expf(2.0f * l) + 1.0f), tanh_clip);
+    return __fdiv_rn(l, temperature);
+  };
+  for (int w = warp; w < W; w += nw) {
+    const int64_t r = (int64_t)w * n_inst + b;
+    const float* lrow = logits + r * (int64_t)N;
+    const uint8_t* mrow = mask + r * (int64_t)N;
+    float mx = -INFINITY;
+    for (int n = lane; n < N; n += 32) mx = fmaxf(mx, mrow[n] ? clipped(lrow, n) : -INFINITY);
+    mx = warp_max(mx);
+    float se = 0.f;
+    for (int n = lane; n < N; n += 32) se += sfexp((mrow[n] ? clipped(lrow, n) : -INFINITY) - mx);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
+    if (lane == 0) {
+      rmx[w] = mx;
+      rse[w] = __logf(se);
+      rsc[w] = score_in[r];
+    }
+  }
+  __syncthreads();
+  // log-prob of node n in beam w's row (-inf when masked) and the candidate value score + lp
+  auto logp = [&](int w, int n) -> float {
+    const int64_t r = (int64_t)w * n_inst + b;
+    if (!mask[r * (int64_t)N + n]) return -INFINITY;
+    return __fsub_rn(__fsub_rn(clipped(logits + r * (int64_t)N, n), rmx[w]), rse[w]);
+  };
+  auto cand_key = [&](int f) -> uint32_t {
+    const int w = f / N;
+    return filter_key(__fadd_rn(rsc[w], logp(w, f - w * N)));
+  };
+  // radix select: K = the W-th largest key; `need` = how many candidates of key K rank among the W
+  uint32_t prefix = 0u, pmask = 0u;
+  int need = W;
+#pragma unroll 1
+  for (int shift = 24; shift >= 0; shift -= 8) {
+    for (int i = tid; i < 256; i += blockDim.x) hist[i] = 0;
+    __syncthreads();
+    for (int f = tid; f < M; f += blockDim.x) {
+      const uint32_t k = cand_key(f);
+      if ((k & pmask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1);
+    }
+    __syncthreads();
+    if (tid == 0) {
+      int acc = 0, d = 255;
+      for (; d > 0; --d) {
+        if (acc + hist[d] >= need) break;
+        acc += hist[d];
+      }
+      s_digit = d;
+      s_need = need - acc;
+    }
+    __syncthreads();
+    prefix |= (uint32_t)s_digit << shift;
+    pmask |= 255u << shift;
+    need = s_need;
+  }
+  const uint32_t K = prefix;
+  const int n_gt = W - need;
+  // collect: every key > K, and the `need` lowest flat indices of key K (block-wide prefix count, in flat order)
+  if (tid == 0) { s_gt = 0; s_eq = 0; }
+  __syncthreads();
+  for (int f0 = 0; f0 < M; f0 += blockDim.x) {
+    const int f = f0 + tid;
+    const uint32_t k = f < M ? cand_key(f) : 0u;
+    const bool eq = f < M && k == K, gt = f < M && k > K;
+    if (gt) {
+      const int slot = atomicAdd(&s_gt, 1);
+      ckey[slot] = k;
+      cidx[slot] = f;
+    }
+    const unsigned bal = __ballot_sync(0xffffffffu, eq);
+    if (lane == 0) wsum[warp] = __popc(bal);
+    __syncthreads();
+    int off = s_eq;
+    for (int i = 0; i < warp; ++i) off += wsum[i];
+    const int rank = off + __popc(bal & ((1u << lane) - 1u));
+    if (eq && rank < need) {
+      ckey[n_gt + rank] = k;
+      cidx[n_gt + rank] = f;
+    }
+    __syncthreads();
+    if (tid == 0) {
+      int t = 0;
+      for (int i = 0; i < nw; ++i) t += wsum[i];
+      s_eq += t;
+    }
+    __syncthreads();
+  }
+  // order the W selected by (value desc, flat index asc); count the finite ones
+  int fin = 0;
+  for (int i = tid; i < W; i += blockDim.x) {
+    const uint32_t ki = ckey[i];
+    const int fi = cidx[i];
+    int rk = 0;
+    for (int j = 0; j < W; ++j) rk += (ckey[j] > ki || (ckey[j] == ki && cidx[j] < fi)) ? 1 : 0;
+    sidx[rk] = fi;
+    fin += ki > filter_key(-INFINITY) ? 1 : 0;
+  }
+  if (tid == 0) s_gt = 0;
+  __syncthreads();
+  if (fin) atomicAdd(&s_gt, fin);
+  __syncthreads();
+  const int finite = s_gt;
+  for (int w = tid; w < W; w += blockDim.x) {
+    const int f = sidx[w < finite ? w : 0];
+    const int pw = f / N, n = f - pw * N;
+    const float lp = logp(pw, n);
+    sval[w] = __fadd_rn(rsc[pw], lp);
+    const int64_t r = (int64_t)w * n_inst + b;
+    action_out[r] = n;
+    parent_out[r] = (int64_t)pw * n_inst + b;
+    logp_out[r] = lp;
+  }
+  __syncthreads();  // every parent score has been read: score_out may alias score_in
+  for (int w = tid; w < W; w += blockDim.x) score_out[(int64_t)w * n_inst + b] = sval[w];
+  if (tid == 0 && finite == 0) atomicOr(status, RRNCO_DEV_NO_FEASIBLE);
+}
+
+// BeamSearch._backtrack: row r of the output is the path of the final beam r, followed back through the parent rows.
+// Step-major inputs [T, R] (row t = what step t wrote; the parents of step 0 are never read); outputs [R, T], log-likelihood =
+// fp64 sum of the aligned log-probs.  A parent row outside [0, R) sets RRNCO_DEV_BAD_PARENT; that row's earlier steps are
+// written as action 0 with log-prob NaN, and its log-likelihood is NaN.
+__global__ void beam_backtrack_kernel(int64_t R, int T, const int64_t* __restrict__ actions,
+                                      const int64_t* __restrict__ parents, const float* __restrict__ logprobs,
+                                      int64_t* __restrict__ actions_out, float* __restrict__ logprob_out,
+                                      float* __restrict__ loglik_out, uint32_t* status) {
+  const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= R) return;
+  int64_t cur = r;
+  double s = 0.0;
+  int t = T - 1;
+  for (; t >= 0; --t) {
+    const int64_t i = (int64_t)t * R + cur;
+    const float lp = logprobs[i];
+    actions_out[r * T + t] = actions[i];
+    if (logprob_out) logprob_out[r * T + t] = lp;
+    s += (double)lp;
+    if (t == 0) break;
+    cur = parents[i];
+    if (cur < 0 || cur >= R) {
+      atomicOr(status, RRNCO_DEV_BAD_PARENT);
+      s = NAN;
+      break;
+    }
+  }
+  for (--t; t >= 0; --t) {  // only after a bad parent
+    actions_out[r * T + t] = 0;
+    if (logprob_out) logprob_out[r * T + t] = NAN;
+  }
+  loglik_out[r] = (float)s;
+}
+
 }  // namespace rrnco
 
 using namespace rrnco;
@@ -590,6 +772,33 @@ int rrnco_select_action_filtered(int64_t n_rollouts, int32_t n_nodes, const floa
   kern<<<grid, kStepWarps * 32, 0, (cudaStream_t)stream>>>(n_rollouts, n_nodes, logits, mask, decode_mode, tanh_clipping,
                                                            temperature, seed, step, forced_action, action_out, logprob_out,
                                                            status, top_k, top_p);
+  return rrnco_launch_status();
+}
+
+int rrnco_beam_select(int64_t n_inst, int32_t beam_width, int32_t n_nodes, const float* logits, const uint8_t* mask,
+                      const float* score_in, float tanh_clipping, float temperature, int64_t* action_out, int64_t* parent_out,
+                      float* logprob_out, float* score_out, uint32_t* status, void* stream) {
+  RRNCO_CHECK_ARG(beam_width >= 2);
+  if (beam_width > RRNCO_MAX_BEAM_WIDTH) return RRNCO_ERR_UNSUPPORTED;
+  if (n_inst == 0) return RRNCO_OK;
+  RRNCO_CHECK_ARG(n_inst > 0 && n_inst <= INT32_MAX && n_nodes > 0 && (int64_t)beam_width * n_nodes <= INT32_MAX);
+  RRNCO_CHECK_ARG(logits && mask && score_in && action_out && parent_out && logprob_out && score_out && status);
+  RRNCO_CHECK_ARG(temperature > 0.f);
+  const size_t smem = (size_t)7 * beam_width * sizeof(float);  // <= 28 KB: no opt-in needed
+  beam_select_kernel<<<(unsigned)n_inst, kBeamThreads, smem, (cudaStream_t)stream>>>(
+      n_inst, beam_width, n_nodes, logits, mask, score_in, tanh_clipping, temperature, action_out, parent_out, logprob_out,
+      score_out, status);
+  return rrnco_launch_status();
+}
+
+int rrnco_beam_backtrack(int64_t n_rows, int32_t n_steps, const int64_t* actions, const int64_t* parents,
+                         const float* logprobs, int64_t* actions_out, float* logprob_out, float* loglik_out,
+                         uint32_t* status, void* stream) {
+  if (n_rows == 0) return RRNCO_OK;
+  RRNCO_CHECK_ARG(n_rows > 0 && n_steps > 0 && actions && parents && logprobs && actions_out && loglik_out && status);
+  const unsigned grid = (unsigned)((n_rows + 127) / 128);
+  beam_backtrack_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(n_rows, n_steps, actions, parents, logprobs, actions_out,
+                                                                 logprob_out, loglik_out, status);
   return rrnco_launch_status();
 }
 

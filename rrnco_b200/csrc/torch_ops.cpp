@@ -12,6 +12,7 @@
 //   tour_reward                        env._get_reward                   rrnco/envs/*/env.py
 //   select_action                      DecodingStrategy.step             rrnco/models/decoding.py:219-298
 //   rollout                            RRNetPolicy.forward decode loop   rrnco/models/policy.py:203-243
+//   beam_select / beam_backtrack       BeamSearch step / _backtrack      rrnco/models/decoding.py:402-542
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
@@ -154,6 +155,45 @@ std::tuple<Tensor, Tensor> select_action(const Tensor& logits, const Tensor& mas
   return {action, logp};
 }
 
+// -> (action, parent row, log-prob, new score), rows in (w b) order; `status` (int32 [1]) is OR-ed in place
+std::tuple<Tensor, Tensor, Tensor, Tensor> beam_select(const Tensor& logits, const Tensor& mask, const Tensor& score,
+                                                       int64_t beam_width, double tanh_clipping, double temperature,
+                                                       Tensor status) {
+  TORCH_CHECK(logits.is_cuda() && logits.dim() == 2, "logits [R,N] on CUDA expected");
+  TORCH_CHECK(beam_width >= 2 && logits.size(0) % beam_width == 0, "beam_select: beam_width >= 2 dividing the rows expected");
+  c10::cuda::CUDAGuard guard(logits.device());
+  Tensor lg = f32c(logits), m = u8c(mask), sc = f32c(score);
+  const int64_t R = lg.size(0), N = lg.size(1);
+  TORCH_CHECK(sc.numel() == R, "beam_select: one score per row expected");
+  auto lopt = lg.options().dtype(at::kLong);
+  Tensor action = at::empty({R}, lopt), parent = at::empty({R}, lopt), logp = at::empty({R}, lg.options()),
+         out = at::empty({R}, lg.options());
+  check_rc(rrnco_beam_select(R / beam_width, (int32_t)beam_width, (int32_t)N, lg.data_ptr<float>(), m.data_ptr<uint8_t>(),
+                             sc.data_ptr<float>(), (float)tanh_clipping, (float)temperature, action.data_ptr<int64_t>(),
+                             parent.data_ptr<int64_t>(), logp.data_ptr<float>(), out.data_ptr<float>(),
+                             reinterpret_cast<uint32_t*>(status.data_ptr<int32_t>()), stream_of(lg)), "beam_select");
+  return {action, parent, logp, out};
+}
+
+// step-major [T, R] actions / parents / log-probs -> (actions [R, T], log-probs [R, T] | empty, log-likelihood [R]);
+// `status` (int32 [1]) is OR-ed in place
+std::tuple<Tensor, Tensor, Tensor> beam_backtrack(const Tensor& actions, const Tensor& parents, const Tensor& logprobs,
+                                                  bool per_step_logprobs, Tensor status) {
+  TORCH_CHECK(actions.is_cuda() && actions.dim() == 2 && parents.sizes() == actions.sizes() &&
+              logprobs.sizes() == actions.sizes(), "actions / parents / logprobs [T,R] on CUDA expected");
+  c10::cuda::CUDAGuard guard(actions.device());
+  Tensor a = actions.to(at::kLong).contiguous(), p = parents.to(at::kLong).contiguous(), l = f32c(logprobs);
+  const int64_t T = a.size(0), R = a.size(1);
+  Tensor a_out = at::empty({R, T}, a.options());
+  Tensor l_out = at::empty({per_step_logprobs ? R : 0, per_step_logprobs ? T : 0}, l.options());
+  Tensor ll = at::empty({R}, l.options());
+  check_rc(rrnco_beam_backtrack(R, (int32_t)T, a.data_ptr<int64_t>(), p.data_ptr<int64_t>(), l.data_ptr<float>(),
+                                a_out.data_ptr<int64_t>(), per_step_logprobs ? l_out.data_ptr<float>() : nullptr,
+                                ll.data_ptr<float>(), reinterpret_cast<uint32_t*>(status.data_ptr<int32_t>()), stream_of(a)),
+           "beam_backtrack");
+  return {a_out, l_out, ll};
+}
+
 // weights: [ffn_w1, ffn_b1, ffn_w2, ffn_b2, ctx_state_w?, ctx_placeholder_q?]
 // cache  : [glimpse_key, glimpse_val, logit_key, ctx_node_proj, ctx_node_proj2?]
 // data   : [distance, duration?, demand?, demand_backhaul?, time_windows?, service_time?, vehicle_capacity?, distance_limit?,
@@ -235,6 +275,10 @@ TORCH_LIBRARY(rrnco_b200, m) {
         "float tanh_clipping, float temperature, Tensor?[] cache, Tensor?[] data, Tensor? forced_actions, int t_cap, "
         "bool per_step_logprobs, Tensor(a!) workspace, int top_k=0, float top_p=0.0) -> "
         "(Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor)");
+  m.def("beam_select(Tensor logits, Tensor mask, Tensor score, int beam_width, float tanh_clipping, float temperature, "
+        "Tensor(a!) status) -> (Tensor, Tensor, Tensor, Tensor)");
+  m.def("beam_backtrack(Tensor actions, Tensor parents, Tensor logprobs, bool per_step_logprobs, Tensor(a!) status) -> "
+        "(Tensor, Tensor, Tensor)");
   m.def("rollout_workspace_bytes(int env, int n_nodes, int n_inst, int n_starts) -> int", &rollout_workspace_bytes);
 }
 
@@ -246,4 +290,6 @@ TORCH_LIBRARY_IMPL(rrnco_b200, CUDA, m) {
   m.impl("tour_reward", &tour_reward);
   m.impl("select_action", &select_action);
   m.impl("rollout", &rollout);
+  m.impl("beam_select", &beam_select);
+  m.impl("beam_backtrack", &beam_backtrack);
 }

@@ -8,8 +8,12 @@ decoder and the whole decode loop running as fused sm_100a kernels (librrnco_b20
 
 The logit filters `top_k` / `top_p` of rl4co's `process_logits` run inside the decode kernels (any decode type), except
 under grad in phase "train" without forced actions: the differentiable replay does not filter, so that call raises.
-Unsupported reference options raise NotImplementedError (beam search, select_best, store_all_logp / return_entropy,
-mask_logits=False, dynamic embeddings): they are not on any BASELINE config.
+`decode_type="beam_search"` (rl4co BeamSearch; `beam_width=`, `select_best=` which defaults to True there) runs the
+per-step kernel pipeline for any N: rrnco_beam_select picks the beams, rrnco_beam_backtrack aligns the sequences.  It
+raises NotImplementedError together with top_k / top_p, with `actions=`, and under grad in phase "train".
+`select_best=True` on a multistart greedy / sampling decode keeps each instance's best start (first maximum of the reward).
+Unsupported reference options raise NotImplementedError (store_all_logp / return_entropy, mask_logits=False, dynamic
+embeddings): they are not on any BASELINE config.
 """
 from __future__ import annotations
 
@@ -298,14 +302,50 @@ class RRNetPolicy(nn.Module):
         if filtered and phase == "train" and torch.is_grad_enabled() and actions is None:
             raise NotImplementedError("top_k / top_p under grad in phase 'train': the differentiable replay of the sampled "
                                       "actions (training.batched_logprobs) does not filter")
-        if decoding_kwargs.get("select_best"):
-            raise NotImplementedError("select_best")
+        decode_type = decoding_kwargs.pop("decode_type", None)
+        beam = decode_type == "beam_search" or (decode_type is None and actions is None
+                                                and getattr(self, f"{phase}_decode_type") == "beam_search")
+        select_best = decoding_kwargs.pop("select_best", None)
+        select_best = beam if select_best is None else bool(select_best)  # BeamSearch defaults to True, the others to False
+        beam_width = decoding_kwargs.pop("beam_width", None)
+        if beam:
+            if actions is not None:
+                raise NotImplementedError("actions= with decode_type 'beam_search': evaluate given actions with the "
+                                          "default decode type")
+            if filtered:
+                raise NotImplementedError("top_k / top_p with decode_type 'beam_search'")
+            if phase == "train" and torch.is_grad_enabled():
+                raise NotImplementedError("beam search under grad in phase 'train': the differentiable replay of the "
+                                          "actions (training.batched_logprobs) does not beam")
+            if beam_width is not None:
+                beam_width = beam_args(beam_width)
         if td.device.type != "cuda":
             td = td.to(env.device)
+        if beam and beam_width is None:
+            beam_width = beam_args(env.get_num_starts(td))  # BeamSearch.pre_decoder_hook
 
         row_emb, col_emb = self.encoder(td, phase=phase)  # policy.py:176
 
-        decode_type = decoding_kwargs.pop("decode_type", None)
+        if beam:
+            cache = self.decoder._precompute_cache((row_emb, col_emb), num_starts=beam_width)
+            self._calls += 1
+            out = beam_search_rollout(self.decoder, cache, env, td, beam_width,
+                                      temperature=decoding_kwargs.pop("temperature", self.temperature),
+                                      tanh_clipping=decoding_kwargs.pop("tanh_clipping", self.tanh_clipping),
+                                      calc_reward=calc_reward or select_best,
+                                      per_step_logprobs=not return_sum_log_likelihood, check=self.decoder.check_nan)
+            outdict = {"reward": out["reward"],
+                       "log_likelihood": out["log_likelihood"] if return_sum_log_likelihood else out["logprobs"]}
+            if "normalized_reward" in out:
+                outdict["normalized_reward"] = out["normalized_reward"]
+            if return_actions:
+                outdict["actions"] = out["actions"]
+            if select_best:
+                outdict = select_best_rows(outdict, beam_width)
+            if return_hidden:
+                outdict["hidden"] = cache
+            return outdict
+
         if actions is not None:
             decode_type = "evaluate"
         elif decode_type is None:
@@ -319,6 +359,7 @@ class RRNetPolicy(nn.Module):
         if multistart and num_starts is None:
             num_starts = env.get_num_starts(td)  # decoding.py:162-163
         S = num_starts if multistart else 1
+        calc_reward = calc_reward or (select_best and S > 1)  # rl4co's _select_best computes the rewards it ranks by
         temperature = decoding_kwargs.pop("temperature", self.temperature)
         tanh_clipping = decoding_kwargs.pop("tanh_clipping", self.tanh_clipping)
 
@@ -362,6 +403,8 @@ class RRNetPolicy(nn.Module):
             outdict["normalized_reward"] = out["normalized_reward"]
         if return_actions:
             outdict["actions"] = out["actions"]
+        if select_best and S > 1:
+            outdict = select_best_rows(outdict, S)
         if return_hidden:
             outdict["hidden"] = cache
         return outdict
@@ -386,6 +429,26 @@ def filter_args(top_k=None, top_p=None) -> Tuple[int, float]:
 def filter_active(top_k: int, top_p: float) -> bool:
     """True when the filters can drop an entry (top_k > 0, or 0 < top_p < 1)."""
     return top_k > 0 or 0.0 < top_p < 1.0
+
+
+def beam_args(beam_width) -> int:
+    """rl4co's `beam_width` as an int; ValueError below 2 (BeamSearch asserts beam_width > 1), NotImplementedError above
+    what rrnco_beam_select serves; both before anything is launched."""
+    if isinstance(beam_width, bool) or int(beam_width) != beam_width or beam_width < 2:
+        raise ValueError(f"beam width must be an integer >= 2 (got {beam_width!r})")
+    if beam_width > _lib.MAX_BEAM_WIDTH:
+        raise NotImplementedError(f"beam width above {_lib.MAX_BEAM_WIDTH} (got {beam_width})")
+    return int(beam_width)
+
+
+def select_best_rows(outdict: dict, num_starts: int) -> dict:
+    """rl4co's _select_best on the [num_starts * B] outputs in (s b) order: per instance the row of highest reward, the
+    lowest s among equal rewards; every [num_starts * B]-leading tensor of `outdict` is cut to those B rows."""
+    reward = outdict["reward"]
+    R = reward.shape[0]
+    B = R // num_starts
+    rows = reward.view(num_starts, B).argmax(0) * B + torch.arange(B, device=reward.device)
+    return {k: (v[rows] if isinstance(v, Tensor) and v.dim() >= 1 and v.shape[0] == R else v) for k, v in outdict.items()}
 
 
 class SoftmaxRangeError(RuntimeError):
@@ -575,6 +638,116 @@ def stepwise_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, nu
     acts = torch.stack(actions, 1)
     lps = torch.stack(logps, 1)
     out = {"actions": acts, "log_likelihood": lps.double().sum(1).float(), "logprobs": lps}
+    has_minmax = "min_distance" in td.keys()
+    if calc_reward:
+        open_route = td["open_route"] if name == "rcvrptw" else None
+        real, norm = tour_reward(acts, td["distance_matrix"], name != "atsp", open_route,
+                                 td["min_distance"] if has_minmax and env.normalize else None,
+                                 td["max_distance"] if has_minmax and env.normalize else None)
+        if env.normalize and has_minmax:
+            out["reward"], out["normalized_reward"] = real, norm
+        else:
+            out["reward"] = norm
+    else:
+        out["reward"] = torch.zeros(R, dtype=torch.float32 if name == "rcvrptw" else torch.bool, device=dev)
+    return out
+
+
+def beam_select(logits, mask, score, beam_width: int, tanh_clipping: float = 10.0, temperature: float = 1.0, status=None):
+    """One BeamSearch step (rl4co decoding.py:402-542, _make_beam_step) over the [W * B, N] decoder output in (w b) order:
+    (action int64, parent row int64, log-prob fp32, new score fp32), each [W * B].  Candidates are ranked by (value
+    descending, flat index w * N + n ascending); include/rrnco_b200.h (rrnco_beam_select) gives the full rule."""
+    W = beam_args(beam_width)
+    if status is None:
+        status = torch.zeros(1, dtype=torch.int32, device=logits.device)
+    from . import torch_ops
+    if torch_ops.enabled():
+        _lib.count_call("rrnco_beam_select")
+        action, parent, logp, new_score = torch_ops.ops().beam_select(logits, mask, score, W, float(tanh_clipping),
+                                                                      float(temperature), status)
+        return action, parent, logp, new_score, status
+    logits, mask, score = logits.float().contiguous(), mask.contiguous(), score.float().contiguous()
+    R, N = logits.shape
+    if R % W:
+        raise ValueError(f"{R} rows are not a whole number of beams of width {W}")
+    action = torch.empty(R, dtype=torch.int64, device=logits.device)
+    parent = torch.empty(R, dtype=torch.int64, device=logits.device)
+    logp = torch.empty(R, dtype=torch.float32, device=logits.device)
+    new_score = torch.empty(R, dtype=torch.float32, device=logits.device)
+    call("rrnco_beam_select", R // W, W, N, ptr(logits), ptr(_u8(mask)), ptr(score), float(tanh_clipping),
+         float(temperature), ptr(action), ptr(parent), ptr(logp), ptr(new_score), ptr(status), stream_ptr(logits.device))
+    return action, parent, logp, new_score, status
+
+
+def beam_backtrack(actions, parents, logprobs, per_step_logprobs: bool = True, status=None):
+    """BeamSearch._backtrack: step-major [T, R] actions / parent rows / log-probs -> (actions [R, T], aligned log-probs
+    [R, T] or None, log-likelihood [R], status).  A parent row outside [0, R) sets DEV_BAD_PARENT in `status`."""
+    if status is None:
+        status = torch.zeros(1, dtype=torch.int32, device=actions.device)
+    from . import torch_ops
+    if torch_ops.enabled():
+        _lib.count_call("rrnco_beam_backtrack")
+        a, lp, ll = torch_ops.ops().beam_backtrack(actions, parents, logprobs, bool(per_step_logprobs), status)
+        return a, (lp if per_step_logprobs else None), ll, status
+    actions, parents, logprobs = actions.contiguous(), parents.contiguous(), logprobs.float().contiguous()
+    T, R = actions.shape
+    dev = actions.device
+    a = torch.empty((R, T), dtype=torch.int64, device=dev)
+    lp = torch.empty((R, T), dtype=torch.float32, device=dev) if per_step_logprobs else None
+    ll = torch.empty(R, dtype=torch.float32, device=dev)
+    call("rrnco_beam_backtrack", R, T, ptr(actions), ptr(parents), ptr(logprobs), ptr(a), ptr(lp), ptr(ll), ptr(status),
+         stream_ptr(dev))
+    return a, lp, ll, status
+
+
+def beam_search_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, beam_width: int,
+                        temperature: float = 1.0, tanh_clipping: float = 10.0, calc_reward: bool = True,
+                        per_step_logprobs: bool = False, check: bool = True) -> dict:
+    """rl4co BeamSearch (decoding.py:402-542) as a per-step kernel pipeline for any N: decoder_logits -> beam_select ->
+    the rollout state of each new beam gathered from its parent row -> env step, then beam_backtrack.  Rows r = w * B + b;
+    the start nodes are env.select_start_nodes(td, W) with log-prob 0.  Only the rollout state is replicated over the
+    beams (what stepwise_rollout replicates), never the instance matrices.  Returns the [W * B] outputs of every beam."""
+    W = beam_args(beam_width)
+    from .tdlite import TensorDictLite, batchify
+    from .envs import tour_reward
+    name = decoder.env_name
+    n_inst, N, _ = cache.glimpse_key.shape
+    R = n_inst * W
+    dev = cache.glimpse_key.device
+    state_keys = _ROLLOUT_STATE_KEYS[name]
+    roll = {k: (batchify(td[k], W) if k in state_keys else td[k]) for k in td.keys() if k != "done"}
+    roll = TensorDictLite(roll, batch_size=[R])
+    a0 = env.select_start_nodes(td, W)
+    roll.set("action", a0)
+    roll = env.step(roll)["next"]
+    actions, parents, logps = [a0], [torch.zeros(R, dtype=torch.int64, device=dev)], [torch.zeros(R, device=dev)]
+    score = torch.zeros(R, dtype=torch.float32, device=dev)
+    done = roll["done"]
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    max_steps = 2 * N + 2
+    while len(actions) <= max_steps:
+        if name == "atsp":  # fixed length: no host sync needed
+            if len(actions) >= N:
+                break
+        elif bool(done.all()):
+            break
+        logits, mask = decoder(roll, cache, W)
+        a, parent, lp, score, status = beam_select(logits, mask, score, W, tanh_clipping, temperature, status)
+        for k in state_keys:  # each new beam continues from its parent's state
+            roll[k] = roll[k].index_select(0, parent)
+        roll.set("action", a)
+        roll = env.step(roll)["next"]
+        done = roll["done"]
+        actions.append(a)
+        parents.append(parent)
+        logps.append(lp)
+    acts, lps, ll, status = beam_backtrack(torch.stack(actions), torch.stack(parents), torch.stack(logps),
+                                           per_step_logprobs, status)
+    if check:
+        _lib.raise_device_status(int(status.item()))
+    out = {"actions": acts, "log_likelihood": ll}
+    if per_step_logprobs:
+        out["logprobs"] = lps
     has_minmax = "min_distance" in td.keys()
     if calc_reward:
         open_route = td["open_route"] if name == "rcvrptw" else None
