@@ -177,7 +177,8 @@ def set_step_tiling(mode):
 
 
 def set_ffn_engine(engine: int):
-    """1 = tcgen05 FFN (default), 0 = mma.sync FFN in the fused rollout kernel."""
+    """Engine of the fused rollout kernel: 2 = lean kernel for N <= 112, else the one-CTA tcgen05 kernel (default), 1 = one-CTA
+    tcgen05 kernel, 0 = mma.sync FFN."""
     check(lib().rrnco_set_ffn_engine(engine))
 
 

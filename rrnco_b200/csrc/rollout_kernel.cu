@@ -1925,7 +1925,8 @@ int rrnco_set_precision(int32_t passes) {
   return RRNCO_OK;
 }
 
-// FFN engine of the fused rollout kernel: 1 = tcgen05.mma + TMEM + TMA weight stream (default), 0 = mma.sync
+// Engine of the fused rollout kernel: 2 = the lean kernel (two CTAs per SM) for N <= 112, else 1 (default); 1 = one CTA
+// per SM, tcgen05.mma + TMEM + TMA weight stream; 0 = the mma.sync FFN
 int rrnco_set_ffn_engine(int32_t engine) {
   if (engine < 0 || engine > 2) return RRNCO_ERR_BAD_ARG;
   g_engine = engine;

@@ -986,7 +986,8 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
 #ifndef RRNCO_LEAN_SELECT3
     // ---- S: select, thread per row, SINGLE pass: two threads own one rollout, 16-column groups dealt round-robin.  Per
     // element: u = 2^(acc k1 - bias log2 e) + 1e-6 (decoder.py:198-201), v = clip (1 - 2 / (u^2 + 1)) (= clip tanh(log u)),
-    // mask; sum of exp(v - shift) with the fixed shift clip / temperature (clipped values are bounded: no maximum pass);
+    // mask; sum of exp(v - shift) with the fixed shift clip / temperature while that bound is within kMaxFixedShift (no
+    // maximum pass), else (low temperatures, large or no clipping) against a running maximum;
     // arg-max by a tree maximum per block + an index search only when the block improves it.  log p(chosen) =
     // (v - max) - log sum.  Greedy = arg-max v (lowest index on ties), sampling = arg-max v + Gumbel, evaluate = the forced
     // column.  (The three-pass form -- values rewritten to TMEM, sum pass, log-softmax pass -- is kept behind
@@ -1011,7 +1012,9 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
         forced = min(max(forced, 0), N - 1);
       }
       const uint2 key2 = make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32));
-      float m = clip > 0.f ? __fdiv_rn(clip, temperature) : -INFINITY;
+      const float mfix = clip > 0.f ? __fdiv_rn(clip, temperature) : INFINITY;
+      const bool fixed_shift = mfix <= kMaxFixedShift;
+      float m = fixed_shift ? mfix : -INFINITY;
       float ssum = 0.f, best = -INFINITY, bestv = -INFINITY, chk = 0.f;
       int besti = 255;
       float cut = -INFINITY;
@@ -1089,7 +1092,7 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
         }
         float bm = fmaxf(fmaxf(fmaxf(val[0], val[1]), fmaxf(val[2], val[3])), fmaxf(fmaxf(val[4], val[5]), fmaxf(val[6], val[7])));
         bm = fmaxf(bm, fmaxf(fmaxf(fmaxf(val[8], val[9]), fmaxf(val[10], val[11])), fmaxf(fmaxf(val[12], val[13]), fmaxf(val[14], val[15]))));
-        if (clip <= 0.f && bm > m) {  // unclipped logits: running maximum
+        if (!fixed_shift && bm > m) {  // running maximum
           ssum *= fexp(m - bm);
           m = bm;
         }

@@ -1136,8 +1136,11 @@ __global__ void __launch_bounds__(kGThreads, 1) rollout_tiled_kernel(const Rollo
       const uint2 key2 = make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32));
       const float k1 = inv_sqrt_e * 1.4426950408889634f;  // raw accumulator -> logit in log2 units
       const float alpha2 = p.w.alpha * 1.4426950408889634f, beta2 = p.w.beta * 1.4426950408889634f;
-      // with clipping every value is <= clip / temperature: a fixed shift for the sum of exp (no running maximum)
-      float m = clip > 0.f ? __fdiv_rn(clip, temperature) : -INFINITY;
+      // with clipping every value is <= clip / temperature: a fixed shift for the sum of exp (no running maximum) while
+      // that bound is within kMaxFixedShift
+      const float mfix = clip > 0.f ? __fdiv_rn(clip, temperature) : INFINITY;
+      const bool fixed_shift = mfix <= kMaxFixedShift;
+      float m = fixed_shift ? mfix : -INFINITY;
       float ssum = 0.f, best = -INFINITY, bestv = -INFINITY, chk = 0.f;
       int besti = 0x7fffffff;
       // Bias rows alpha . D[cur, :]: a thread-per-row read from global memory is one L1 wavefront per ELEMENT (32 lanes, 32
@@ -1257,9 +1260,9 @@ __global__ void __launch_bounds__(kGThreads, 1) rollout_tiled_kernel(const Rollo
             }
             float bm = fmaxf(fmaxf(fmaxf(val[0], val[1]), fmaxf(val[2], val[3])), fmaxf(fmaxf(val[4], val[5]), fmaxf(val[6], val[7])));
             bm = fmaxf(bm, fmaxf(fmaxf(fmaxf(val[8], val[9]), fmaxf(val[10], val[11])), fmaxf(fmaxf(val[12], val[13]), fmaxf(val[14], val[15]))));
-            // sum of exp against a shift (masked columns contribute exp(-inf) = 0): with clipping the values are bounded
-            // by clip / temperature, a fixed shift; otherwise the running maximum
-            if (clip <= 0.f && bm > m) {
+            // sum of exp against a shift (masked columns contribute exp(-inf) = 0): the fixed bound clip / temperature
+            // (kMaxFixedShift), otherwise the running maximum
+            if (!fixed_shift && bm > m) {
               ssum *= fexp(m - bm);  // m = -inf: 0 (ssum is 0 then anyway)
               m = bm;
             }
@@ -1316,7 +1319,8 @@ __global__ void __launch_bounds__(kGThreads, 1) rollout_tiled_kernel(const Rollo
         // this CTA's partial over its key tiles: the two groups merged (larger key wins, ties -> lower index)
         float m0 = sm.xf[0][0][row], m1 = sm.xf[0][1][row];
         float mx = fmaxf(m0, m1);
-        float tot = sm.xf[1][0][row] * fexp(m0 - mx) + sm.xf[1][1][row] * fexp(m1 - mx);
+        // (under a running maximum a group whose key tiles are all masked for this row has m = -inf, s = 0)
+        float tot = rescaled_sum(sm.xf[1][0][row], m0, mx) + rescaled_sum(sm.xf[1][1][row], m1, mx);
         int win = 0;
         if (sm.xf[2][1][row] > sm.xf[2][0][row] || (sm.xf[2][1][row] == sm.xf[2][0][row] && sm.xi[1][row] < sm.xi[0][row])) win = 1;
         float bkey = sm.xf[2][win][row], bval = sm.xf[3][win][row];
@@ -1341,7 +1345,7 @@ __global__ void __launch_bounds__(kGThreads, 1) rollout_tiled_kernel(const Rollo
           const float va = rank ? vp : bval, vb2 = rank ? bval : vp;
           const int ia = rank ? ip : act, ib = rank ? act : ip;
           mx = fmaxf(ma, mb);
-          tot = sa * fexp(ma - mx) + sb * fexp(mb - mx);
+          tot = rescaled_sum(sa, ma, mx) + rescaled_sum(sb, mb, mx);
           const bool second = kb2 > ka || (kb2 == ka && ib < ia);
           bkey = second ? kb2 : ka;
           bval = p.mode == RRNCO_DECODE_EVALUATE ? fmaxf(va, vb2) : (second ? vb2 : va);

@@ -437,7 +437,7 @@ def test_ffn_engines_agree(rb, engine):
         test_greedy_rollout_vs_oracle(rb, "rcvrp", 50, 8)
         test_greedy_rollout_vs_oracle(rb, "rcvrptw", 20, 4)
     finally:
-        rb.set_ffn_engine(1)
+        rb.set_ffn_engine(2)  # the default: the lean kernel for N <= 112
 
 
 def test_pointer_ffn_tcgen05(rb):
