@@ -365,6 +365,35 @@ int rrnco_rollout_filtered(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t
                            void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Fused beam search: the whole BeamSearch decode (rl4co decoding.py:402-542) in one launch of the lean rollout kernel,
+ * one CTA per instance whose beam_width rows are the beams.  Same semantics as a loop of rrnco_beam_select steps:
+ *   Rows r = w * n_inst + b.  The beams start at select_start_nodes (start w % num_loc + has_depot, log-prob 0, score 0).
+ *   Each step computes every beam row's log-probs as rrnco_rollout does (tanh clipping, mask, temperature, log-softmax),
+ *   ranks the candidates score + lp (fp32) of an instance by (value descending, flat index w * n_nodes + n ascending),
+ *   keeps the beam_width largest (ranks from #finite upward copy rank 0; none finite sets RRNCO_DEV_NO_FEASIBLE), moves
+ *   each new beam's rollout state to its parent row and steps the env with its action.  Scores: score_t = score_{t-1} + lp_t.
+ *   An instance whose beams are all done keeps them: parent = the row itself, action 0, log-prob 0, as a further
+ *   rrnco_beam_select step on its depot-only masks would.
+ *   step_actions / step_parents int64, step_logprobs fp32: step-major [t_cap, R], the inputs of rrnco_beam_backtrack
+ *   (rows 0 .. *n_steps_out - 1 are written; step 0 holds the starts).  *n_steps_out (device int32) = the number of
+ *   steps of the longest instance, the T of the per-step loop.  t_cap: 2 * n_nodes + 3 for the VRPs, n_nodes for ATSP
+ *   (the per-step loop's bound); an instance still running at t_cap sets RRNCO_DEV_TRUNCATED.
+ *   workspace: >= rrnco_beam_rollout_workspace_bytes(...) bytes, 16-byte aligned, scratch only.
+ *   Built for the default engine and precision only (fp32-faithful operands: rrnco_set_ffn_engine(2),
+ *   rrnco_set_precision(3)).  beam_width < 2: RRNCO_ERR_BAD_ARG; beam_width > RRNCO_MAX_BEAM_WIDTH_FUSED,
+ *   n_nodes > 112, another engine or precision: RRNCO_ERR_UNSUPPORTED; all before any CUDA call (the per-step entry
+ *   points serve those calls).
+ * rrnco_beam_rollout_workspace_bytes: the workspace size, or 0 when rrnco_beam_rollout does not serve the call (the
+ *   same width, size, engine and precision rule): callers route on it.
+ * ---------------------------------------------------------------------------------------------- */
+#define RRNCO_MAX_BEAM_WIDTH_FUSED 128
+int64_t rrnco_beam_rollout_workspace_bytes(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t beam_width);
+int rrnco_beam_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t beam_width, const rrnco_decoder_weights_t* w,
+                       const rrnco_decoder_cache_t* cache, const rrnco_instance_data_t* data, int32_t t_cap,
+                       int64_t* step_actions, int64_t* step_parents, float* step_logprobs, int32_t* n_steps_out,
+                       uint32_t* status, void* workspace, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Encoder hot spot (SURVEY.md 8(f) rank 4): gating neural adaptive bias of an attention-free block, variant without the
  * duration channel -- DistAngleFusion.forward, rrnco/models/nn/attn_freenet.py:242-289 (ATSP / RCVRP encoders,
  * rrnco/models/encoder.py:63-66), times the block's `alpha` (attn_freenet.py:424-430).

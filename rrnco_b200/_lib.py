@@ -20,6 +20,8 @@ DEV_BAD_PARENT = 32
 MAX_NODES_TILE = 128     # one key tile: rrnco_decoder_logits, single-tile fused kernels
 MAX_NODES_FUSED = 1024   # rrnco_rollout (key-tiled kernel above MAX_NODES_TILE)
 MAX_BEAM_WIDTH = 1024   # rrnco_beam_select
+MAX_BEAM_WIDTH_FUSED = 128   # rrnco_beam_rollout (and N <= MAX_NODES_LEAN, default engine and precision)
+MAX_NODES_LEAN = 112     # the lean rollout kernel
 MIN_STARTS_TILED = 8   # RRNetDecoder.forward: starts per instance from which the any-N tile kernels serve every N
 
 _f = C.c_void_p  # every device pointer travels as void*
@@ -94,6 +96,9 @@ _SIGNATURES = {
     "rrnco_pointer_ffn_workspace_bytes": (C.c_int64, []),
     "rrnco_pointer_ffn": (C.c_int, [C.c_int64, _f, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_rollout_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int64, C.c_int32]),
+    "rrnco_beam_rollout_workspace_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int64, C.c_int32]),
+    "rrnco_beam_rollout": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.POINTER(DecoderWeights),
+                                     C.POINTER(DecoderCache), C.POINTER(InstanceData), C.c_int32, _f, _f, _f, _f, _f, _f, _f]),
     "rrnco_rollout": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_uint64,
                                 C.POINTER(DecoderWeights), C.POINTER(DecoderCache), C.POINTER(InstanceData), _f,
                                 C.c_int32, C.c_int32, _f, _f, _f, _f, _f, _f, _f, _f, _f]),
@@ -105,7 +110,7 @@ _SIGNATURES = {
 _lib = None
 launch_count = 0  # library calls that enqueued work
 kernel_count = 0  # CUDA kernels those calls launched (bench.py reports it as gpu_launches)
-_KERNELS_PER_CALL = {"rrnco_rollout": 3, "rrnco_rollout_filtered": 3, "rrnco_pointer_ffn": 2, "rrnco_decoder_logits_large": 4}  # rollout: weight pack + rollout + finalize  # rollout_kernel + finalize_kernel; every other entry point launches one
+_KERNELS_PER_CALL = {"rrnco_rollout": 3, "rrnco_rollout_filtered": 3, "rrnco_beam_rollout": 3, "rrnco_pointer_ffn": 2, "rrnco_decoder_logits_large": 4}  # rollout: weight pack + rollout + finalize  # rollout_kernel + finalize_kernel; every other entry point launches one
 
 
 def lib():

@@ -36,6 +36,11 @@ struct RolloutParams {
   int32_t top_k;                    // logit filters (filter_cut, common.cuh): read by the filtered instantiations only
   float top_p;
 };
+// The lean kernel's beam search (rrnco_beam_rollout): actions / logprob are step-major [t_cap, R] there, with the parent
+// rows beside them.  (A derived struct: the parameter layout of every other kernel stays as it is.)
+struct BeamParams : RolloutParams {
+  int64_t* beam_parent;
+};
 
 // Transcendentals of the softmax / bias / clip chain on the SFU (ex2 / lg2 / rcp .approx): absolute error
 // <~ 1e-6 on the ranges that occur here, i.e. below the 3xTF32 noise of the logits themselves (~3e-6).

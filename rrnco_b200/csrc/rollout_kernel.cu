@@ -1835,6 +1835,7 @@ int dispatch_env_tc(const RolloutParams& p, int env, int passes, cudaStream_t st
 #else
 int dispatch_env_tc(const RolloutParams& p, int env, int passes, cudaStream_t st);  // rollout_kernel_tc.cu
 int dispatch_env_lean(const RolloutParams& p, int env, int passes, cudaStream_t st);  // rollout_lean.cu
+int dispatch_env_lean_beam(const BeamParams& p, int env, cudaStream_t st);            // rollout_lean.cu
 int pack_ffn_lean(const float* w1, const float* w2, const float* b1, const float* b2, void* packed, uint32_t* status,
                   cudaStream_t st);
 constexpr int64_t kLeanBiasBytes = 4096;  // scaled biases behind the packed weight slices
@@ -1901,6 +1902,25 @@ void rollout_tiling(int32_t n_nodes, int64_t n_inst, int32_t n_starts, int* tile
   *n_tiles = (n_starts + tr - 1) / tr;
 }
 bool g_last_tiled = false;  // the last rrnco_rollout call ran the key-tiled kernel (which counters rrnco_debug_phase_cycles reads)
+// rrnco_rollout_workspace_bytes' layout: per-rollout tour lengths and log-likelihoods (fp64), the CTA tiles' step counts, the
+// packed FFN weights and scaled biases, the packed K / V / logit-key tiles
+void set_workspace(RolloutParams& p, void* workspace, int64_t R) {
+  p.ws_len = reinterpret_cast<double*>(workspace);
+  p.ws_lp = p.ws_len + R;
+  p.ws_tile_steps = reinterpret_cast<int32_t*>(p.ws_lp + R);
+  const int64_t tiles = p.n_inst * p.n_tiles;
+  unsigned char* packed = reinterpret_cast<unsigned char*>(p.ws_tile_steps) + ((tiles * (int64_t)sizeof(int32_t) + 15) & ~15LL);
+  p.ffn_packed = packed;
+  p.ffn_bias_scaled = reinterpret_cast<const float*>(packed + kFfnPackedBytes);
+  p.kv_pack = packed + kFfnPackedBytes + kLeanBiasBytes;  // 16-byte aligned: every part above is a multiple of 16 bytes
+}
+int check_instance_data(int32_t env, const rrnco_instance_data_t* data) {
+  if (env == RRNCO_ENV_RCVRP) RRNCO_CHECK_ARG(data->demand && data->vehicle_capacity);
+  if (env == RRNCO_ENV_RCVRPTW)
+    RRNCO_CHECK_ARG(data->demand && data->demand_backhaul && data->time_windows && data->service_time &&
+                    data->vehicle_capacity && data->distance_limit && data->open_route && data->backhaul_class);
+  return RRNCO_OK;
+}
 int g_engine = 2;  // engine of the fused rollout: 2 = tcgen05, two lean CTAs per SM (N <= 112; else 1), 1 = tcgen05, one CTA
                    // per SM, 0 = mma.sync
 
@@ -2002,10 +2022,8 @@ int rrnco_rollout_filtered(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t
   RRNCO_CHECK_ARG(multistart || n_starts == 1);
   RRNCO_CHECK_ARG(decode_mode != RRNCO_DECODE_EVALUATE || (forced_actions && forced_T > 0));
   RRNCO_CHECK_ARG(real_reward_out == nullptr || (data->min_distance && data->max_distance));
-  if (env == RRNCO_ENV_RCVRP) RRNCO_CHECK_ARG(data->demand && data->vehicle_capacity);
-  if (env == RRNCO_ENV_RCVRPTW)
-    RRNCO_CHECK_ARG(data->demand && data->demand_backhaul && data->time_windows && data->service_time &&
-                    data->vehicle_capacity && data->distance_limit && data->open_route && data->backhaul_class);
+  rc = check_instance_data(env, data);
+  if (rc != RRNCO_OK) return rc;
   if (env == RRNCO_ENV_ATSP && !multistart) RRNCO_CHECK_ARG(w->ctx_placeholder_q != nullptr);
   cudaStream_t st = (cudaStream_t)stream;
   RolloutParams p{};
@@ -2017,14 +2035,8 @@ int rrnco_rollout_filtered(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t
   p.w = *w; p.c = *cache; p.d = *data;
   p.forced = forced_actions; p.actions = actions_out; p.logprob = logprob_out;
   const int64_t R = n_inst * n_starts;
-  p.ws_len = reinterpret_cast<double*>(workspace);
-  p.ws_lp = p.ws_len + R;
-  p.ws_tile_steps = reinterpret_cast<int32_t*>(p.ws_lp + R);
-  const int64_t tiles = n_inst * p.n_tiles;
-  unsigned char* packed = reinterpret_cast<unsigned char*>(p.ws_tile_steps) + ((tiles * (int64_t)sizeof(int32_t) + 15) & ~15LL);
-  p.ffn_packed = packed;
-  p.ffn_bias_scaled = reinterpret_cast<const float*>(packed + kFfnPackedBytes);
-  p.kv_pack = packed + kFfnPackedBytes + kLeanBiasBytes;  // 16-byte aligned: every part above is a multiple of 16 bytes
+  set_workspace(p, workspace, R);
+  void* packed = const_cast<unsigned char*>(p.ffn_packed);
   p.max_steps_out = max_steps_out; p.status = status;
   p.top_k = filtered ? top_k : 0; p.top_p = filtered ? top_p : 0.f;
   if (cudaMemsetAsync(max_steps_out, 0, sizeof(int32_t), st) != cudaSuccess) return RRNCO_ERR_CUDA;
@@ -2054,6 +2066,43 @@ int rrnco_rollout_filtered(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t
     default: finalize_kernel<RRNCO_ENV_RCVRPTW><<<fgrid, 256, 0, st>>>(p, loglik_out, norm_reward_out, real_reward_out); break;
   }
   return rrnco_launch_status();
+}
+
+int64_t rrnco_beam_rollout_workspace_bytes(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t beam_width) {
+  if (beam_width < 2 || beam_width > RRNCO_MAX_BEAM_WIDTH_FUSED || n_nodes < 2 || n_nodes > kLeanMaxNodes || g_engine != 2 ||
+      g_passes != 3)
+    return 0;
+  return rrnco_rollout_workspace_bytes(env, n_nodes, n_inst, beam_width);
+}
+
+int rrnco_beam_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t beam_width, const rrnco_decoder_weights_t* w,
+                       const rrnco_decoder_cache_t* cache, const rrnco_instance_data_t* data, int32_t t_cap,
+                       int64_t* step_actions, int64_t* step_parents, float* step_logprobs, int32_t* n_steps_out,
+                       uint32_t* status, void* workspace, void* stream) {
+  RRNCO_CHECK_ARG(beam_width >= 2);
+  if (beam_width > RRNCO_MAX_BEAM_WIDTH_FUSED || n_nodes > kLeanMaxNodes || g_engine != 2 || g_passes != 3)
+    return RRNCO_ERR_UNSUPPORTED;
+  int rc = check_common(env, n_nodes, n_inst, beam_width, w, cache, data);
+  if (rc != RRNCO_OK) return rc;
+  RRNCO_CHECK_ARG(step_actions && step_parents && step_logprobs && n_steps_out && status && workspace && aligned16(workspace));
+  RRNCO_CHECK_ARG(t_cap > 1);
+  rc = check_instance_data(env, data);
+  if (rc != RRNCO_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  BeamParams p{};
+  p.N = n_nodes; p.NT = (n_nodes + 7) / 8; p.S = beam_width; p.tile_rows = kRows; p.n_tiles = 1;
+  p.n_state = env == RRNCO_ENV_ATSP ? 0 : env == RRNCO_ENV_RCVRP ? 1 : 4;
+  p.n_inst = n_inst; p.multistart = 1; p.mode = RRNCO_DECODE_GREEDY;
+  p.t_cap = t_cap; p.max_steps = t_cap - 1;
+  p.w = *w; p.c = *cache; p.d = *data;
+  p.actions = step_actions; p.beam_parent = step_parents; p.logprob = step_logprobs;
+  set_workspace(p, workspace, n_inst * beam_width);
+  p.max_steps_out = n_steps_out; p.status = status;
+  if (cudaMemsetAsync(n_steps_out, 0, sizeof(int32_t), st) != cudaSuccess) return RRNCO_ERR_CUDA;
+  g_last_tiled = false;
+  rc = pack_ffn_lean(w->ffn_w1, w->ffn_w2, w->ffn_b1, w->ffn_b2, const_cast<unsigned char*>(p.ffn_packed), status, st);
+  if (rc != RRNCO_OK) return rc;
+  return dispatch_env_lean_beam(p, env, st);
 }
 
 int rrnco_rollout(int32_t env, int32_t n_nodes, int64_t n_inst, int32_t n_starts, int32_t multistart,

@@ -19,6 +19,7 @@
 // zeroing passes), one elected thread of warp 8 issues every bulk copy; warps 0-7 run the element-wise passes
 // thread-per-rollout.  Results are bitwise reproducible and identical in value to rollout_kernel<..., kTc = true>.
 #include <cstdio>
+#include <type_traits>
 #include "common.cuh"
 #include "tc05.cuh"
 #include "ffn_pack.cuh"
@@ -89,6 +90,22 @@ struct LeanSmem {
   uint64_t bar_acc;      // issuer -> compute: logits complete
   uint32_t tmem_base;
   volatile int exit_flag;
+};
+// beam search: the running score of each beam row (fp32, score_t = score_{t-1} + lp_t), moved with the rest of the row's
+// state when the rows are permuted to their parents
+template <int kEnv>
+struct LeanBeamSmem : LeanSmem<kEnv> {
+  float score[kRows];
+};
+// beam select scratch in the activation region: behind the bias tile (which holds the candidates' log-probs) over the
+// exchange arrays, dead once the rows' (max, log sum) are read, and one radix histogram behind those
+constexpr int kLXchgEnd = kLBiasBytes + 4 * 2 * kRows * 4 + 2 * kRows;
+struct LeanBeamScratch {
+  uint32_t key[kRows];   // selected candidates (unordered): order-preserving key of score + lp
+  int idx[kRows];        // their flat index w N + j
+  int rowoff[kRows];     // candidates of key == K per row, then their exclusive prefix over the rows
+  int ranked[kRows];     // flat index of rank w
+  int digit, need, n_gt, all_fin;
 };
 
 __device__ __forceinline__ void lean_sync() { asm volatile("bar.sync 1, 256;\n" ::: "memory"); }
@@ -178,11 +195,225 @@ __device__ __forceinline__ float lean_transition(LeanSmem<kEnv>& sm, int N, int 
   return leg;
 }
 
+// ---- one beam search step (rl4co BeamSearch._make_beam_step; rrnco_beam_select's rule) on the compute warps, after the
+// single-pass select has left each row's processed values over its bias row and its (max, sum) partials in xf.
+//   1. lp = (v - max) - log sum in place: the rollout's log-prob of every column.
+//   2. The p.S largest candidates score[w] + lp[w, j] (flat index w N + j): a 4-pass 8-bit radix select over the finite
+//      candidates on the order-preserving key of filter_key, then every key > K and the lowest flat indices of key == K.
+//   3. A rank count orders them (value desc, flat index asc); ranks from #finite upward copy rank 0 (_fill_up_beams).
+//   4. Each beam row reads its parent row's state, and after a barrier writes it to itself and steps the env.
+// Writes the step's (action, parent row, lp) step-major at t_out, the layout rrnco_beam_backtrack reads.
+template <int kEnv>
+__device__ __forceinline__ void lean_beam_step(LeanBeamSmem<kEnv>& sm, const BeamParams& p, float (*xf)[2][kRows],
+                                               float* vrow, int nq, int64_t b, int t_out, const float* D, const float* U,
+                                               float closed) {
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int row = (warp & 3) * 32 + lane;
+  const int W = p.S, N = p.N;
+  const float* lpt = reinterpret_cast<const float*>(sm.A);  // [kRows][kLBiasLd]
+  LeanBeamScratch& bs = *reinterpret_cast<LeanBeamScratch*>(sm.A + kLBiasBytes);
+  int* hist = reinterpret_cast<int*>(sm.A + kLXchgEnd);  // [256]
+  {
+    const float m0 = xf[0][0][row], m1 = xf[0][1][row];
+    const float mx = fmaxf(m0, m1);
+    const float se = flog(xf[1][0][row] * fexp(m0 - mx) + xf[1][1][row] * fexp(m1 - mx));
+#pragma unroll 1
+    for (int q = 0; q < nq; ++q) {
+#pragma unroll
+      for (int i = 0; i < 16; ++i) vrow[32 * q + i] = __fsub_rn(__fsub_rn(vrow[32 * q + i], mx), se);
+    }
+    hist[tid] = 0;
+  }
+  lean_sync();  // every lp written, the exchange arrays read
+  if (tid == 0) bs.n_gt = 0;
+  const uint32_t kNone = filter_key(-INFINITY);
+  auto cand_key = [&](int w, int j) -> uint32_t {  // this warp's candidates: rows w = warp + 8 k < W, columns j = lane + 32 c
+    return j < N ? filter_key(__fadd_rn(sm.score[w], lpt[w * kLBiasLd + j])) : kNone;
+  };
+  uint32_t prefix = 0u, pmask = 0u;
+  int need = W;
+  bool all_fin = false;
+#pragma unroll 1
+  for (int shift = 24; shift >= 0; shift -= 8) {
+#pragma unroll 1
+    for (int w = warp; w < W; w += 8) {
+#pragma unroll
+      for (int c = 0; c < 4; ++c) {
+        const uint32_t k = cand_key(w, 32 * c + lane);
+        const bool hit = k > kNone && (k & pmask) == prefix;  // non-finite candidates are never ranked (fill-up instead)
+        const uint32_t bin = (k >> shift) & 255u;
+        if (__ballot_sync(0xffffffffu, hit)) {  // one shared-memory atomic per distinct bin of the warp
+          const uint32_t peers = __match_any_sync(0xffffffffu, hit ? bin : 0xffffffffu);
+          if (hit && __ffs(peers) - 1 == lane) atomicAdd(&hist[bin], __popc(peers));
+        }
+      }
+    }
+    lean_sync();
+    if (warp == 0) {  // the digit of the need-th largest: lane l holds bins 255 - 8 l .. 248 - 8 l, counted from the top
+      int cnt[8], s = 0;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        cnt[e] = hist[255 - 8 * lane - e];
+        s += cnt[e];
+      }
+      int incl = s;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+      }
+      const uint32_t over = __ballot_sync(0xffffffffu, incl >= need);
+      if (over == 0u) {  // fewer finite candidates than beams (first pass only): every finite one is kept
+        if (lane == 0) bs.all_fin = 1;
+      } else if (lane == __ffs(over) - 1) {
+        int acc = incl - s, d = -1, rest = 0;
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+          if (d < 0 && acc + cnt[e] >= need) {
+            d = 255 - 8 * lane - e;
+            rest = need - acc;
+          }
+          if (d < 0) acc += cnt[e];
+        }
+        bs.digit = d;
+        bs.need = rest;
+        bs.all_fin = 0;
+      }
+      __syncwarp();
+#pragma unroll
+      for (int e = 0; e < 8; ++e) hist[8 * lane + e] = 0;
+    }
+    lean_sync();
+    if (bs.all_fin) {
+      all_fin = true;
+      break;
+    }
+    prefix |= (uint32_t)bs.digit << shift;
+    pmask |= 255u << shift;
+    need = bs.need;
+  }
+  // collect every key > K (unordered), and count the keys == K of each row
+  const uint32_t K = all_fin ? kNone : prefix;
+  const int n_eq = all_fin ? 0 : need;
+#pragma unroll 1
+  for (int w = warp; w < W; w += 8) {
+    int cnt = 0;
+#pragma unroll
+    for (int c = 0; c < 4; ++c) {
+      const int j = 32 * c + lane;
+      const uint32_t k = cand_key(w, j);
+      if (k > K) {
+        const int s = atomicAdd(&bs.n_gt, 1);
+        bs.key[s] = k;
+        bs.idx[s] = w * N + j;
+      }
+      cnt += __popc(__ballot_sync(0xffffffffu, k == K));
+    }
+    if (lane == 0) bs.rowoff[w] = cnt;
+  }
+  lean_sync();
+  if (warp == 0) {  // exclusive prefix of the per-row counts over the rows (4 rows per lane): flat order of the ties
+    int v[4], s = 0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const int w = 4 * lane + e;
+      v[e] = w < W ? bs.rowoff[w] : 0;
+      s += v[e];
+    }
+    int incl = s;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int t = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += t;
+    }
+    int off = incl - s;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const int w = 4 * lane + e;
+      if (w < W) bs.rowoff[w] = off;
+      off += v[e];
+    }
+  }
+  lean_sync();
+  const int n_gt = bs.n_gt;
+  if (n_eq > 0) {  // the n_eq lowest flat indices of key == K
+#pragma unroll 1
+    for (int w = warp; w < W; w += 8) {
+      int base = bs.rowoff[w];
+      if (base >= n_eq) continue;
+#pragma unroll
+      for (int c = 0; c < 4; ++c) {
+        const int j = 32 * c + lane;
+        const bool eq = cand_key(w, j) == K;
+        const uint32_t bal = __ballot_sync(0xffffffffu, eq);
+        const int rank = base + __popc(bal & ((1u << lane) - 1u));
+        if (eq && rank < n_eq) {
+          bs.key[n_gt + rank] = K;
+          bs.idx[n_gt + rank] = w * N + j;
+        }
+        base += __popc(bal);
+      }
+    }
+  }
+  lean_sync();
+  const int n_sel = n_gt + n_eq;
+  if (tid < n_sel) {  // rank: (value desc, flat index asc)
+    const uint32_t ki = bs.key[tid];
+    const int fi = bs.idx[tid];
+    int rk = 0;
+#pragma unroll 4
+    for (int i = 0; i < n_sel; ++i) rk += (bs.key[i] > ki || (bs.key[i] == ki && bs.idx[i] < fi)) ? 1 : 0;
+    bs.ranked[rk] = fi;
+  }
+  lean_sync();
+  const int fin = all_fin ? n_gt : W;  // (a full selection holds finite keys only: K is the key of a finite candidate)
+  int par = 0, act = 0;
+  float lp = 0.f, sc = 0.f;
+  int cur = 0, first = 0, done = 0;
+  uint4 vis = make_uint4(0u, 0u, 0u, 0u);
+  float fs[LeanSmem<kEnv>::kStateArrays];
+  if (tid < W) {
+    const int f = fin > 0 ? bs.ranked[tid < fin ? tid : 0] : 0;
+    par = f / N;
+    act = f - par * N;
+    lp = lpt[par * kLBiasLd + act];
+    sc = __fadd_rn(sm.score[par], lp);
+    cur = sm.cur[par];
+    first = sm.first[par];
+    done = sm.done[par];
+    vis = *reinterpret_cast<const uint4*>(sm.vis[par]);
+#pragma unroll
+    for (int k = 0; k < LeanSmem<kEnv>::kStateArrays; ++k) fs[k] = sm.f[k][par];
+  }
+  if (tid == 0 && fin == 0) atomicOr(p.status, RRNCO_DEV_NO_FEASIBLE);
+  lean_sync();  // every parent state read
+  if (tid < W) {
+    const int w = tid;
+    sm.cur[w] = (unsigned char)cur;
+    sm.first[w] = (unsigned char)first;
+    sm.done[w] = (unsigned char)done;
+    *reinterpret_cast<uint4*>(sm.vis[w]) = vis;
+#pragma unroll
+    for (int k = 0; k < LeanSmem<kEnv>::kStateArrays; ++k) sm.f[k][w] = fs[k];
+    sm.score[w] = sc;
+    lean_transition<kEnv>(sm, N, w, act, D, U, closed, true);
+    if (t_out < p.t_cap) {
+      const int64_t i = (int64_t)t_out * (p.n_inst * W) + (int64_t)w * p.n_inst + b;
+      p.actions[i] = act;
+      p.beam_parent[i] = (int64_t)par * p.n_inst + b;
+      p.logprob[i] = lp;
+    }
+  }
+}
+
 // kFilter: decode with the top-k / top-p filters of p (single-pass select only)
-template <int kEnv, int kPasses, bool kFilter>
-__global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const RolloutParams p) {
+// kBeam: beam search (rrnco_beam_rollout): the p.S <= kRows rows of the CTA's one tile are the beams of instance b; each
+// step ranks the S x N candidates score + lp across the tile and moves every row's state to its parent row
+template <int kEnv, int kPasses, bool kFilter, bool kBeam = false>
+__global__ void __launch_bounds__(kLThreads, 2)
+    rollout_lean_kernel(const typename std::conditional<kBeam, BeamParams, RolloutParams>::type p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  using SmemT = LeanSmem<kEnv>;
+  using SmemT = typename std::conditional<kBeam, LeanBeamSmem<kEnv>, LeanSmem<kEnv>>::type;
   SmemT& sm = *reinterpret_cast<SmemT*>(smem_raw);
   constexpr int kNA = SmemT::kNodeArrays - 1, kSA = SmemT::kStateArrays - 1;
   // node-array / state-array indices, clamped so that every instantiation stays in bounds
@@ -317,7 +548,14 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
       const int a0 = s % num_loc + (kEnv == RRNCO_ENV_ATSP ? 0 : 1);  // select_start_nodes
       len_acc += (double)lean_transition<kEnv>(sm, N, row, a0, D, U, closed, /*count_leg=*/false);  // depot -> a0 (VRPs)
       sm.first[row] = (unsigned char)a0;
-      if (active) {
+      if constexpr (kBeam) {  // step 0 of the beam records: the start, log-prob 0 (its parent is never read)
+        sm.score[row] = 0.f;
+        if (active) {
+          p.actions[r] = a0;
+          p.beam_parent[r] = 0;
+          p.logprob[r] = 0.f;
+        }
+      } else if (active) {
         p.actions[r * p.t_cap] = a0;
         if (p.logprob) p.logprob[r * p.t_cap] = 0.f;
       }
@@ -1099,7 +1337,11 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
         const float ms2 = (m == -INFINITY ? 0.f : m) * 1.4426950408889634f;
 #pragma unroll
         for (int i = 0; i < 16; ++i) ssum += ex2a(fmaf(val[i], 1.4426950408889634f, -ms2));
-        if (p.mode == RRNCO_DECODE_SAMPLING) {
+        if constexpr (kBeam) {  // the values over this thread's columns of the bias tile: the beam select reads them
+          float* vw = const_cast<float*>(brow) + 32 * q;
+#pragma unroll
+          for (int i = 0; i < 16; i += 4) *reinterpret_cast<float4*>(vw + i) = make_float4(val[i], val[i + 1], val[i + 2], val[i + 3]);
+        } else if (p.mode == RRNCO_DECODE_SAMPLING) {
 #pragma unroll 1
           for (int i4 = 0; i4 < 16; i4 += 4) {
             const float4 gn = gumbel4(make_uint4((uint32_t)rg, (uint32_t)(rg >> 32), (uint32_t)step, (uint32_t)((cbase + i4) >> 2)), key2);
@@ -1138,7 +1380,9 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
       LSTAMP(17);
       lean_sync();
       LSTAMP(18);
-      if (colhalf == 0) {
+      if constexpr (kBeam) {
+        lean_beam_step<kEnv>(sm, p, xf, const_cast<float*>(brow), nq, b, t_out, D, U, closed);
+      } else if (colhalf == 0) {
         const float m0 = xf[0][0][row], m1 = xf[0][1][row];
         const float mx = fmaxf(m0, m1);
         const float se = flog(xf[1][0][row] * fexp(m0 - mx) + xf[1][1][row] * fexp(m1 - mx));
@@ -1322,7 +1566,7 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
   }
 
   // ---------------- exit: close the tours, publish per-rollout sums ----------------
-  if (tid < kRows && sm.active[tid]) {  // tid < 128 = warps 0-3 = column half 0: the threads that own len_acc / lp_acc
+  if (!kBeam && tid < kRows && sm.active[tid]) {  // tid < 128 = warps 0-3 = column half 0: the threads that own len_acc / lp_acc
     const int row = tid;
     const int64_t r = (int64_t)(tile * kRows + row) * p.n_inst + b;
     const int last = sm.cur[row];
@@ -1348,12 +1592,13 @@ __global__ void __launch_bounds__(kLThreads, 2) rollout_lean_kernel(const Rollou
   if (warp == 0) tc05::tmem_dealloc(sm.tmem_base, 256);
 }
 
-template <int kEnv, int kPasses, bool kFilter>
-static int launch_lean(const RolloutParams& p, cudaStream_t st) {
-  auto kern = rollout_lean_kernel<kEnv, kPasses, kFilter>;
+template <int kEnv, int kPasses, bool kFilter, bool kBeam = false>
+static int launch_lean(const typename std::conditional<kBeam, BeamParams, RolloutParams>::type& p, cudaStream_t st) {
+  auto kern = rollout_lean_kernel<kEnv, kPasses, kFilter, kBeam>;
+  constexpr int kSmem = (int)sizeof(typename std::conditional<kBeam, LeanBeamSmem<kEnv>, LeanSmem<kEnv>>::type);
   static PerDeviceOnce once;
   if (once.first()) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(LeanSmem<kEnv>)) != cudaSuccess ||
+    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem) != cudaSuccess ||
         cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) != cudaSuccess) {
       once.undo();
       return RRNCO_ERR_CUDA;
@@ -1361,8 +1606,23 @@ static int launch_lean(const RolloutParams& p, cudaStream_t st) {
   }
   const int64_t grid = p.n_inst * p.n_tiles;
   if (grid <= 0 || grid > 0x7fffffffLL) return RRNCO_ERR_UNSUPPORTED;
-  kern<<<(unsigned)grid, kLThreads, sizeof(LeanSmem<kEnv>), st>>>(p);
+  kern<<<(unsigned)grid, kLThreads, kSmem, st>>>(p);
   return rrnco_launch_status();
+}
+
+// After a beam rollout: the steps that a tile did not run (all its beams were done) keep every beam as it was, as the
+// per-step pipeline does for such an instance: parent = the row itself, action 0, log-prob 0.
+__global__ void __launch_bounds__(256) beam_tail_kernel(const BeamParams p) {
+  const int64_t R = p.n_inst * (int64_t)p.S;
+  const int t_glob = min(*p.max_steps_out, p.t_cap);
+  for (int64_t r = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; r < R; r += (int64_t)gridDim.x * blockDim.x) {
+    for (int t = p.ws_tile_steps[r % p.n_inst]; t < t_glob; ++t) {
+      const int64_t i = (int64_t)t * R + r;
+      p.actions[i] = 0;
+      p.beam_parent[i] = r;
+      p.logprob[i] = 0.f;
+    }
+  }
 }
 
 // entry points used by rrnco_rollout (rollout_kernel.cu)
@@ -1384,6 +1644,31 @@ int phase_cycles_lean(long long* h_out, int reset) {
   }
   return RRNCO_OK;
 }
+// rrnco_beam_rollout (rollout_kernel.cu): one CTA per instance (p.n_tiles == 1), fp32-faithful operands only
+int dispatch_env_lean_beam(const BeamParams& p, int env, cudaStream_t st) {
+  static_assert(sizeof(LeanBeamSmem<RRNCO_ENV_RCVRPTW>) <= 115712 && sizeof(LeanBeamSmem<RRNCO_ENV_RCVRP>) <= 115712 &&
+                    sizeof(LeanBeamSmem<RRNCO_ENV_ATSP>) <= 115712, "two CTAs per SM need <= 113 KB of shared memory each");
+  static_assert(kLBiasBytes + (int)sizeof(LeanBeamScratch) <= kLXchgEnd && kLXchgEnd + 256 * 4 <= kRows * kE * 4,
+                "beam select scratch and histogram fit the A region");
+#ifdef RRNCO_LEAN_SELECT3
+  (void)p; (void)env; (void)st;
+  return RRNCO_ERR_UNSUPPORTED;  // the beam select is built on the single-pass form
+#else
+  int rc;
+  switch (env) {
+    case RRNCO_ENV_ATSP: rc = launch_lean<RRNCO_ENV_ATSP, 3, false, true>(p, st); break;
+    case RRNCO_ENV_RCVRP: rc = launch_lean<RRNCO_ENV_RCVRP, 3, false, true>(p, st); break;
+    case RRNCO_ENV_RCVRPTW: rc = launch_lean<RRNCO_ENV_RCVRPTW, 3, false, true>(p, st); break;
+    default: return RRNCO_ERR_BAD_ARG;
+  }
+  if (rc != RRNCO_OK) return rc;
+  const int64_t R = p.n_inst * (int64_t)p.S;
+  const unsigned grid = (unsigned)((R + 255) / 256 > 4096 ? 4096 : (R + 255) / 256);
+  beam_tail_kernel<<<grid, 256, 0, st>>>(p);
+  return rrnco_launch_status();
+#endif
+}
+
 int dispatch_env_lean(const RolloutParams& p, int env, int passes, cudaStream_t st) {
   static_assert(sizeof(LeanSmem<RRNCO_ENV_RCVRPTW>) <= 115712 && sizeof(LeanSmem<RRNCO_ENV_RCVRP>) <= 115712 &&
                     sizeof(LeanSmem<RRNCO_ENV_ATSP>) <= 115712, "two CTAs per SM need <= 113 KB of shared memory each");

@@ -13,6 +13,7 @@
 //   select_action                      DecodingStrategy.step             rrnco/models/decoding.py:219-298
 //   rollout                            RRNetPolicy.forward decode loop   rrnco/models/policy.py:203-243
 //   beam_select / beam_backtrack       BeamSearch step / _backtrack      rrnco/models/decoding.py:402-542
+//   beam_rollout                       BeamSearch decode loop, fused     rrnco/models/decoding.py:402-542
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
@@ -198,6 +199,35 @@ std::tuple<Tensor, Tensor, Tensor> beam_backtrack(const Tensor& actions, const T
 // cache  : [glimpse_key, glimpse_val, logit_key, ctx_node_proj, ctx_node_proj2?]
 // data   : [distance, duration?, demand?, demand_backhaul?, time_windows?, service_time?, vehicle_capacity?, distance_limit?,
 //           open_route?, backhaul_class?, min_distance?, max_distance?]   (the members of rrnco_instance_data_t, in order)
+struct DecoderArgs {
+  rrnco_decoder_weights_t w{};
+  rrnco_decoder_cache_t c{};
+  rrnco_instance_data_t d{};
+};
+DecoderArgs decoder_args(const c10::List<OptTensor>& weights, double alpha, double beta, double tanh_clipping, double temperature,
+                         const c10::List<OptTensor>& cache, const c10::List<OptTensor>& data) {
+  TORCH_CHECK(weights.size() == 6 && cache.size() == 5 && data.size() == 12, "weights[6], cache[5], data[12] expected");
+  auto W = [&](size_t i) -> OptTensor { return weights.get(i); };
+  auto C = [&](size_t i) -> OptTensor { return cache.get(i); };
+  auto D = [&](size_t i) -> OptTensor { return data.get(i); };
+  DecoderArgs a;
+  rrnco_decoder_weights_t& w = a.w;
+  w.ffn_w1 = cptr<float>(W(0)); w.ffn_b1 = cptr<float>(W(1)); w.ffn_w2 = cptr<float>(W(2)); w.ffn_b2 = cptr<float>(W(3));
+  w.ctx_state_w = cptr<float>(W(4)); w.ctx_placeholder_q = cptr<float>(W(5));
+  w.alpha = (float)alpha; w.beta = (float)beta; w.tanh_clipping = (float)tanh_clipping; w.temperature = (float)temperature;
+  rrnco_decoder_cache_t& c = a.c;
+  c.glimpse_key = cptr<float>(C(0)); c.glimpse_val = cptr<float>(C(1)); c.logit_key = cptr<float>(C(2));
+  c.ctx_node_proj = cptr<float>(C(3)); c.ctx_node_proj2 = cptr<float>(C(4));
+  TORCH_CHECK(D(0).has_value(), "data[0] (distance) is required");
+  rrnco_instance_data_t& d = a.d;
+  d.data_rows = D(0)->size(0);
+  d.distance = cptr<float>(D(0)); d.duration = cptr<float>(D(1)); d.demand = cptr<float>(D(2)); d.demand_backhaul = cptr<float>(D(3));
+  d.time_windows = cptr<float>(D(4)); d.service_time = cptr<float>(D(5)); d.vehicle_capacity = cptr<float>(D(6));
+  d.distance_limit = cptr<float>(D(7)); d.open_route = cptr<uint8_t>(D(8)); d.backhaul_class = cptr<float>(D(9));
+  d.min_distance = cptr<float>(D(10)); d.max_distance = cptr<float>(D(11));
+  return a;
+}
+
 // -> (actions [R, t_cap], logprob [R, t_cap] | empty, log_likelihood [R], normalised reward [R], real reward [R] | empty,
 //     info int32 [2] = (longest rollout T, device status word), tile_steps int32 [n_inst * ceil(S / rrnco_rollout_tile_rows)])
 std::tuple<Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor> rollout(
@@ -205,28 +235,15 @@ std::tuple<Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor> rollout(
     double alpha, double beta, double tanh_clipping, double temperature, const c10::List<OptTensor>& cache,
     const c10::List<OptTensor>& data, const OptTensor& forced_actions, int64_t t_cap, bool per_step_logprobs, Tensor workspace,
     int64_t top_k, double top_p) {
-  TORCH_CHECK(weights.size() == 6 && cache.size() == 5 && data.size() == 12, "rollout: weights[6], cache[5], data[12] expected");
-  auto W = [&](size_t i) -> OptTensor { return weights.get(i); };
-  auto C = [&](size_t i) -> OptTensor { return cache.get(i); };
-  auto D = [&](size_t i) -> OptTensor { return data.get(i); };
-  TORCH_CHECK(C(0).has_value() && C(0)->is_cuda() && C(0)->dim() == 3, "cache tensors [n_inst,N,E] on CUDA expected");
-  const Tensor& key = *C(0);
+  TORCH_CHECK(cache.size() == 5 && cache.get(0).has_value() && cache.get(0)->is_cuda() && cache.get(0)->dim() == 3,
+              "cache tensors [n_inst,N,E] on CUDA expected");
+  const Tensor key = *cache.get(0);
   c10::cuda::CUDAGuard guard(key.device());
   const int64_t n_inst = key.size(0), N = key.size(1), R = n_inst * n_starts;
-  rrnco_decoder_weights_t w{};
-  w.ffn_w1 = cptr<float>(W(0)); w.ffn_b1 = cptr<float>(W(1)); w.ffn_w2 = cptr<float>(W(2)); w.ffn_b2 = cptr<float>(W(3));
-  w.ctx_state_w = cptr<float>(W(4)); w.ctx_placeholder_q = cptr<float>(W(5));
-  w.alpha = (float)alpha; w.beta = (float)beta; w.tanh_clipping = (float)tanh_clipping; w.temperature = (float)temperature;
-  rrnco_decoder_cache_t c{};
-  c.glimpse_key = cptr<float>(C(0)); c.glimpse_val = cptr<float>(C(1)); c.logit_key = cptr<float>(C(2));
-  c.ctx_node_proj = cptr<float>(C(3)); c.ctx_node_proj2 = cptr<float>(C(4));
-  TORCH_CHECK(D(0).has_value(), "data[0] (distance) is required");
-  rrnco_instance_data_t d{};
-  d.data_rows = D(0)->size(0);
-  d.distance = cptr<float>(D(0)); d.duration = cptr<float>(D(1)); d.demand = cptr<float>(D(2)); d.demand_backhaul = cptr<float>(D(3));
-  d.time_windows = cptr<float>(D(4)); d.service_time = cptr<float>(D(5)); d.vehicle_capacity = cptr<float>(D(6));
-  d.distance_limit = cptr<float>(D(7)); d.open_route = cptr<uint8_t>(D(8)); d.backhaul_class = cptr<float>(D(9));
-  d.min_distance = cptr<float>(D(10)); d.max_distance = cptr<float>(D(11));
+  const DecoderArgs args = decoder_args(weights, alpha, beta, tanh_clipping, temperature, cache, data);
+  const rrnco_decoder_weights_t& w = args.w;
+  const rrnco_decoder_cache_t& c = args.c;
+  const rrnco_instance_data_t& d = args.d;
   const bool has_mm = d.min_distance != nullptr;
   Tensor forced;
   int64_t forced_T = 0;
@@ -255,6 +272,33 @@ std::tuple<Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor> rollout(
   return {actions, logprob, ll, norm, real, info, tile_steps};
 }
 
+// The whole beam search in one fused launch (rrnco_beam_rollout): -> (actions, parent rows, log-probs: step-major
+// [t_cap, R], rows >= T unwritten; info int32 [2] = (steps T, device status word)), the inputs of beam_backtrack
+std::tuple<Tensor, Tensor, Tensor, Tensor> beam_rollout(int64_t env, int64_t beam_width, const c10::List<OptTensor>& weights,
+                                                        double alpha, double beta, double tanh_clipping, double temperature,
+                                                        const c10::List<OptTensor>& cache, const c10::List<OptTensor>& data,
+                                                        int64_t t_cap, Tensor workspace) {
+  TORCH_CHECK(cache.size() == 5 && cache.get(0).has_value() && cache.get(0)->is_cuda() && cache.get(0)->dim() == 3,
+              "cache tensors [n_inst,N,E] on CUDA expected");
+  const Tensor key = *cache.get(0);
+  c10::cuda::CUDAGuard guard(key.device());
+  const int64_t n_inst = key.size(0), N = key.size(1), R = n_inst * beam_width;
+  const DecoderArgs args = decoder_args(weights, alpha, beta, tanh_clipping, temperature, cache, data);
+  const int64_t need = rrnco_beam_rollout_workspace_bytes((int32_t)env, (int32_t)N, n_inst, (int32_t)beam_width);
+  TORCH_CHECK(workspace.is_cuda() && workspace.scalar_type() == at::kByte && workspace.numel() >= need,
+              "beam_rollout: workspace of >= ", need, " bytes (uint8, CUDA) expected");
+  auto lopt = key.options().dtype(at::kLong);
+  Tensor actions = at::empty({t_cap, R}, lopt), parents = at::empty({t_cap, R}, lopt);
+  Tensor logprob = at::empty({t_cap, R}, key.options().dtype(at::kFloat));
+  Tensor info = at::zeros({2}, key.options().dtype(at::kInt));
+  check_rc(rrnco_beam_rollout((int32_t)env, (int32_t)N, n_inst, (int32_t)beam_width, &args.w, &args.c, &args.d, (int32_t)t_cap,
+                              actions.data_ptr<int64_t>(), parents.data_ptr<int64_t>(), logprob.data_ptr<float>(),
+                              info.data_ptr<int32_t>(), reinterpret_cast<uint32_t*>(info.data_ptr<int32_t>() + 1),
+                              workspace.data_ptr<uint8_t>(), stream_of(key)),
+           "beam_rollout");
+  return {actions, parents, logprob, info};
+}
+
 int64_t rollout_workspace_bytes(int64_t env, int64_t n_nodes, int64_t n_inst, int64_t n_starts) {
   return rrnco_rollout_workspace_bytes((int32_t)env, (int32_t)n_nodes, n_inst, (int32_t)n_starts);
 }
@@ -279,6 +323,8 @@ TORCH_LIBRARY(rrnco_b200, m) {
         "Tensor(a!) status) -> (Tensor, Tensor, Tensor, Tensor)");
   m.def("beam_backtrack(Tensor actions, Tensor parents, Tensor logprobs, bool per_step_logprobs, Tensor(a!) status) -> "
         "(Tensor, Tensor, Tensor)");
+  m.def("beam_rollout(int env, int beam_width, Tensor?[] weights, float alpha, float beta, float tanh_clipping, "
+        "float temperature, Tensor?[] cache, Tensor?[] data, int t_cap, Tensor(a!) workspace) -> (Tensor, Tensor, Tensor, Tensor)");
   m.def("rollout_workspace_bytes(int env, int n_nodes, int n_inst, int n_starts) -> int", &rollout_workspace_bytes);
 }
 
@@ -292,4 +338,5 @@ TORCH_LIBRARY_IMPL(rrnco_b200, CUDA, m) {
   m.impl("rollout", &rollout);
   m.impl("beam_select", &beam_select);
   m.impl("beam_backtrack", &beam_backtrack);
+  m.impl("beam_rollout", &beam_rollout);
 }

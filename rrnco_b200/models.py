@@ -8,9 +8,10 @@ decoder and the whole decode loop running as fused sm_100a kernels (librrnco_b20
 
 The logit filters `top_k` / `top_p` of rl4co's `process_logits` run inside the decode kernels (any decode type), except
 under grad in phase "train" without forced actions: the differentiable replay does not filter, so that call raises.
-`decode_type="beam_search"` (rl4co BeamSearch; `beam_width=`, `select_best=` which defaults to True there) runs the
-per-step kernel pipeline for any N: rrnco_beam_select picks the beams, rrnco_beam_backtrack aligns the sequences.  It
-raises NotImplementedError together with top_k / top_p, with `actions=`, and under grad in phase "train".
+`decode_type="beam_search"` (rl4co BeamSearch; `beam_width=`, `select_best=` which defaults to True there) runs in one
+launch of the lean rollout kernel (rrnco_beam_rollout) for N <= 112 and up to 128 beams under the default engine and
+precision, and on the per-step kernel pipeline otherwise (rrnco_beam_select picks the beams); rrnco_beam_backtrack aligns
+the sequences.  It raises NotImplementedError together with top_k / top_p, with `actions=`, and under grad in phase "train".
 `select_best=True` on a multistart greedy / sampling decode keeps each instance's best start (first maximum of the reward).
 Unsupported reference options raise NotImplementedError (store_all_logp / return_entropy, mask_logits=False, dynamic
 embeddings): they are not on any BASELINE config.
@@ -29,7 +30,7 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import DECODE_ID, ENV_ID, DecoderCache, DecoderWeights, InstanceData, call, ptr, stream_ptr
-from .envs import _u8
+from .envs import _u8, tour_reward
 
 CTX_IN = {"atsp": 256, "rcvrp": 129, "rcvrptw": 132}
 N_STATE = {"atsp": 0, "rcvrp": 1, "rcvrptw": 4}
@@ -329,7 +330,8 @@ class RRNetPolicy(nn.Module):
         if beam:
             cache = self.decoder._precompute_cache((row_emb, col_emb), num_starts=beam_width)
             self._calls += 1
-            out = beam_search_rollout(self.decoder, cache, env, td, beam_width,
+            fused = fused_beam_serves(self.env_name, cache.glimpse_key.shape[1], beam_width)
+            out = (fused_beam_rollout if fused else beam_search_rollout)(self.decoder, cache, env, td, beam_width,
                                       temperature=decoding_kwargs.pop("temperature", self.temperature),
                                       tanh_clipping=decoding_kwargs.pop("tanh_clipping", self.tanh_clipping),
                                       calc_reward=calc_reward or select_best,
@@ -700,6 +702,81 @@ def beam_backtrack(actions, parents, logprobs, per_step_logprobs: bool = True, s
     return a, lp, ll, status
 
 
+def fused_beam_serves(env_name: str, n_nodes: int, beam_width: int) -> bool:
+    """Whether rrnco_beam_rollout serves a beam search of this size: N <= 112 and 2..128 beams, under the default engine and
+    precision (rrnco_set_ffn_engine(2), rrnco_set_precision(3)); beam_search_rollout serves every other call."""
+    return _lib.lib().rrnco_beam_rollout_workspace_bytes(ENV_ID[env_name], int(n_nodes), 1, int(beam_width)) > 0
+
+
+def fused_beam_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, beam_width: int,
+                       temperature: float = 1.0, tanh_clipping: float = 10.0, calc_reward: bool = True,
+                       per_step_logprobs: bool = False, check: bool = True) -> dict:
+    """beam_search_rollout in one launch of the lean rollout kernel (rrnco_beam_rollout): one CTA per instance whose W rows
+    are the beams; same rule, same outputs.  N <= 112 and W <= 128 under the default engine and precision only
+    (fused_beam_serves); NotImplementedError otherwise."""
+    W = beam_args(beam_width)
+    name = decoder.env_name
+    dev = cache.glimpse_key.device
+    n_inst, N, _ = cache.glimpse_key.shape
+    R = n_inst * W
+    ws_bytes = _lib.lib().rrnco_beam_rollout_workspace_bytes(ENV_ID[name], N, n_inst, W)
+    if ws_bytes <= 0:
+        raise NotImplementedError(f"the fused beam search serves N <= {_lib.MAX_NODES_LEAN} and beam widths up to "
+                                  f"{_lib.MAX_BEAM_WIDTH_FUSED} under the default engine and precision (got N={N}, W={W}): "
+                                  "use beam_search_rollout")
+    num_loc = getattr(getattr(env, "generator", None), "num_loc", None)
+    if num_loc is not None and num_loc != (N if name == "atsp" else N - 1):
+        raise ValueError(f"env.generator.num_loc = {num_loc} does not match the instance size ({N} nodes): the fused "
+                         "kernel's start-node rule would differ from env.select_start_nodes")
+    t_cap = N if name == "atsp" else 2 * N + 3  # the per-step loop's bound (beam_search_rollout)
+    ws = _workspace(dev, ws_bytes)
+    from . import torch_ops
+    if torch_ops.enabled():
+        wt, alpha, beta = decoder.kernel_weight_tensors()
+        acts, parents, lps, info = torch_ops.ops().beam_rollout(
+            ENV_ID[name], W, wt, alpha, beta, float(tanh_clipping), float(temperature),
+            [cache.glimpse_key, cache.glimpse_val, cache.logit_key, cache.ctx_node_proj, cache.ctx_node_proj2],
+            instance_tensors_from_td(name, td), t_cap, ws)
+        _lib.count_call("rrnco_beam_rollout")
+    else:
+        keep = []
+        w, keep_w = decoder.kernel_weights(temperature, tanh_clipping)
+        data = instance_data_from_td(name, td, keep)
+        acts = torch.empty((t_cap, R), dtype=torch.int64, device=dev)
+        parents = torch.empty((t_cap, R), dtype=torch.int64, device=dev)
+        lps = torch.empty((t_cap, R), dtype=torch.float32, device=dev)
+        info = torch.zeros(2, dtype=torch.int32, device=dev)  # [steps, status]
+        cs = cache.struct()
+        call("rrnco_beam_rollout", ENV_ID[name], N, n_inst, W, C.byref(w), C.byref(cs), C.byref(data), t_cap, ptr(acts),
+             ptr(parents), ptr(lps), ptr(info[0:1]), ptr(info[1:2]), ptr(ws), stream_ptr(dev))
+    T = int(info[0].item())
+    acts, lps, ll, status = beam_backtrack(acts[:T], parents[:T], lps[:T], per_step_logprobs, info[1:2])
+    if check:
+        _lib.raise_device_status(int(status.item()))
+    return _beam_outputs(name, env, td, acts, lps, ll, per_step_logprobs, calc_reward)
+
+
+def _beam_outputs(name, env, td, acts, lps, ll, per_step_logprobs, calc_reward) -> dict:
+    """The out-dict of a beam search from its backtracked sequences: actions, log_likelihood, logprobs, rewards."""
+    out = {"actions": acts, "log_likelihood": ll}
+    if per_step_logprobs:
+        out["logprobs"] = lps
+    has_minmax = "min_distance" in td.keys()
+    if calc_reward:
+        open_route = td["open_route"] if name == "rcvrptw" else None
+        real, norm = tour_reward(acts, td["distance_matrix"], name != "atsp", open_route,
+                                 td["min_distance"] if has_minmax and env.normalize else None,
+                                 td["max_distance"] if has_minmax and env.normalize else None)
+        if env.normalize and has_minmax:
+            out["reward"], out["normalized_reward"] = real, norm
+        else:
+            out["reward"] = norm
+    else:
+        out["reward"] = torch.zeros(acts.shape[0], dtype=torch.float32 if name == "rcvrptw" else torch.bool,
+                                    device=acts.device)
+    return out
+
+
 def beam_search_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td, beam_width: int,
                         temperature: float = 1.0, tanh_clipping: float = 10.0, calc_reward: bool = True,
                         per_step_logprobs: bool = False, check: bool = True) -> dict:
@@ -709,7 +786,6 @@ def beam_search_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td,
     beams (what stepwise_rollout replicates), never the instance matrices.  Returns the [W * B] outputs of every beam."""
     W = beam_args(beam_width)
     from .tdlite import TensorDictLite, batchify
-    from .envs import tour_reward
     name = decoder.env_name
     n_inst, N, _ = cache.glimpse_key.shape
     R = n_inst * W
@@ -745,19 +821,4 @@ def beam_search_rollout(decoder: RRNetDecoder, cache: PrecomputedCache, env, td,
                                            per_step_logprobs, status)
     if check:
         _lib.raise_device_status(int(status.item()))
-    out = {"actions": acts, "log_likelihood": ll}
-    if per_step_logprobs:
-        out["logprobs"] = lps
-    has_minmax = "min_distance" in td.keys()
-    if calc_reward:
-        open_route = td["open_route"] if name == "rcvrptw" else None
-        real, norm = tour_reward(acts, td["distance_matrix"], name != "atsp", open_route,
-                                 td["min_distance"] if has_minmax and env.normalize else None,
-                                 td["max_distance"] if has_minmax and env.normalize else None)
-        if env.normalize and has_minmax:
-            out["reward"], out["normalized_reward"] = real, norm
-        else:
-            out["reward"] = norm
-    else:
-        out["reward"] = torch.zeros(R, dtype=torch.float32 if name == "rcvrptw" else torch.bool, device=dev)
-    return out
+    return _beam_outputs(name, env, td, acts, lps, ll, per_step_logprobs, calc_reward)

@@ -1,8 +1,10 @@
 """Cost of beam search: whole RRNetPolicy.forward calls with a fixed encoder output, beam_search (all beams kept,
 select_best=False) against multistart greedy at the same instances x width, timed with CUDA events after a warm-up of
-every shape.  Beam search runs the per-step kernel pipeline (rrnco_decoder_logits[_large] -> rrnco_beam_select -> env
-step, then rrnco_beam_backtrack); multistart greedy runs the fused rollout kernel.  On the first decode step's inputs it
-also times one decoder step (RRNetDecoder.forward) and rrnco_beam_select alone, median of 20 calls each.
+every shape, all in the same run.  Beam search runs on two routes where both serve the shape: the fused lean kernel
+(rrnco_beam_rollout, N <= 112 and W <= 128: what RRNetPolicy.forward picks there) and the per-step kernel pipeline
+(rrnco_decoder_logits[_large] -> rrnco_beam_select -> env step); both end in rrnco_beam_backtrack.  Multistart greedy
+runs the fused rollout kernel.  On the first decode step's inputs it also times one decoder step (RRNetDecoder.forward)
+and rrnco_beam_select alone, median of 20 calls each.
   * RCVRPTW n=100 and RCVRP n=100, 1024 instances x 100 beams / starts;
   * ATSP n=200, 64 x 100.
    python tools/beam_search_probe.py [--reps 5]"""
@@ -102,14 +104,30 @@ def main():
     for name, n, B, W in SHAPES:
         env, td, pol = setup(name, n, B)
         ms_g, t_g, out_g = timed(lambda: pol(td, env, phase="test", decode_type="multistart_greedy", num_starts=W), args.reps)
-        ms_b, t_b, out_b = timed(lambda: pol(td, env, phase="test", decode_type="beam_search", beam_width=W,
-                                             select_best=False), args.reps)
+        beam = lambda: pol(td, env, phase="test", decode_type="beam_search", beam_width=W, select_best=False)  # noqa: E731
+        fused = models.fused_beam_serves(name, td["action_mask"].shape[-1], W)
+        if fused:
+            ms_f, t_f, out_f = timed(beam, args.reps)
+        serves = models.fused_beam_serves
+        models.fused_beam_serves = lambda *a: False  # the per-step pipeline for every shape
+        try:
+            ms_b, t_b, out_b = timed(beam, args.reps)
+        finally:
+            models.fused_beam_serves = serves
         best_g = out_g["reward"].view(W, B).max(0)[0].mean().item()
         best_b = out_b["reward"].view(W, B).max(0)[0].mean().item()
         T = out_b["actions"].shape[1]
         print(f"{name} n={n} {B}x{W}: multistart greedy {ms_g:9.2f} ms (fused kernel; spread {min(t_g):.2f}-{max(t_g):.2f}); "
               f"beam search {ms_b:9.2f} ms (per-step pipeline, {T} steps, {ms_b / T * 1e3:.0f} us/step; spread "
               f"{min(t_b):.2f}-{max(t_b):.2f}); {ms_b / ms_g:6.2f}x; mean best reward greedy {best_g:.4f}, beam {best_b:.4f}")
+        if fused:
+            best_f = out_f["reward"].view(W, B).max(0)[0].mean().item()
+            same = sum(sorted(map(tuple, out_f["actions"].view(W, B, -1)[:, b].tolist()))
+                       == sorted(map(tuple, out_b["actions"].view(W, B, -1)[:, b].tolist()))
+                       for b in range(B)) if out_f["actions"].shape == out_b["actions"].shape else 0
+            print(f"{name} n={n} {B}x{W}: fused beam search {ms_f:9.2f} ms (rrnco_beam_rollout; spread {min(t_f):.2f}-"
+                  f"{max(t_f):.2f}); {ms_f / ms_g:6.2f}x multistart greedy, {ms_b / ms_f:6.2f}x faster than per-step; "
+                  f"mean best reward {best_f:.4f}; identical beam sets with per-step on {same} / {B} instances")
         t_dec, t_sel = step_times(env, td, pol, name, W)
         print(f"{name} n={n} {B}x{W}: first beam step: decoder {t_dec * 1e3:7.0f} us, rrnco_beam_select {t_sel * 1e3:7.0f} us "
               f"({t_sel / (t_dec + t_sel):.0%} of the two)")
